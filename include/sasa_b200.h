@@ -172,6 +172,24 @@ SASA_B200_API int sasa_b200_batch_run_device(sasa_b200_batch *batch, const float
  * reports deferred errors (e.g. SASA_B200_ERR_NON_FINITE). */
 SASA_B200_API int sasa_b200_batch_sync(sasa_b200_batch *batch, sasa_b200_stats *stats /* nullable */);
 
+/* Grouped runs: buried surface area in one pass.  group holds one label per atom; only equality within a structure matters.
+ *   out           the complex: exactly what sasa_b200_batch_run_host / _device give for the same input, bit for bit.
+ *   out_isolated  every atom as the engine computes it when its group runs alone (the group's atoms as their own structure,
+ *                 in original order, same id_class rule): neighbour j occludes atom i only if group[j] == group[i].  Level sums
+ *                 use the batch's segments with the same summation order, so they equal the sums over the isolated per-atom
+ *                 areas bit for bit wherever the plain run's sums are sequential (<= 16,384 atoms per sum).
+ * Buried area = isolated - complex; the caller derives it.  count_isolated[i] >= count[i]; one group for all atoms gives
+ * isolated == complex; one group per atom gives count_isolated[i] == n_points.  Every output field of both structs is
+ * nullable.  group == NULL: SASA_B200_ERR_INVALID_ARGUMENT; params->flags != 0: SASA_B200_ERR_UNSUPPORTED.  Non-finite
+ * input: SASA_B200_ERR_NON_FINITE with both output sets NaN-filled for that structure.  The host form uses the per-chunk
+ * pipeline; the device form behaves like sasa_b200_batch_run_device (stream-ordered, errors via sasa_b200_batch_sync). */
+SASA_B200_API int sasa_b200_batch_run_groups_host(sasa_b200_batch *batch, const float *xyzr, const uint32_t *id_class,
+                                    const uint32_t *group, const sasa_b200_params *params, const sasa_b200_outputs *out,
+                                    const sasa_b200_outputs *out_isolated, sasa_b200_stats *stats /* nullable */);
+SASA_B200_API int sasa_b200_batch_run_groups_device(sasa_b200_batch *batch, const float *d_xyzr, const uint32_t *d_id_class,
+                                      const uint32_t *d_group, const sasa_b200_params *params, const sasa_b200_outputs *d_out,
+                                      const sasa_b200_outputs *d_out_isolated, void *stream);
+
 /* MD-trajectory form (what mdsasa-bolt feeds calculate_sasa_internal per frame): a batch
  * created with S = n_frames equal-sized structures; xyz holds n_frames * n_atoms_per_frame
  * * 3 floats, radii n_atoms_per_frame floats shared by every frame (12 B/atom/frame on the

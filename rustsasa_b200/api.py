@@ -11,11 +11,13 @@ Same names, argument meaning and error behaviour as the crate (rust-sasa 0.9.2):
 
 The numeric core is the C ABI (include/sasa_b200.h); there is no CPU path here.
 ``process_many`` is the batched form the CLI's directory mode (src/main.rs:342-480) maps onto.
+``process_interface`` adds buried surface area: every structure in the complex and with each chain group standing alone,
+from one grouped batch call.
 """
 from __future__ import annotations
 
 from dataclasses import dataclass
-from typing import List, Optional, Sequence
+from typing import Any, List, Optional, Sequence
 
 import numpy as np
 
@@ -63,6 +65,15 @@ class ProteinResult:
     global_total: float
     polar_total: float
     non_polar_total: float
+
+
+@dataclass
+class InterfaceResult:
+    """One structure of ``SASAOptions.process_interface``: the level's result in the complex and with every chain group
+    standing alone, and the buried area isolated - complex of the protein totals (global)."""
+    complex: Any
+    isolated: Any
+    buried_area: float
 
 
 class AtomLevel:
@@ -152,6 +163,32 @@ class SASAOptions:
         """Batched form: all structures go through ONE pipelined batch call.  A structure whose extraction
         fails is reported as its ``SASACalcError`` in the result list (directory mode logs and continues,
         src/main.rs:447-453)."""
+        return self._run_many(structures, engine, None)
+
+    def process_interface(self, structures: Sequence[Structure], chain_groups: Optional[Sequence[str]] = None,
+                          engine: Optional[Engine] = None) -> List:
+        """Buried surface area: per structure an :class:`InterfaceResult` with the level's result in the complex and
+        with every chain group standing alone (only atoms of its own group occlude an atom), both from ONE grouped batch
+        call.  ``chain_groups``: strings of chain ids, e.g. ``["AB", "C"]`` puts chains A and B in one group; a chain not
+        listed is a group of its own; None: one group per chain.  Chains are keyed by chain id across models.  A structure
+        whose extraction fails is reported as its ``SASACalcError``, as in ``process_many``."""
+        return self._run_many(structures, engine, list(chain_groups) if chain_groups is not None else [])
+
+    @staticmethod
+    def _chain_groups(atom_chain: np.ndarray, chain_groups: List[str]) -> np.ndarray:
+        """Dense per-atom group labels of one structure."""
+        label = {}
+        for g, ids in enumerate(chain_groups):
+            for c in ids:
+                label.setdefault(c, g)
+        out = np.empty(atom_chain.shape[0], np.uint32)
+        for i, c in enumerate(atom_chain):
+            if c not in label:
+                label[c] = len(chain_groups) + len(label)
+            out[i] = label[c]
+        return out
+
+    def _run_many(self, structures: Sequence[Structure], engine: Optional[Engine], chain_groups: Optional[List[str]]) -> List:
         eng = engine or default_engine()
         packed: List[Optional[PackedStructure]] = []
         results: List = [None] * len(structures)
@@ -183,23 +220,34 @@ class SASAOptions:
         batch = Batch(eng, struct_off, seg_be if seg_be.shape[0] else None, seg_off if seg_be.shape[0] else None,
                       polar if seg_be.shape[0] else None)
         try:
-            res = batch.run_host(xyzr, id_class, self.probe_radius, self.n_points, want=want)
+            if chain_groups is None:
+                res = batch.run_host(xyzr, id_class, self.probe_radius, self.n_points, want=want)
+            else:   # the protein totals give the buried area: always requested
+                group = np.concatenate([self._chain_groups(packed[i].atom_chain, chain_groups) for i in good])
+                cpx, iso = batch.run_groups_host(xyzr, group, id_class, self.probe_radius, self.n_points,
+                                                 want=tuple(set(want) | {"protein"}))
         finally:
             batch.close()
-        for k, i in enumerate(good):
-            p = packed[i]
+
+        def level_result(res, k, p):
             a0, a1 = int(struct_off[k]), int(struct_off[k + 1])
             g0, g1 = int(seg_off[k]), int(seg_off[k + 1])
             if level == "atom":
-                results[i] = res.atom_sasa[a0:a1].copy()
-            elif level == "residue":
-                results[i] = [ResidueResult(m["serial_number"], m["insertion_code"], float(v), m["name"],
-                                            m["is_polar"], m["chain_id"])
-                              for m, v in zip(p.seg_meta, res.seg_sasa[g0:g1])] if g1 > g0 else []
-            elif level == "chain":
-                results[i] = [ChainResult(m["name"], float(v)) for m, v in zip(p.seg_meta, res.seg_sasa[g0:g1])] \
+                return res.atom_sasa[a0:a1].copy()
+            if level == "residue":
+                return [ResidueResult(m["serial_number"], m["insertion_code"], float(v), m["name"],
+                                      m["is_polar"], m["chain_id"])
+                        for m, v in zip(p.seg_meta, res.seg_sasa[g0:g1])] if g1 > g0 else []
+            if level == "chain":
+                return [ChainResult(m["name"], float(v)) for m, v in zip(p.seg_meta, res.seg_sasa[g0:g1])] \
                     if g1 > g0 else []
+            t = res.protein[k]
+            return ProteinResult(float(t[0]), float(t[1]), float(t[2]))
+
+        for k, i in enumerate(good):
+            if chain_groups is None:
+                results[i] = level_result(res, k, packed[i])
             else:
-                t = res.protein[k]
-                results[i] = ProteinResult(float(t[0]), float(t[1]), float(t[2]))
+                results[i] = InterfaceResult(level_result(cpx, k, packed[i]), level_result(iso, k, packed[i]),
+                                             float(iso.protein[k, 0]) - float(cpx.protein[k, 0]))
         return results

@@ -48,9 +48,9 @@ struct Points {
 
 struct SmallCfg {
     int nt, minb;
-    uint32_t cap[2];   // atom capacity without / with id classes (compile-time constants of the configuration)
+    uint32_t cap[4];   // atom capacity, index = has_cls + 2 * grouped (compile-time constants of the configuration)
     uint32_t cmax;
-    size_t smem[2];    // dynamic shared memory of a launch: without / with id classes
+    size_t smem[4];    // dynamic shared memory of a launch, same index
     int proto;
 };
 
@@ -115,7 +115,7 @@ struct sasa_b200_ctx {
     LargeWorkspace large;
     cudaEvent_t ev_large = nullptr;
     bool large_used = false;
-    bool attr_done[8][6] = {};   // [kernel configuration][instantiation]: shared-memory attribute set (at first launch)
+    bool attr_done[8][8] = {};   // [kernel configuration][instantiation]: shared-memory attribute set (at first launch)
     // jobs: one per host-buffer run in flight (submit / wait); recycled, so events and the pinned status word are made once
     std::vector<sasa_b200_job *> free_jobs;
     cudaEvent_t ev_tail[kStreams] = {};   // end of the previous job on each copy stream (the next job's first stream waits on them)
@@ -222,18 +222,22 @@ int get_points(sasa_b200_ctx *ctx, uint32_t n, const Points **out) {
 // Shared-memory configurations of the fused kernel, smallest atom capacity first.  nmax is derived from the
 // per-CTA budget that lets `minb` CTAs share one SM (228 KB per SM, 1 KB reserved per CTA, 227 KB per CTA max).
 typedef void (*SmallKernel)(const KParams);
+typedef void (*GroupKernel)(const KParams, const GroupParams);
 struct Proto {
     int nt, minb;
     uint32_t cmax;
-    uint32_t cap[2];     // max_atoms(...) without / with id classes
+    uint32_t cap[4];     // max_atoms(...), index = has_cls + 2 * grouped
     SmallKernel fn[6];   // index = has_cls + 2 * tight (tight: n_points <= 128, no statistics / forced streaming)
                          //         + 2 more when the tight kernel compiled for 3 body slots applies (65..96 body points)
+    GroupKernel fng[2];  // grouped runs (n_points <= 128), index = has_cls
 };
 #define SASA_PROTO(NT, MINB, CMAX)                                                                                     \
-    Proto { NT, MINB, CMAX, { max_atoms(NT, MINB, CMAX, false), max_atoms(NT, MINB, CMAX, true) },                     \
+    Proto { NT, MINB, CMAX, { max_atoms(NT, MINB, CMAX, false), max_atoms(NT, MINB, CMAX, true),                       \
+                              max_atoms(NT, MINB, CMAX, false, true), max_atoms(NT, MINB, CMAX, true, true) },         \
             { sasa_small_kernel<NT, MINB, false, CMAX>, sasa_small_kernel<NT, MINB, true, CMAX>,                       \
               sasa_tight_kernel<NT, MINB, false, CMAX, 0>, sasa_tight_kernel<NT, MINB, true, CMAX, 0>,                 \
-              sasa_tight_kernel<NT, MINB, false, CMAX, 3>, sasa_tight_kernel<NT, MINB, true, CMAX, 3> } }
+              sasa_tight_kernel<NT, MINB, false, CMAX, 3>, sasa_tight_kernel<NT, MINB, true, CMAX, 3> },               \
+            { sasa_tight_groups_kernel<NT, MINB, false, CMAX>, sasa_tight_groups_kernel<NT, MINB, true, CMAX> } }
 // 0-2 keep 32 warps resident per SM (64 registers/thread); 3-4 keep 24 warps (85 registers/thread)
 #ifndef SASA_ALL_PROTOS   // the shipped build instantiates the two default configurations only (half the build time and library
                          // size); -DSASA_ALL_PROTOS adds the three tuning configurations selectable with SASA_B200_CFGS
@@ -255,9 +259,9 @@ int build_cfgs(sasa_b200_ctx *ctx) {
     for (int i = 0; i < kNumProtos; ++i) {
         const Proto &pr = kProtos[i];
         if (!strchr(only, '0' + i)) continue;
-        SmallCfg c{pr.nt, pr.minb, {pr.cap[0], pr.cap[1]}, pr.cmax, {0, 0}, i};
-        for (int v = 0; v < 2; ++v) c.smem[v] = small_layout(c.cap[v], c.cmax, c.nt / 32, v == 1).total;
-        if (c.cap[0] == 0 || c.cap[1] == 0 || std::max(c.smem[0], c.smem[1]) > ctx->smem_optin)
+        SmallCfg c{pr.nt, pr.minb, {pr.cap[0], pr.cap[1], pr.cap[2], pr.cap[3]}, pr.cmax, {0, 0, 0, 0}, i};
+        for (int v = 0; v < 4; ++v) c.smem[v] = small_layout(c.cap[v], c.cmax, c.nt / 32, (v & 1) == 1, v >= 2).total;
+        if (*std::min_element(c.cap, c.cap + 4) == 0 || *std::max_element(c.smem, c.smem + 4) > ctx->smem_optin)
             return fail(ctx, SASA_B200_ERR_UNSUPPORTED, "the fused kernels are laid out for 228 KB of shared memory per SM (B200); this device offers %zu per block",
                         ctx->smem_optin);
         // (the MaxDynamicSharedMemorySize attribute is set at a kernel's first launch, enqueue_chunk: touching all thirty
@@ -269,7 +273,9 @@ int build_cfgs(sasa_b200_ctx *ctx) {
     return SASA_B200_OK;
 }
 
-uint32_t cfg_capacity(const sasa_b200_ctx *, const SmallCfg &c, bool has_cls) { return c.cap[has_cls ? 1 : 0]; }
+uint32_t cfg_capacity(const sasa_b200_ctx *, const SmallCfg &c, bool has_cls, bool grouped = false) {
+    return c.cap[(has_cls ? 1 : 0) + (grouped ? 2 : 0)];
+}
 
 struct Launch {
     int cfg;          // index into ctx->cfgs, or -1 for the large-structure path
@@ -293,20 +299,21 @@ struct sasa_b200_batch {
     bool single_latency = false;   // one-structure convenience calls: prefer the multi-CTA large-structure path (see build_plan)
     std::vector<uint32_t> h_off;      // S+1
     std::vector<uint32_t> h_seg_off;  // S+1
-    // two launch plans (without / with id classes: capacities differ)
-    // index = variant + 2*mode; variant: 0 without / 1 with id classes (capacities differ);
-    // mode: 0 = chunked for the pipelined host entry points, 1 = one chunk for device-resident runs
-    std::vector<Chunk> plan[4];
-    std::vector<uint32_t> h_order[4];
+    // launch plans, index = variant + 2*mode + 4*grouped; variant: 0 without / 1 with id classes (capacities differ);
+    // mode: 0 = chunked for the pipelined host entry points, 1 = one chunk for device-resident runs; grouped: the plans of
+    // sasa_b200_batch_run_groups_* (8 B more shared memory per atom)
+    std::vector<Chunk> plan[8];
+    std::vector<uint32_t> h_order[8];
     // gated single-launch pipeline (host plans 0 / 1 only): the whole batch as ONE queue in an order that follows the arrival of
     // the chunks, and per queue position the number of chunks that must have arrived (empty: the plan does not qualify)
     std::vector<uint32_t> h_gorder[2], h_gneed[2];
     uint32_t *d_gorder[2] = {nullptr, nullptr}, *d_gneed[2] = {nullptr, nullptr};
-    uint32_t n_counters[4] = {0, 0, 0, 0};
-    uint32_t max_large = 0;             // largest structure that takes the large-structure path in ANY plan (workspace size)
-    uint32_t max_large_v[4] = {0, 0, 0, 0};   // ... per plan: a structure may fit the fused kernels without id classes only
+    uint32_t n_counters[8] = {};
+    uint32_t max_large = 0;             // largest structure that takes the large-structure path in any ungrouped plan (workspace size)
+    uint32_t max_large_v[8] = {};       // ... per plan: a structure may fit the fused kernels without id classes only
+    uint32_t max_struct = 0;            // largest structure (grouped runs with n_points > 128 take the large-structure path throughout)
     // device topology
-    uint32_t *d_off = nullptr, *d_seg_off = nullptr, *d_order[4] = {nullptr, nullptr, nullptr, nullptr}, *d_counters = nullptr;
+    uint32_t *d_off = nullptr, *d_seg_off = nullptr, *d_order[8] = {}, *d_counters = nullptr;
     uint2 *d_seg_be = nullptr;
     uint8_t *d_polar = nullptr;
     sasa_b200_stats last = {};
@@ -381,14 +388,14 @@ int arena_reserve(sasa_b200_ctx *ctx, size_t bytes) {
 
 void build_plan(sasa_b200_batch *b, int variant) {
     sasa_b200_ctx *ctx = b->ctx;
-    const bool has_cls = (variant & 1) == 1;
+    const bool has_cls = (variant & 1) == 1, grouped = (variant & 4) != 0;
     static const size_t chunk_env = [] {
         const char *e = getenv("SASA_B200_CHUNK_ATOMS");   // tuning aid: atoms per pipelined chunk of the host entry points
         return e ? (size_t)atoll(e) : kChunkAtoms;
     }();
     const size_t chunk_atoms = (variant & 2) ? ~(size_t)0 : chunk_env;
     std::vector<uint32_t> cap;
-    for (const SmallCfg &c : ctx->cfgs) cap.push_back(cfg_capacity(ctx, c, has_cls));
+    for (const SmallCfg &c : ctx->cfgs) cap.push_back(cfg_capacity(ctx, c, has_cls, grouped));
     std::vector<Chunk> &plan = b->plan[variant];
     std::vector<uint32_t> &order = b->h_order[variant];
     plan.clear();
@@ -435,7 +442,7 @@ void build_plan(sasa_b200_batch *b, int variant) {
             if (b->single_latency && b->S == 1 && n >= kSingleLargeMin) k = cap.size();
             bucket[k].push_back(i);
             if (k == cap.size()) {
-                b->max_large = std::max(b->max_large, n);
+                if (!grouped) b->max_large = std::max(b->max_large, n);   // (grouped runs reserve the workspace at run time)
                 b->max_large_v[variant] = std::max(b->max_large_v[variant], n);
             }
         }
@@ -550,8 +557,9 @@ int check_params(sasa_b200_ctx *ctx, const sasa_b200_params *p) {
 // Enqueue every kernel of one chunk: the first fused launch on `st`, the others on sibling streams forked from and
 // joined back into `st` (so the caller still sees one stream-ordered unit of work).  Large-structure pipelines stay
 // on `st`.
+// gp: grouped runs (group labels and isolated outputs), else null.
 int enqueue_chunk(sasa_b200_batch *b, int variant, const Chunk &ch, const KParams &base, cudaStream_t st,
-                  uint32_t *launches, const uint32_t *order_override = nullptr) {
+                  uint32_t *launches, const uint32_t *order_override = nullptr, const GroupParams *gp = nullptr) {
     sasa_b200_ctx *ctx = b->ctx;
     int n_small = 0;
     for (const Launch &L : ch.launches) n_small += L.cfg >= 0;
@@ -561,42 +569,46 @@ int enqueue_chunk(sasa_b200_batch *b, int variant, const Chunk &ch, const KParam
     const bool fork = !no_fork && (variant & 2) && n_small > 1 && n_small <= sasa_b200_ctx::kSide + 1;
     if (fork) CU_TRY(ctx, cudaEventRecord(ctx->ev_fork, st));
     int small_idx = 0, forked = 0;
+    // grouped runs with more than 128 points: no fused kernel, every structure takes the large-structure path
+    const bool all_large = gp && base.n_points > 128;
     for (const Launch &L : ch.launches) {
         KParams kp = base;
         kp.order = order_override ? order_override : b->d_order[variant] + L.order_off;
         kp.n_work = L.n_work;
         kp.work_counter = b->d_counters + L.counter;
-        if (L.cfg < 0) {
+        if (L.cfg < 0 || all_large) {
             if (ctx->large_used) CU_TRY(ctx, cudaStreamWaitEvent(st, ctx->ev_large, 0));
             int rc = large_enqueue(ctx->sm_count, ctx->large, kp, &b->h_order[variant][L.order_off], L.n_work,
-                                   b->h_off.data(), b->h_seg_off.empty() ? nullptr : b->h_seg_off.data(), st, launches);
+                                   b->h_off.data(), b->h_seg_off.empty() ? nullptr : b->h_seg_off.data(), st, launches, 0, 1, gp);
             if (rc != 0) return fail(ctx, rc, "large-structure path failed: %s", cudaGetErrorString(cudaGetLastError()));
             CU_TRY(ctx, cudaEventRecord(ctx->ev_large, st));
             ctx->large_used = true;
             continue;
         }
         const SmallCfg &c = ctx->cfgs[L.cfg];
-        const bool has_cls = (variant & 1) == 1;
-        kp.nmax = cfg_capacity(ctx, c, has_cls);
+        const bool has_cls = (variant & 1) == 1, grouped = gp != nullptr;
+        kp.nmax = cfg_capacity(ctx, c, has_cls, grouped);
         kp.cmax = c.cmax;
-        const size_t smem = c.smem[has_cls ? 1 : 0];
+        const size_t smem = c.smem[(has_cls ? 1 : 0) + (grouped ? 2 : 0)];
         const int grid = (int)std::min<uint32_t>(L.n_work, (uint32_t)(ctx->sm_count * c.minb));
         cudaStream_t ls = st;
         if (fork && small_idx > 0) {
             ls = ctx->side[small_idx - 1];
             CU_TRY(ctx, cudaStreamWaitEvent(ls, ctx->ev_fork, 0));
         }
-        void *args[] = {(void *)&kp};
+        void *args[] = {(void *)&kp, (void *)gp};
         const bool tight = kp.n_points <= 128 && (kp.flags & 3u) == 0;
         const uint32_t body = std::min(kp.n_points, kp.n_body);
-        const int which = (has_cls ? 1 : 0) + (tight ? (SASA_OPT_NSLT && body > 64 && body <= 96 ? 4 : 2) : 0);
+        // (attribute slots 6 / 7: the grouped kernels)
+        const int which = grouped ? 6 + (has_cls ? 1 : 0) : (has_cls ? 1 : 0) + (tight ? (SASA_OPT_NSLT && body > 64 && body <= 96 ? 4 : 2) : 0);
+        const void *fn = grouped ? (const void *)kProtos[c.proto].fng[has_cls ? 1 : 0] : (const void *)kProtos[c.proto].fn[which];
         if (!ctx->attr_done[c.proto][which]) {
-            cudaError_t ea = cudaFuncSetAttribute((const void *)kProtos[c.proto].fn[which], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            cudaError_t ea = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
             if (ea != cudaSuccess)
                 return fail(ctx, SASA_B200_ERR_CUDA, "cudaFuncSetAttribute(MaxDynamicSharedMemorySize=%zu) failed: %s", smem, cudaGetErrorString(ea));
             ctx->attr_done[c.proto][which] = true;
         }
-        cudaError_t e = cudaLaunchKernel((const void *)kProtos[c.proto].fn[which], dim3(grid), dim3(c.nt), args, smem, ls);
+        cudaError_t e = cudaLaunchKernel(fn, dim3(grid), dim3(c.nt), args, smem, ls);
         if (e != cudaSuccess) return fail(ctx, SASA_B200_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(e));
         if (ls != st) {
             CU_TRY(ctx, cudaEventRecord(ctx->ev_join[small_idx - 1], ls));
@@ -812,8 +824,9 @@ static int batch_create_impl(sasa_b200_ctx *ctx, const uint64_t *struct_off, siz
                                         (unsigned long long)k, s));
         }
     }
-    for (int v = 0; v < 4; ++v) build_plan(b, v);
+    for (int v = 0; v < 8; ++v) build_plan(b, v);
     for (int v = 0; v < 2; ++v) build_gated_order(b, v);
+    for (size_t i = 0; i < S; ++i) b->max_struct = std::max(b->max_struct, b->h_off[i + 1] - b->h_off[i]);
 #define B_TRY(expr)                                                                                            \
     do {                                                                                                       \
         cudaError_t e__ = (expr);                                                                              \
@@ -825,7 +838,7 @@ static int batch_create_impl(sasa_b200_ctx *ctx, const uint64_t *struct_off, siz
     B_TRY(cudaSetDevice(ctx->device));
     B_TRY(cudaMallocAsync(&b->d_off, (S + 1) * sizeof(uint32_t), ps));
     B_TRY(cudaMemcpyAsync(b->d_off, b->h_off.data(), (S + 1) * sizeof(uint32_t), cudaMemcpyHostToDevice, ps));
-    for (int v = 0; v < 4; ++v) {
+    for (int v = 0; v < 8; ++v) {
         B_TRY(cudaMallocAsync(&b->d_order[v], std::max<size_t>(1, b->h_order[v].size()) * sizeof(uint32_t), ps));
         if (!b->h_order[v].empty())
             B_TRY(cudaMemcpyAsync(b->d_order[v], b->h_order[v].data(), b->h_order[v].size() * sizeof(uint32_t), cudaMemcpyHostToDevice, ps));
@@ -837,7 +850,7 @@ static int batch_create_impl(sasa_b200_ctx *ctx, const uint64_t *struct_off, siz
         B_TRY(cudaMemcpyAsync(b->d_gorder[v], b->h_gorder[v].data(), b->h_gorder[v].size() * sizeof(uint32_t), cudaMemcpyHostToDevice, ps));
         B_TRY(cudaMemcpyAsync(b->d_gneed[v], b->h_gneed[v].data(), b->h_gneed[v].size() * sizeof(uint32_t), cudaMemcpyHostToDevice, ps));
     }
-    B_TRY(cudaMallocAsync(&b->d_counters, std::max<uint32_t>(1, *std::max_element(b->n_counters, b->n_counters + 4)) * sizeof(uint32_t), ps));
+    B_TRY(cudaMallocAsync(&b->d_counters, std::max<uint32_t>(1, *std::max_element(b->n_counters, b->n_counters + 8)) * sizeof(uint32_t), ps));
     if (b->n_seg) {
         B_TRY(cudaMallocAsync(&b->d_seg_be, b->n_seg * sizeof(uint2), ps));
         B_TRY(cudaMemcpyAsync(b->d_seg_be, seg_be, b->n_seg * sizeof(uint2), cudaMemcpyHostToDevice, ps));
@@ -872,7 +885,7 @@ void sasa_b200_batch_destroy(sasa_b200_batch *b) {
     cudaStream_t ps = b->ctx->streams[0];
     if (b->d_off) cudaFreeAsync(b->d_off, ps);
     if (b->d_seg_off) cudaFreeAsync(b->d_seg_off, ps);
-    for (int v = 0; v < 4; ++v)
+    for (int v = 0; v < 8; ++v)
         if (b->d_order[v]) cudaFreeAsync(b->d_order[v], ps);
     for (int v = 0; v < 2; ++v) {
         if (b->d_gorder[v]) cudaFreeAsync(b->d_gorder[v], ps);
@@ -884,31 +897,65 @@ void sasa_b200_batch_destroy(sasa_b200_batch *b) {
     delete b;
 }
 
-int sasa_b200_batch_run_device(sasa_b200_batch *b, const float *d_xyzr, const uint32_t *d_id_class,
-                               const sasa_b200_params *params, const sasa_b200_outputs *d_out, void *stream) {
+// Checks of the grouped entry points (after check_params), and the large-structure workspace their plan needs: structures that
+// no longer fit the fused kernels with the group arrays, or -- n_points > 128 -- every structure.  (ctx->mu is held.)
+static int prepare_groups(sasa_b200_batch *b, const uint32_t *group, const sasa_b200_params *params, const sasa_b200_outputs *out_iso,
+                          int variant) {
+    sasa_b200_ctx *ctx = b->ctx;
+    if (!group && b->n_atoms) return fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "group is NULL");
+    if (!out_iso) return fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "out_isolated is NULL");
+    if (params->flags != 0)
+        return fail(ctx, SASA_B200_ERR_UNSUPPORTED, "grouped runs support no flags (boundary statistics, forced streaming), got %u", params->flags);
+    const uint32_t need = params->n_points > 128 ? b->max_struct : b->max_large_v[variant];
+    if (need > ctx->large.cap_atoms) {
+        cudaDeviceSynchronize();   // growing frees buffers a run in flight may still use
+        int rc = large_reserve(ctx->large, need);
+        if (rc) return fail(ctx, rc, "allocating the large-structure workspace (%u atoms) failed", need);
+    }
+    return SASA_B200_OK;
+}
+
+static int run_device_impl(sasa_b200_batch *b, const float *d_xyzr, const uint32_t *d_id_class, const uint32_t *d_group,
+                           const sasa_b200_params *params, const sasa_b200_outputs *d_out, const sasa_b200_outputs *d_iso, void *stream) {
     if (!b) return SASA_B200_ERR_INVALID_ARGUMENT;
     sasa_b200_ctx *ctx = b->ctx;
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (!d_out || (!d_xyzr && b->n_atoms)) return fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "d_xyzr / d_out is NULL");
     int rc = check_params(ctx, params);
     if (rc) return rc;
+    const bool grouped = d_iso != nullptr;
+    const int variant = (d_id_class ? 1 : 0) + 2 + (grouped ? 4 : 0);
     CU_TRY(ctx, cudaSetDevice(ctx->device));
+    if (grouped && (rc = prepare_groups(b, d_group, params, d_iso, variant)) != 0) return rc;
     cudaStream_t st = stream ? (cudaStream_t)stream : ctx->streams[0];
     RunArgs ra;
     ra.d_xyzr = reinterpret_cast<const float4 *>(d_xyzr);
     ra.d_cls = d_id_class;
     ra.d_out = *d_out;
+    GroupParams gp{};
+    if (grouped) gp = GroupParams{d_group, d_iso->counts, d_iso->atom_sasa, b->n_seg ? d_iso->seg_sasa : nullptr, d_iso->protein};
     ra.prm = *params;
     if ((rc = get_points(ctx, params->n_points, &ra.pts)) != 0) return rc;
-    const int variant = (d_id_class ? 1 : 0) + 2;
     KParams base;
     make_kparams(b, ra, &base);
     b->launches_last = 0;
     if (b->n_counters[variant])
         CU_TRY(ctx, cudaMemsetAsync(b->d_counters, 0, b->n_counters[variant] * sizeof(uint32_t), st));
     for (const Chunk &ch : b->plan[variant])
-        if ((rc = enqueue_chunk(b, variant, ch, base, st, &b->launches_last)) != 0) return rc;
+        if ((rc = enqueue_chunk(b, variant, ch, base, st, &b->launches_last, nullptr, grouped ? &gp : nullptr)) != 0) return rc;
     return SASA_B200_OK;
+}
+
+int sasa_b200_batch_run_device(sasa_b200_batch *b, const float *d_xyzr, const uint32_t *d_id_class,
+                               const sasa_b200_params *params, const sasa_b200_outputs *d_out, void *stream) {
+    return run_device_impl(b, d_xyzr, d_id_class, nullptr, params, d_out, nullptr, stream);
+}
+
+int sasa_b200_batch_run_groups_device(sasa_b200_batch *b, const float *d_xyzr, const uint32_t *d_id_class, const uint32_t *d_group,
+                                      const sasa_b200_params *params, const sasa_b200_outputs *d_out,
+                                      const sasa_b200_outputs *d_out_isolated, void *stream) {
+    if (b && !d_out_isolated) return fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "d_out_isolated is NULL");
+    return run_device_impl(b, d_xyzr, d_id_class, d_group, params, d_out, d_out_isolated, stream);
 }
 
 int sasa_b200_batch_sync(sasa_b200_batch *b, sasa_b200_stats *stats) {
@@ -964,7 +1011,8 @@ static int job_abort(sasa_b200_ctx *ctx, sasa_b200_job *j, int rc) {
 
 static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *xyz3, const float *radii,
                             const uint32_t *id_class, const sasa_b200_params *params, const sasa_b200_outputs *out,
-                            sasa_b200_job **out_job, const uint8_t *ridx = nullptr, size_t n_palette = 0) {
+                            sasa_b200_job **out_job, const uint8_t *ridx = nullptr, size_t n_palette = 0,
+                            const uint32_t *group = nullptr, const sasa_b200_outputs *out_iso = nullptr) {
     sasa_b200_ctx *ctx = b->ctx;
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (!out || !out_job) return fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "out / out_job is NULL");
@@ -975,7 +1023,9 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
     if (rc) return rc;
     CU_TRY(ctx, cudaSetDevice(ctx->device));
     const size_t N = b->n_atoms, S = b->S, G = b->n_seg;
-    const int variant = id_class ? 1 : 0;
+    const bool grouped = out_iso != nullptr;   // sasa_b200_batch_run_groups_host: per-chunk pipeline only
+    const int variant = (id_class ? 1 : 0) + (grouped ? 4 : 0);
+    if (grouped && (rc = prepare_groups(b, group, params, out_iso, variant)) != 0) return rc;
     const bool indexed = xyz3 != nullptr && ridx != nullptr;   // 13 B/atom: coordinates + a palette index per atom
     const bool frames = xyz3 != nullptr;                       // any 12-byte coordinate form
     size_t fN = 0;  // atoms per frame (MD form) / palette entries (indexed form)
@@ -1008,6 +1058,11 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
     const size_t o_atom = o;   o += out->atom_sasa ? al(N * 4) : 0;
     const size_t o_seg = o;    o += (out->seg_sasa && G) ? al(G * 4) : 0;
     const size_t o_prot = o;   o += out->protein ? al(S * 12) : 0;
+    const size_t o_grp = o;    o += grouped ? al(N * 4) : 0;
+    const size_t o_icnt = o;   o += (grouped && out_iso->counts) ? al(N * 4) : 0;
+    const size_t o_iatom = o;  o += (grouped && out_iso->atom_sasa) ? al(N * 4) : 0;
+    const size_t o_iseg = o;   o += (grouped && out_iso->seg_sasa && G) ? al(G * 4) : 0;
+    const size_t o_iprot = o;  o += (grouped && out_iso->protein) ? al(S * 12) : 0;
     cudaStream_t s0 = ctx->streams[0];
     // the previous job may still be running on the sibling streams: this job's first stream starts behind all of them
     if (ctx->tail_valid)
@@ -1038,6 +1093,14 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
     ra.d_out.atom_sasa = out->atom_sasa ? reinterpret_cast<float *>(base_p + o_atom) : nullptr;
     ra.d_out.seg_sasa = (out->seg_sasa && G) ? reinterpret_cast<float *>(base_p + o_seg) : nullptr;
     ra.d_out.protein = out->protein ? reinterpret_cast<float *>(base_p + o_prot) : nullptr;
+    GroupParams gp{};
+    if (grouped) {
+        gp.grp = reinterpret_cast<const uint32_t *>(base_p + o_grp);
+        gp.counts = out_iso->counts ? reinterpret_cast<uint32_t *>(base_p + o_icnt) : nullptr;
+        gp.atom = out_iso->atom_sasa ? reinterpret_cast<float *>(base_p + o_iatom) : nullptr;
+        gp.seg = (out_iso->seg_sasa && G) ? reinterpret_cast<float *>(base_p + o_iseg) : nullptr;
+        gp.protein = out_iso->protein ? reinterpret_cast<float *>(base_p + o_iprot) : nullptr;
+    }
     // ---- gated single-launch pipeline ----------------------------------------------------------------------------------
     // Thirteen launches of 148 persistent CTAs cost the pipelined run 0.25 ms over the same work as ONE launch (CTA start-ups
     // with a cold first structure, per-chunk instead of batch-wide queue; DESIGN.md section 6).  When every chunk of the plan is one
@@ -1099,7 +1162,7 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
     static const bool trace_chunks = getenv("SASA_B200_TRACE_CHUNKS") != nullptr;
     std::vector<cudaEvent_t> trace_ev;
     // the large-structure workspace is shared by all chunks: keep such batches on a single stream
-    const int nstreams = b->max_large_v[variant] ? 1 : kStreams;
+    const int nstreams = b->max_large_v[variant] || (grouped && params->n_points > 128) ? 1 : kStreams;
     if (gated) {
         // the one kernel first (it starts at once and waits for chunk 0 at the gate), then the copies on the first stream
         uint32_t *d_ready = reinterpret_cast<uint32_t *>(reinterpret_cast<unsigned char *>(d_status) + 64);
@@ -1153,6 +1216,7 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
                 J_TRY(cudaMemcpyAsync(base_p + o_xyzr + ch.a0 * 16, xyzr + ch.a0 * 4, na * 16, cudaMemcpyHostToDevice, st));
             }
             if (id_class) J_TRY(cudaMemcpyAsync(base_p + o_cls + ch.a0 * 4, id_class + ch.a0, na * 4, cudaMemcpyHostToDevice, st));
+            if (grouped) J_TRY(cudaMemcpyAsync(base_p + o_grp + ch.a0 * 4, group + ch.a0, na * 4, cudaMemcpyHostToDevice, st));
         }
         if (trace_chunks) {
             cudaEvent_t e;
@@ -1160,7 +1224,7 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
             cudaEventRecord(e, st);
             trace_ev.push_back(e);
         }
-        if ((rc = enqueue_chunk(b, variant, ch, kbase, st, &job->launches)) != 0) return job_abort(ctx, job, rc);
+        if ((rc = enqueue_chunk(b, variant, ch, kbase, st, &job->launches, nullptr, grouped ? &gp : nullptr)) != 0) return job_abort(ctx, job, rc);
         if (trace_chunks) {
             cudaEvent_t e;
             cudaEventCreate(&e);
@@ -1176,6 +1240,17 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
         if (out->protein && ch.s1 > ch.s0)
             J_TRY(cudaMemcpyAsync(out->protein + 3 * (size_t)ch.s0, base_p + o_prot + 12 * (size_t)ch.s0,
                                   12 * (size_t)(ch.s1 - ch.s0), cudaMemcpyDeviceToHost, st));
+        if (grouped) {
+            if (na && out_iso->counts)
+                J_TRY(cudaMemcpyAsync(out_iso->counts + ch.a0, base_p + o_icnt + ch.a0 * 4, na * 4, cudaMemcpyDeviceToHost, st));
+            if (na && out_iso->atom_sasa)
+                J_TRY(cudaMemcpyAsync(out_iso->atom_sasa + ch.a0, base_p + o_iatom + ch.a0 * 4, na * 4, cudaMemcpyDeviceToHost, st));
+            if (out_iso->seg_sasa && ch.g1 > ch.g0)
+                J_TRY(cudaMemcpyAsync(out_iso->seg_sasa + ch.g0, base_p + o_iseg + ch.g0 * 4, (ch.g1 - ch.g0) * 4, cudaMemcpyDeviceToHost, st));
+            if (out_iso->protein && ch.s1 > ch.s0)
+                J_TRY(cudaMemcpyAsync(out_iso->protein + 3 * (size_t)ch.s0, base_p + o_iprot + 12 * (size_t)ch.s0,
+                                      12 * (size_t)(ch.s1 - ch.s0), cudaMemcpyDeviceToHost, st));
+        }
     }
     // join the sibling streams into the first one, read the status words back, free the arena in stream order
     for (int i = 1; i < kStreams; ++i) {
@@ -1281,6 +1356,17 @@ int sasa_b200_batch_run_indexed_host(sasa_b200_batch *b, const float *xyz, const
 
 int sasa_b200_job_wait(sasa_b200_job *job, sasa_b200_stats *stats) {
     if (!job || !job->active) return SASA_B200_ERR_INVALID_ARGUMENT;
+    return wait_job_impl(job, stats);
+}
+
+int sasa_b200_batch_run_groups_host(sasa_b200_batch *b, const float *xyzr, const uint32_t *id_class, const uint32_t *group,
+                                    const sasa_b200_params *params, const sasa_b200_outputs *out,
+                                    const sasa_b200_outputs *out_isolated, sasa_b200_stats *stats) {
+    if (!b) return SASA_B200_ERR_INVALID_ARGUMENT;
+    if (!out_isolated) return fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "out_isolated is NULL");
+    sasa_b200_job *job = nullptr;
+    int rc = submit_host_impl(b, xyzr, nullptr, nullptr, id_class, params, out, &job, nullptr, 0, group, out_isolated);
+    if (rc) return rc;
     return wait_job_impl(job, stats);
 }
 

@@ -79,6 +79,37 @@ struct KParams {
     unsigned long long *stat;     // [0] boundary points, [1] neighbour pairs, [2] streamed atoms
 };
 
+// Grouped runs (sasa_b200_batch_run_groups_*), a kernel argument of their own next to KParams: one group label per atom and the
+// outputs of every atom with its group standing alone (nullable each).
+struct GroupParams {
+    const uint32_t *grp;
+    uint32_t *counts;
+    float *atom, *seg, *protein;
+};
+
+// The run parameters with the isolated outputs in place of the complex ones (the output stages of grouped runs).
+__host__ __device__ __forceinline__ KParams iso_outputs(const KParams &p, const GroupParams &gp) {
+    KParams q = p;
+    q.out_counts = gp.counts;
+    q.out_atom = gp.atom;
+    q.out_seg = gp.seg;
+    q.out_protein = gp.protein;
+    return q;
+}
+
+// Atom accessor of an isolated evaluation: an atom of another group than `gi` reads as a far-away sentinel, so it fails every
+// distance test and never occludes -- the neighbour search and occlusion routines run unchanged on the group standing alone.
+template <bool GLOBAL>
+struct GroupAtoms {
+    const float4 *a;
+    const uint32_t *grp;
+    uint32_t gi;
+    __device__ __forceinline__ float4 operator()(int j) const {
+        const uint32_t gj = GLOBAL ? __ldg(grp + j) : grp[j];
+        return gj == gi ? (GLOBAL ? __ldg(a + j) : a[j]) : make_float4(1.0e18f, 1.0e18f, 1.0e18f, 0.0f);
+    }
+};
+
 struct Grid {
     float minx, miny, minz, inv_c;
     int nx, ny, nz, e;

@@ -41,6 +41,8 @@ struct LargeWorkspace {
     float4 *sorted = nullptr;
     uint32_t *orig = nullptr, *cellid = nullptr, *rank = nullptr, *cls_sorted = nullptr, *bstart = nullptr;
     float *val = nullptr;
+    uint32_t *grp_sorted = nullptr;   // grouped runs: group labels in cell-sorted order, per-atom areas with the group standing alone
+    float *val_iso = nullptr;
     // one allocation, zeroed by one memset per structure: header | tile states (u64) | cell counters
     unsigned char *zero_block = nullptr;
     LargeHeader *hdr = nullptr;
@@ -249,6 +251,15 @@ __global__ void __launch_bounds__(256) large_scatter_kernel(const float4 *__rest
         orig[at_pos] = (uint32_t)i;
         if (cls) cls_sorted[at_pos] = cls[i];
     }
+}
+
+// Grouped runs: the group labels into the cell-sorted order of large_scatter_kernel.
+__global__ void __launch_bounds__(256) large_scatter_groups_kernel(const uint32_t *__restrict__ grp, int N, const LargeHeader *h,
+                                                                   const uint32_t *cells, const uint32_t *cellid, const uint32_t *rank,
+                                                                   uint32_t *grp_sorted) {
+    if (h->ncell == 0) return;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < N; i += gridDim.x * blockDim.x)
+        grp_sorted[cells[cellid[i]] + rank[i]] = grp[i];
 }
 
 // Work block handed out by claim number t: rank r of n owns every n-th GROUP of kLGroup consecutive blocks, so each rank's
@@ -621,6 +632,97 @@ __global__ void __launch_bounds__(256, 2) large_atoms_kernel(const KParams p, in
     }
 }
 
+// One atom of the grouped atoms kernel with the list-based or streaming routines: neighbours cand[0, k) (k < 0: too many,
+// streamed).  Atoms: the plain accessor (complex) or GroupAtoms (isolated).
+template <class Atoms>
+__device__ __forceinline__ float large_eval_atom(const KParams &p, const Grid &g, const Atoms &atoms, const uint32_t *cells,
+                                                 const uint32_t *cls_sorted, int pos, const float4 ai, int k, uint32_t *cand,
+                                                 float4 *ent, const float4 *s_pts, unsigned long long &streamed) {
+    if (k >= 0) {
+        const float r = __fadd_rn(ai.w, p.probe);
+        const int nfront = build_entries(p, atoms, ai, __fmul_rn(r, r), __fmul_rn(2.0f, r), cand, k, ent);
+        return atom_fast(p, ent, k, nfront, reinterpret_cast<uint16_t *>(cand), s_pts);
+    }
+    streamed += 1;
+    return atom_streaming<Atoms, uint32_t, false>(p, g, atoms, cells, cls_sorted, pos, ent, nullptr);
+}
+
+// Atoms kernel of grouped runs: every atom in the complex and with its group standing alone.  n_points <= 128: one pass with
+// cap_atom_groups over the complex neighbour list; otherwise (and for atoms with more than kNbCap neighbours) two evaluations,
+// the second with the atoms of other groups hidden (GroupAtoms).  Writes val (complex areas) and val_iso.
+__global__ void __launch_bounds__(256, 2) large_groups_kernel(const KParams p, const GroupParams gp, int N, uint32_t a0, LargeHeader *h,
+                                                              const float4 *__restrict__ sorted, const uint32_t *__restrict__ orig,
+                                                              const uint32_t *__restrict__ cls_sorted, const uint32_t *__restrict__ grp_sorted,
+                                                              const uint32_t *__restrict__ cells, const uint32_t *__restrict__ bstart,
+                                                              float *val, float *val_iso, uint32_t blk) {
+    __shared__ __align__(16) float4 s_ent[8 * kNbCap];
+    __shared__ uint32_t s_cand[8 * kNbCap];
+    __shared__ __align__(16) float4 s_ptab[128];
+    if (h->ncell == 0) {
+        large_blank_outputs(p, N, a0);
+        large_blank_outputs(iso_outputs(p, gp), N, a0);
+        return;
+    }
+    const Grid g = h->grid;
+    const int lane = lane_id(), warp = threadIdx.x >> 5;
+    float4 *w_ent = s_ent + warp * kNbCap;
+    uint32_t *w_cand = s_cand + warp * kNbCap;
+    const GlobalAtoms atoms{sorted};
+    unsigned long long pairs = 0, streamed = 0;
+    const float4 *s_pts = p.n_points <= 128 ? s_ptab : nullptr;
+    const bool use_cap = p.cap != nullptr && p.n_points <= 128;
+    const int nbody = (int)min(p.n_points, p.n_body);
+    if (threadIdx.x < 128) {
+        const bool v = threadIdx.x < p.n_points;
+        s_ptab[threadIdx.x] = make_float4(v ? __ldg(p.px + threadIdx.x) : 0.f, v ? __ldg(p.py + threadIdx.x) : 0.f,
+                                          v ? __ldg(p.pz + threadIdx.x) : 0.f, 0.f);
+    }
+    __syncthreads();
+    const unsigned nblocks = ((unsigned)N + blk - 1) / blk;
+    CandCache<uint32_t> cc;
+    for (;;) {
+        unsigned b = 0;
+        if (lane == 0) b = atomicAdd(&h->next_block, 1u);
+        b = __shfl_sync(kFull, b, 0);
+        if (b >= nblocks) break;
+        cc.cell = -1;
+        cc.total = -1;
+        const int pend = (int)__ldg(bstart + b + 1);
+        for (int pos = (int)__ldg(bstart + b); pos < pend; ++pos) {
+            const float4 ai = atoms(pos);
+            const uint32_t gi = __ldg(grp_sorted + pos);
+            const int cx = cell_coord(ai.x, g.minx, g.inv_c, g.nx), cy = cell_coord(ai.y, g.miny, g.inv_c, g.ny),
+                      cz = cell_coord(ai.z, g.minz, g.inv_c, g.nz);
+            const int cid = (cz * g.ny + cy) * g.nx + cx;
+            if (cid != cc.cell) fill_cache(g, cells, cx, cy, cz, cid, cc);
+            const int k = cc.total >= 0 ? gather_cached(p, atoms, cls_sorted, pos, ai, cc, w_cand)
+                                        : gather_candidates(p, g, atoms, cells, cls_sorted, pos, ai, w_cand);
+            float cnt, cnt_iso;
+            if (k >= 0) pairs += (unsigned)k;
+            if (k >= 0 && use_cap) {
+                int iso;
+                cnt = (float)cap_atom_groups(p.cap, atoms, ai, p.probe, w_cand, k, grp_sorted, gi, s_ptab, (int)p.n_points, nbody, 0ull, &iso);
+                cnt_iso = (float)iso;
+            } else {
+                cnt = large_eval_atom(p, g, atoms, cells, cls_sorted, pos, ai, k, w_cand, w_ent, s_pts, streamed);
+                __syncwarp();
+                const GroupAtoms<true> iso_atoms{sorted, grp_sorted, gi};
+                const int k2 = cc.total >= 0 ? gather_cached(p, iso_atoms, cls_sorted, pos, ai, cc, w_cand)
+                                             : gather_candidates(p, g, iso_atoms, cells, cls_sorted, pos, ai, w_cand);
+                cnt_iso = large_eval_atom(p, g, iso_atoms, cells, cls_sorted, pos, ai, k2, w_cand, w_ent, s_pts, streamed);
+            }
+            const uint32_t oi = orig[pos];
+            large_store(p, lane, a0 + oi, oi, val, atom_area(ai.w, p.probe, cnt, p.inv_n), (uint32_t)cnt);
+            large_store(iso_outputs(p, gp), lane, a0 + oi, oi, val_iso, atom_area(ai.w, p.probe, cnt_iso, p.inv_n), (uint32_t)cnt_iso);
+            __syncwarp();
+        }
+    }
+    if (lane == 0 && p.stat) {
+        if (pairs) atomicAdd(p.stat + 1, pairs);
+        if (streamed) atomicAdd(p.stat + 2, streamed);
+    }
+}
+
 __device__ __forceinline__ float warp_sum_range(const float *v, uint32_t b, uint32_t e) {
     float t = 0.0f;
     for (uint32_t i = b + lane_id(); i < e; i += 32) t += v[i];
@@ -784,7 +886,7 @@ __global__ void __launch_bounds__(256) pack_indexed_kernel(const float *__restri
 
 inline void large_release(LargeWorkspace &w) {
     cudaFree(w.sorted); cudaFree(w.orig); cudaFree(w.cellid); cudaFree(w.rank); cudaFree(w.cls_sorted);
-    cudaFree(w.bstart); cudaFree(w.val); cudaFree(w.zero_block);
+    cudaFree(w.bstart); cudaFree(w.val); cudaFree(w.zero_block); cudaFree(w.grp_sorted); cudaFree(w.val_iso);
     w = LargeWorkspace{};
 }
 
@@ -798,6 +900,7 @@ inline int large_reserve(LargeWorkspace &w, uint32_t n_atoms) {
     if (cudaMalloc(&w.sorted, (size_t)n_atoms * 16) != cudaSuccess || cudaMalloc(&w.orig, (size_t)n_atoms * 4) != cudaSuccess ||
         cudaMalloc(&w.cellid, (size_t)n_atoms * 4) != cudaSuccess || cudaMalloc(&w.rank, (size_t)n_atoms * 4) != cudaSuccess ||
         cudaMalloc(&w.cls_sorted, (size_t)n_atoms * 4) != cudaSuccess || cudaMalloc(&w.val, (size_t)n_atoms * 4) != cudaSuccess ||
+        cudaMalloc(&w.grp_sorted, (size_t)n_atoms * 4) != cudaSuccess || cudaMalloc(&w.val_iso, (size_t)n_atoms * 4) != cudaSuccess ||
         cudaMalloc(&w.bstart, ((size_t)n_atoms + 2) * 4) != cudaSuccess ||
         cudaMalloc(&w.zero_block, sizeof(LargeHeader) + tiles_bytes + (want_cells + 2) * 4) != cudaSuccess) {
         large_release(w);
@@ -814,10 +917,11 @@ inline int large_reserve(LargeWorkspace &w, uint32_t n_atoms) {
 // Enqueue the whole pipeline for each large structure of one launch group: one memset + bounds, count, scan, scatter,
 // atoms (+ the level sums when asked for).  `order` / `off` are host arrays.  range_n > 1 selects the atom-range split
 // (BASELINE cfg5): the cell list is built for the whole structure, only the work blocks owned by `range_rank` are
-// evaluated, and no sums are produced.
+// evaluated, and no sums are produced.  Grouped runs (gp set; no atom-range split, no flags) go through
+// large_groups_kernel and produce the level sums of both value vectors.
 inline int large_enqueue(int sm_count, LargeWorkspace &w, const KParams &kp, const uint32_t *order, uint32_t n_work,
                          const uint32_t *off, const uint32_t *seg_off, cudaStream_t st, uint32_t *launches,
-                         uint32_t range_rank = 0, uint32_t range_n = 1) {
+                         uint32_t range_rank = 0, uint32_t range_n = 1, const GroupParams *gp = nullptr) {
     for (uint32_t q = 0; q < n_work; ++q) {
         const uint32_t sid = order[q];
         const uint32_t a0 = off[sid];
@@ -826,6 +930,7 @@ inline int large_enqueue(int sm_count, LargeWorkspace &w, const KParams &kp, con
         if ((uint32_t)N > w.cap_atoms) return 5;
         if (N == 0) {   // nothing to evaluate; the sums of an empty structure are zeros
             if (range_n == 1) large_enqueue_sums(sm_count, kp, sid, 0, seg_off ? seg_off[sid] : 0, nseg, w.val, nullptr, nullptr, 0, st, launches);
+            if (gp) large_enqueue_sums(sm_count, iso_outputs(kp, *gp), sid, 0, seg_off ? seg_off[sid] : 0, nseg, w.val_iso, nullptr, nullptr, 0, st, launches);
             continue;
         }
         const float4 *at = kp.xyzr + a0;
@@ -848,7 +953,13 @@ inline int large_enqueue(int sm_count, LargeWorkspace &w, const KParams &kp, con
         large_scan_kernel<<<gs, 256, 0, st>>>(w.hdr, w.cells, w.tiles, w.bstart, (uint32_t)N, blk);
         large_scatter_kernel<<<gc, 256, 0, st>>>(at, cls, N, w.hdr, w.cells, w.cellid, w.rank, w.sorted, w.orig, w.cls_sorted);
         const bool table = (kp.n_points <= 128 && kp.cap) || (kp.n_points > 128 && kp.n_points <= 1024 && kp.capm_in);
-        if (!cls && (kp.flags & 3u) == 0 && table) {
+        if (gp) {
+            large_scatter_groups_kernel<<<gc, 256, 0, st>>>(gp->grp + a0, N, w.hdr, w.cells, w.cellid, w.rank, w.grp_sorted);
+            const int ga = std::max(1, std::min((N + 8 * (int)blk - 1) / (8 * (int)blk), sm_count * 2));
+            large_groups_kernel<<<ga, 256, 0, st>>>(kp, *gp, N, a0, w.hdr, w.sorted, w.orig, cls ? w.cls_sorted : nullptr, w.grp_sorted, w.cells,
+                                                    w.bstart, w.val, w.val_iso, blk);
+            *launches += 1;
+        } else if (!cls && (kp.flags & 3u) == 0 && table) {
             const int ga = std::max(1, std::min((owned + 8 * (int)blk - 1) / (8 * (int)blk), sm_count * 4));
             // chunked tables are always laid out for eight chunks (the fused kernel shares them): one instantiation
 #define SASA_LARGE_CELLS(NCHP, TEX) large_cells_kernel<NCHP, TEX><<<ga, 256, 0, st>>>(kp, N, a0, w.hdr, w.sorted, w.orig, w.cells, w.bstart, w.val, range_rank, range_n, blk)
@@ -870,6 +981,9 @@ inline int large_enqueue(int sm_count, LargeWorkspace &w, const KParams &kp, con
         if (range_n == 1)
             large_enqueue_sums(sm_count, kp, sid, N, seg_off ? seg_off[sid] : 0, nseg, w.val, w.hdr, reinterpret_cast<float *>(w.rank),
                                w.cap_atoms, st, launches);
+        if (gp)
+            large_enqueue_sums(sm_count, iso_outputs(kp, *gp), sid, N, seg_off ? seg_off[sid] : 0, nseg, w.val_iso, w.hdr,
+                               reinterpret_cast<float *>(w.rank), w.cap_atoms, st, launches);
         if (cudaGetLastError() != cudaSuccess) return 2;
     }
     return 0;

@@ -28,9 +28,9 @@ struct SmemAtoms {
 // Shared-memory layout.  Everything the per-atom loops touch sits at compile-time offsets (given the warp
 // count), so no base pointer has to stay in a register: point table | per-warp entries | per-warp index
 // lists | per-warp cell candidate lists | reduction scratch | misc | atoms (+1 sentinel) | per-atom values |
-// [classes] | original indices | cell table.
+// [isolated values] | [classes] | [groups] | original indices | cell table.
 struct SmallLayout {
-    size_t pts, ent, cand, list, red, misc, atom, val, cls, orig, cellw, total;
+    size_t pts, ent, cand, list, red, misc, atom, val, val2, cls, grp, orig, cellw, total;
 };
 
 // Per-warp scratch is ONE contiguous block per warp -- entries | candidate lists | cell candidate list -- so that a single
@@ -44,7 +44,8 @@ __host__ __device__ constexpr size_t small_fixed_bytes(int nwarps) {
     return kOffWarpBlocks + (size_t)nwarps * kWarpBlockBytes + 32 * 8 * 4 + 64;
 }
 
-__host__ __device__ constexpr SmallLayout small_layout(uint32_t nmax, uint32_t cmax, int nwarps, bool has_cls) {
+// has_grp: grouped runs add the isolated values and the group labels (8 B per atom).
+__host__ __device__ constexpr SmallLayout small_layout(uint32_t nmax, uint32_t cmax, int nwarps, bool has_cls, bool has_grp = false) {
     SmallLayout L{};
     size_t o = 0;
     L.pts = o;   o += 128 * 16;
@@ -56,7 +57,9 @@ __host__ __device__ constexpr SmallLayout small_layout(uint32_t nmax, uint32_t c
     L.misc = o;  o += 64;
     L.atom = o;  o += ((size_t)nmax + 1) * 16;   // +1: the far-away sentinel atom the tight kernel pads its lists with
     L.val = o;   o += (size_t)nmax * 4;
+    L.val2 = o;  o += has_grp ? (size_t)nmax * 4 : 0;   // 16-byte aligned like val (seq_sum): nmax is a multiple of 16
     L.cls = o;   o += has_cls ? (size_t)nmax * 4 : 0;
+    L.grp = o;   o += has_grp ? (size_t)nmax * 4 : 0;
     L.orig = o;  o += (size_t)nmax * 2;
     o = (o + 3) & ~(size_t)3;
     L.cellw = o; o += (((size_t)cmax + 2 + 1) / 2) * 4;
@@ -72,11 +75,11 @@ __host__ __device__ constexpr size_t cta_budget(int minb) {
     return kSmemPerSM / (size_t)minb - kSmemCtaReserve < kSmemPerCtaMax ? kSmemPerSM / (size_t)minb - kSmemCtaReserve : kSmemPerCtaMax;
 }
 // Largest atom capacity (multiple of 16, < 65520 for the u16 indices) whose layout fits the budget of the configuration.
-__host__ __device__ constexpr uint32_t max_atoms(int nt, int minb, uint32_t cmax, bool has_cls) {
+__host__ __device__ constexpr uint32_t max_atoms(int nt, int minb, uint32_t cmax, bool has_cls, bool has_grp = false) {
     uint32_t lo = 0, hi = 65520 / 16 - 1;
     while (lo < hi) {
         const uint32_t mid = (lo + hi + 1) / 2;
-        if (small_layout(mid * 16, cmax, nt / 32, has_cls).total <= cta_budget(minb)) lo = mid;
+        if (small_layout(mid * 16, cmax, nt / 32, has_cls, has_grp).total <= cta_budget(minb)) lo = mid;
         else hi = mid - 1;
     }
     return lo * 16;
@@ -129,15 +132,17 @@ struct SmemView {
     float *val;         // per-atom exposed-point count, then area, by ORIGINAL index
     uint16_t *cellid, *rank;   // alias val during the counting sort
     uint32_t *cls;      // id classes in sorted order (HAS_CLS)
+    float *val2;        // grouped runs: per-atom values with the atom's group standing alone, by ORIGINAL index
+    uint32_t *grp;      // grouped runs: group labels in sorted order
     uint16_t *orig;     // sorted position -> original index
     uint32_t *cellw;    // cell table as u32 words (pairs of u16 counters) during counting
     uint16_t *cell;     // cell table: start position of every cell, cell[ncell] = N
 };
 
-template <int NT, bool HAS_CLS, uint32_t NMAX, uint32_t CMAX>
+template <int NT, bool HAS_CLS, uint32_t NMAX, uint32_t CMAX, bool HAS_GRP = false>
 __device__ __forceinline__ SmemView smem_view(unsigned char *smem) {
     constexpr int NW = NT / 32;
-    constexpr SmallLayout L = small_layout(NMAX, CMAX, NW, HAS_CLS);
+    constexpr SmallLayout L = small_layout(NMAX, CMAX, NW, HAS_CLS, HAS_GRP);
     SmemView v;
     v.ptab = reinterpret_cast<float4 *>(smem);
     v.atom = reinterpret_cast<float4 *>(smem + small_fixed_bytes(NW));
@@ -147,6 +152,8 @@ __device__ __forceinline__ SmemView smem_view(unsigned char *smem) {
     v.cellid = reinterpret_cast<uint16_t *>(smem + L.val);
     v.rank = v.cellid + NMAX;
     v.cls = HAS_CLS ? reinterpret_cast<uint32_t *>(smem + L.cls) : nullptr;
+    v.val2 = HAS_GRP ? reinterpret_cast<float *>(smem + L.val2) : nullptr;
+    v.grp = HAS_GRP ? reinterpret_cast<uint32_t *>(smem + L.grp) : nullptr;
     v.orig = reinterpret_cast<uint16_t *>(smem + L.orig);
     v.cellw = reinterpret_cast<uint32_t *>(smem + L.cellw);
     v.cell = reinterpret_cast<uint16_t *>(smem + L.cellw);
@@ -180,9 +187,9 @@ __device__ __forceinline__ Grid load_grid(const int *misc) {
 // block reduction), the cell grid, a counting sort with shared-memory atomics and the exclusive scan of the
 // cell counts.  Replaces SpatialGrid::new (src/structures/spatial_grid.rs:28-106).  Returns false when the
 // structure holds a non-finite value (outputs are then NaN-filled and the error flag raised).
-template <int NT, bool HAS_CLS, uint32_t CMAX>
+template <int NT, bool HAS_CLS, uint32_t CMAX, bool HAS_GRP = false>
 __device__ __forceinline__ bool structure_setup(const KParams &p, const SmemView &V, uint32_t sid, uint32_t a0, int N,
-                                                Grid &g, int &ncell) {
+                                                Grid &g, int &ncell, const GroupParams &gp = GroupParams{}) {
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     // ---- bounds, r_max, finiteness (maxima of {-min, max, r, bad}) -------------------------------------
     float red8[8] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY, -INFINITY, -INFINITY, 0.0f, 0.0f};
@@ -208,6 +215,15 @@ __device__ __forceinline__ bool structure_setup(const KParams &p, const SmemView
         if (p.seg_be && p.out_seg)
             for (uint32_t k = p.struct_seg_off[sid] + tid; k < p.struct_seg_off[sid + 1]; k += NT) p.out_seg[k] = qn;
         if (p.out_protein && tid < 3) p.out_protein[3 * (size_t)sid + tid] = qn;
+        if (HAS_GRP) {   // grouped run: the isolated outputs alike
+            for (int i = tid; i < N; i += NT) {
+                if (gp.counts) gp.counts[a0 + i] = 0u;
+                if (gp.atom) gp.atom[a0 + i] = qn;
+            }
+            if (p.seg_be && gp.seg)
+                for (uint32_t k = p.struct_seg_off[sid] + tid; k < p.struct_seg_off[sid + 1]; k += NT) gp.seg[k] = qn;
+            if (gp.protein && tid < 3) gp.protein[3 * (size_t)sid + tid] = qn;
+        }
         return false;
     }
     // ---- cell grid: cell edge >= half the largest possible pair cutoff, grown until it fits ----------------
@@ -270,6 +286,7 @@ __device__ __forceinline__ bool structure_setup(const KParams &p, const SmemView
         V.atom[at] = load_atom(p, a0, i);
         V.orig[at] = (uint16_t)i;
         if (HAS_CLS) V.cls[at] = p.cls[a0 + i];
+        if (HAS_GRP) V.grp[at] = gp.grp[a0 + i];
     }
     if (tid == 0) {
         V.misc[1] = 0;

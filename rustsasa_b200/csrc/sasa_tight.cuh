@@ -461,18 +461,17 @@ __device__ __forceinline__ int tight_atom(const KParams &p, const float4 *ent, i
 // forced a coarser grid) take the generic per-atom gather and the generic chunked evaluation; atoms with more
 // than kNbCap neighbours (denser than any protein) the list-free streaming routine.  Returns the exposed-point
 // count and adds the atom's list length to misc[6] (pairs), or 1 to misc[7] (streamed atoms).
-template <bool HAS_CLS>
-__device__ __noinline__ int tight_cold_atom(const float *px, const float *py, const float *pz, uint32_t n_points, uint32_t n_body,
-                                            float probe, float near2, int m_min, int m_max, Grid g, const float4 *s_atom,
-                                            const uint16_t *s_cell, const uint32_t *s_cls, const float4 *s_pts, int pos,
-                                            float4 *ent, uint16_t *cand, int *misc) {
+template <bool HAS_CLS, class Atoms>
+__device__ __forceinline__ int tight_cold_eval(const float *px, const float *py, const float *pz, uint32_t n_points, uint32_t n_body,
+                                               float probe, float near2, int m_min, int m_max, Grid g, const Atoms &atoms,
+                                               const uint16_t *s_cell, const uint32_t *s_cls, const float4 *s_pts, int pos,
+                                               float4 *ent, uint16_t *cand, int *misc) {
     KParams q;
     q.px = px; q.py = py; q.pz = pz;
     q.n_points = n_points; q.n_body = n_body; q.probe = probe;
     q.near2 = near2; q.m_min = m_min; q.m_max = m_max; q.bcast_min = 16;
-    const SmemAtoms atoms{s_atom};
     const uint32_t *cls = HAS_CLS ? s_cls : nullptr;
-    const float4 ai = s_atom[pos];
+    const float4 ai = atoms(pos);
     const int k = gather_candidates(q, g, atoms, s_cell, cls, pos, ai, cand);
     if (k >= 0) {
         const float r = __fadd_rn(ai.w, probe);
@@ -481,17 +480,36 @@ __device__ __noinline__ int tight_cold_atom(const float *px, const float *py, co
         return (int)atom_fast(q, ent, k, nfront, cand, s_pts);
     }
     if (lane_id() == 0) atomicAdd(&misc[7], 1);
-    return (int)atom_streaming<SmemAtoms, uint16_t, false>(q, g, atoms, s_cell, cls, pos, ent, nullptr);
+    return (int)atom_streaming<Atoms, uint16_t, false>(q, g, atoms, s_cell, cls, pos, ent, nullptr);
+}
+template <bool HAS_CLS>
+__device__ __noinline__ int tight_cold_atom(const float *px, const float *py, const float *pz, uint32_t n_points, uint32_t n_body,
+                                            float probe, float near2, int m_min, int m_max, Grid g, const float4 *s_atom,
+                                            const uint16_t *s_cell, const uint32_t *s_cls, const float4 *s_pts, int pos,
+                                            float4 *ent, uint16_t *cand, int *misc) {
+    return tight_cold_eval<HAS_CLS>(px, py, pz, n_points, n_body, probe, near2, m_min, m_max, g, SmemAtoms{s_atom}, s_cell, s_cls,
+                                    s_pts, pos, ent, cand, misc);
+}
+// The same with the atom's group standing alone (grouped runs): atoms of other groups are invisible.
+template <bool HAS_CLS>
+__device__ __noinline__ int tight_cold_atom_iso(const float *px, const float *py, const float *pz, uint32_t n_points, uint32_t n_body,
+                                                float probe, float near2, int m_min, int m_max, Grid g, const float4 *s_atom,
+                                                const uint32_t *s_grp, const uint16_t *s_cell, const uint32_t *s_cls,
+                                                const float4 *s_pts, int pos, float4 *ent, uint16_t *cand, int *misc) {
+    return tight_cold_eval<HAS_CLS>(px, py, pz, n_points, n_body, probe, near2, m_min, m_max, g, GroupAtoms<false>{s_atom, s_grp, s_grp[pos]},
+                                    s_cell, s_cls, s_pts, pos, ent, cand, misc);
 }
 
 // NSLT: number of 32-point body slots the kernel is compiled for (3 = the reference's default of 100 points on 8- and
 // 16-lane builds, 96 body points), or 0 to choose per launch among 1..4.
-template <int NT, int MINB, bool HAS_CLS, uint32_t CMAX, int NSLT>
-__global__ void __launch_bounds__(NT, MINB) sasa_tight_kernel(const KParams p) {
+// HAS_GRP: grouped run -- every atom is evaluated in the complex and with its group standing alone (the cap path in one pass,
+// cap_atom_groups; the cold path twice), and the output stage runs once per value array.
+template <int NT, int MINB, bool HAS_CLS, uint32_t CMAX, int NSLT, bool HAS_GRP>
+__device__ __forceinline__ void tight_kernel_body(const KParams &p, const GroupParams &gp) {
     extern __shared__ __align__(16) unsigned char smem[];
     constexpr int NW = NT / 32;
-    constexpr uint32_t NMAX = max_atoms(NT, MINB, CMAX, HAS_CLS);
-    const SmemView V = smem_view<NT, HAS_CLS, NMAX, CMAX>(smem);
+    constexpr uint32_t NMAX = max_atoms(NT, MINB, CMAX, HAS_CLS, HAS_GRP);
+    const SmemView V = smem_view<NT, HAS_CLS, NMAX, CMAX, HAS_GRP>(smem);
 #if SASA_OPT_UWARP
     const int lane = lane_id(), warp = uniform_i32((int)(threadIdx.x >> 5));
 #else
@@ -525,7 +543,7 @@ __global__ void __launch_bounds__(NT, MINB) sasa_tight_kernel(const KParams p) {
 #endif
         Grid g0;   // also parked in V.misc by the setup (load_grid)
         int ncell;
-        const bool ok = structure_setup<NT, HAS_CLS, CMAX>(p, V, sid, a0, N, g0, ncell);
+        const bool ok = structure_setup<NT, HAS_CLS, CMAX, HAS_GRP>(p, V, sid, a0, N, g0, ncell, gp);
 #if SASA_OPT_NEXT
         if (warp == 0) claim_next_and_prefetch(p, V.misc);   // every structure, also after a rejected one
 #endif
@@ -608,7 +626,7 @@ __global__ void __launch_bounds__(NT, MINB) sasa_tight_kernel(const KParams p) {
 #endif
                 const int total = tight_fill_list(g, V.cell, cx, cy, cz, w_list, N);
 #if SASA_OPT_PAIR && SASA_OPT_CAP
-                if (!HAS_CLS && total >= 0) {
+                if (!HAS_CLS && !HAS_GRP && total >= 0) {
                     uint16_t *const w_cand2 = w_nbb;   // the entry strip is idle on the cap path
                     uint16_t *const w_cand = w_nba;
                     while (pos + 1 < cell_end) {
@@ -635,10 +653,16 @@ __global__ void __launch_bounds__(NT, MINB) sasa_tight_kernel(const KParams p) {
 #endif
                     int k = total >= 0 ? tight_gather<HAS_CLS>(V.atom, V.cls, w_list, total, pos, ai, ai.w + reach0, w_nb)
                                        : kNbCap + 1;
+                    int cnt_iso = 0;
                     if (k <= kNbCap) {
 #if SASA_OPT_CAP
-                        cnt = cap_atom<SASA_CAP_TEX != 0>(p.cap, SmemAtoms{V.atom}, ai, p.probe, w_nb, k, V.ptab, (int)p.n_points, nbody, p.cap_tex);
+                        if (HAS_GRP)
+                            cnt = cap_atom_groups<SASA_CAP_TEX != 0>(p.cap, SmemAtoms{V.atom}, ai, p.probe, w_nb, k, V.grp, V.grp[pos], V.ptab,
+                                                                     (int)p.n_points, nbody, p.cap_tex, &cnt_iso);
+                        else
+                            cnt = cap_atom<SASA_CAP_TEX != 0>(p.cap, SmemAtoms{V.atom}, ai, p.probe, w_nb, k, V.ptab, (int)p.n_points, nbody, p.cap_tex);
 #else
+                        static_assert(!HAS_GRP, "grouped runs need the cap path");
                         const float r = __fadd_rn(ai.w, p.probe);
                         const int nfront = tight_entries(V.atom, ai, p.probe, __fmul_rn(r, r), __fmul_rn(2.0f, r), p.near2,
                                                          w_nb, k, w_ent);
@@ -652,9 +676,13 @@ __global__ void __launch_bounds__(NT, MINB) sasa_tight_kernel(const KParams p) {
                     } else {
                         cnt = tight_cold_atom<HAS_CLS>(p.px, p.py, p.pz, p.n_points, p.n_body, p.probe, p.near2, p.m_min, p.m_max,
                                                        g, V.atom, V.cell, V.cls, V.ptab, pos, w_ent, w_cand, V.misc);
+                        if (HAS_GRP)
+                            cnt_iso = tight_cold_atom_iso<HAS_CLS>(p.px, p.py, p.pz, p.n_points, p.n_body, p.probe, p.near2, p.m_min,
+                                                                   p.m_max, g, V.atom, V.grp, V.cell, V.cls, V.ptab, pos, w_ent, w_cand, V.misc);
                     }
                     if (lane == 0) {
                         const int oi = (int)V.orig[pos];
+                        if (HAS_GRP) V.val2[oi] = (float)cnt_iso;
 #if SASA_OPT_AREA
                         V.val[oi] = atom_area(ai.w, p.probe, (float)cnt, p.inv_n);
                         if (p.out_counts) p.out_counts[a0 + oi] = (uint32_t)cnt;
@@ -673,7 +701,25 @@ __global__ void __launch_bounds__(NT, MINB) sasa_tight_kernel(const KParams p) {
             if (V.misc[7]) atomicAdd(p.stat + 2, (unsigned long long)(unsigned)V.misc[7]);
         }
         structure_outputs<NT, SASA_OPT_AREA != 0>(p, V, sid, a0, N, smem + kOffWarpBlocks);
+        if (HAS_GRP) {
+            static_assert(!HAS_GRP || !SASA_OPT_AREA, "grouped runs store counts");
+            SmemView W = V;
+            W.val = V.val2;
+            __syncthreads();   // the output stage's scratch is refilled
+            structure_outputs<NT>(iso_outputs(p, gp), W, sid, a0, N, smem + kOffWarpBlocks);
+        }
     }
+}
+
+template <int NT, int MINB, bool HAS_CLS, uint32_t CMAX, int NSLT>
+__global__ void __launch_bounds__(NT, MINB) sasa_tight_kernel(const KParams p) {
+    tight_kernel_body<NT, MINB, HAS_CLS, CMAX, NSLT, false>(p, GroupParams{});
+}
+
+// Grouped runs (n_points <= 128): complex and isolated outputs of every structure in one pass.
+template <int NT, int MINB, bool HAS_CLS, uint32_t CMAX>
+__global__ void __launch_bounds__(NT, MINB) sasa_tight_groups_kernel(const KParams p, const GroupParams gp) {
+    tight_kernel_body<NT, MINB, HAS_CLS, CMAX, 0, true>(p, gp);
 }
 
 }  // namespace sasa

@@ -261,6 +261,51 @@ class Batch:
         self.engine._check(self._L.sasa_b200_batch_run_device(self._h, _ptr(d_xyzr), _ptr(d_id_class), C.byref(prm),
                                                              C.byref(outs), _stream(stream)))
 
+    def run_groups_host(self, xyzr, group, id_class=None, probe_radius=1.4, n_points=100, simd_lanes=8, flags=0,
+                        want=("counts", "atom", "seg", "protein")):
+        """Grouped run (buried surface area): one label per atom in `group`.  Returns (complex, isolated) BatchResults: the
+        complex is what run_host gives; isolated is every atom with its group standing alone (only same-group neighbours
+        occlude).  Buried area = isolated - complex."""
+        xyzr = _np(xyzr, np.float32, (-1, 4))
+        assert xyzr.shape[0] == self.n_atoms, "xyzr does not match struct_off"
+        group = _np(group, np.uint32)
+        assert group is None or group.shape[0] == self.n_atoms, "group does not match struct_off"
+        id_class = _np(id_class, np.uint32)
+        cpx, iso = self._host_outputs(want, "numpy"), self._host_outputs(want, "numpy")
+        outs = [_lib.Outputs(_ptr(r.counts), _ptr(r.atom_sasa), _ptr(r.seg_sasa), _ptr(r.protein)) for r in (cpx, iso)]
+        prm = self._params(probe_radius, n_points, simd_lanes, flags)
+        st = _lib.Stats()
+        self.engine._check(self._L.sasa_b200_batch_run_groups_host(self._h, _ptr(xyzr), _ptr(id_class), _ptr(group), C.byref(prm),
+                                                                  C.byref(outs[0]), C.byref(outs[1]), C.byref(st)))
+        cpx.stats = iso.stats = st.as_dict()
+        return cpx, iso
+
+    def run_groups_device(self, d_xyzr, d_group, d_id_class=None, probe_radius=1.4, n_points=100, simd_lanes=8, flags=0,
+                          want=("counts", "atom", "seg", "protein"), stream=None):
+        """run_groups_host on torch CUDA tensors: allocates the outputs on the input's device, enqueues on `stream` (None =
+        torch's current stream) and returns (complex, isolated) BatchResults of tensors without synchronising."""
+        import torch
+        dev = d_xyzr.device
+
+        def outputs():
+            r = BatchResult()
+            if "counts" in want:
+                r.counts = torch.zeros(self.n_atoms, dtype=torch.int32, device=dev)
+            if "atom" in want:
+                r.atom_sasa = torch.zeros(self.n_atoms, dtype=torch.float32, device=dev)
+            if "seg" in want and self.n_seg:
+                r.seg_sasa = torch.zeros(self.n_seg, dtype=torch.float32, device=dev)
+            if "protein" in want:
+                r.protein = torch.zeros((max(self.S, 0), 3), dtype=torch.float32, device=dev)
+            return r
+        cpx, iso = outputs(), outputs()
+        outs = [_lib.Outputs(_ptr(r.counts), _ptr(r.atom_sasa), _ptr(r.seg_sasa), _ptr(r.protein)) for r in (cpx, iso)]
+        prm = self._params(probe_radius, n_points, simd_lanes, flags)
+        self.engine._check(self._L.sasa_b200_batch_run_groups_device(self._h, _ptr(d_xyzr), _ptr(d_id_class), _ptr(d_group),
+                                                                    C.byref(prm), C.byref(outs[0]), C.byref(outs[1]),
+                                                                    _stream(stream)))
+        return cpx, iso
+
     def run_atom_range_device(self, d_xyzr, rank: int, n_ranks: int, d_id_class=None, probe_radius=1.4, n_points=100,
                               simd_lanes=8, counts=None, atom_sasa=None, stream=None):
         """Atom-range split (cfg5): slice `rank` of `n_ranks` of every structure's cell-sorted atom order; the

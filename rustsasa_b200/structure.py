@@ -372,6 +372,7 @@ class PackedStructure:
     seg_be: np.ndarray          # (n_seg, 2) uint32 [begin, end) atom ranges, relative to atom 0
     seg_polar: np.ndarray       # (n_seg,) uint8, residue-level polar flag
     seg_meta: list              # per segment: dict of the host-side result fields
+    atom_chain: Optional[np.ndarray] = None   # (N,) chain id of every atom (str), the key of grouped runs
 
 
 def build_atoms_and_mapping(st: Structure, level: str = "residue", radii_config=None, allow_vdw_fallback=False,
@@ -385,10 +386,11 @@ def build_atoms_and_mapping(st: Structure, level: str = "residue", radii_config=
     """
     xyzr: List[Tuple[float, float, float, float]] = []
     ids: List[int] = []
+    atom_chain: List[str] = []
     key_to_range: Dict[object, Tuple[int, int]] = {}
     order: List[Tuple[object, dict]] = []
 
-    def push(atom: AtomRec, resname: str, altloc: str) -> bool:
+    def push(atom: AtomRec, resname: str, altloc: str, chain_id: str) -> bool:
         if atom.element is None:
             raise SASACalcError("ElementMissing", "Element missing for atom")
         if atom.element == "H" and not include_hydrogens:
@@ -412,17 +414,19 @@ def build_atoms_and_mapping(st: Structure, level: str = "residue", radii_config=
         xyzr.append((np.float32(atom.x), np.float32(atom.y), np.float32(atom.z), radius))
         # id = FNV(altloc, serial): only equality is observable, so a tuple hash stands in.
         ids.append(hash((altloc, atom.serial)) & 0xFFFFFFFFFFFFFFFF)
+        atom_chain.append(chain_id)
         return True
 
     if level == "atom":
-        for res in st.residues():
-            resname = res.name()
-            if resname is None:
-                raise SASACalcError("FailedToGetResidueName", "Failed to get residue name")
-            if res.conformers:
-                conf = res.conformers[0]
-                for a in conf.atoms:
-                    push(a, resname, conf.altloc or "")
+        for chain in st.chains():   # (st.residues() order)
+            for res in chain.residues.values():
+                resname = res.name()
+                if resname is None:
+                    raise SASACalcError("FailedToGetResidueName", "Failed to get residue name")
+                if res.conformers:
+                    conf = res.conformers[0]
+                    for a in conf.atoms:
+                        push(a, resname, conf.altloc or "", chain.id)
     else:
         for chain in st.chains():
             chain_key = serialize_chain_id(chain.id)
@@ -435,7 +439,7 @@ def build_atoms_and_mapping(st: Structure, level: str = "residue", radii_config=
                 if res.conformers:
                     conf = res.conformers[0]
                     for a in conf.atoms:
-                        push(a, resname, "" if level == "protein" else (conf.altloc or ""))
+                        push(a, resname, "" if level == "protein" else (conf.altloc or ""), chain.id)
                     if level in ("residue", "protein"):
                         key_to_range[(chain.id, res.serial, res.icode or "")] = (begin, len(xyzr))
                 if level in ("residue", "protein"):
@@ -456,4 +460,4 @@ def build_atoms_and_mapping(st: Structure, level: str = "residue", radii_config=
         seg_polar[k] = 1 if m.get("is_polar") else 0
         meta.append(m)
     arr = np.asarray(xyzr, dtype=np.float32).reshape(-1, 4)
-    return PackedStructure(arr, np.asarray(ids, dtype=np.uint64), seg_be, seg_polar, meta)
+    return PackedStructure(arr, np.asarray(ids, dtype=np.uint64), seg_be, seg_polar, meta, np.asarray(atom_chain, dtype=object))
