@@ -190,6 +190,22 @@ SASA_B200_API int sasa_b200_batch_run_groups_device(sasa_b200_batch *batch, cons
                                       const uint32_t *d_group, const sasa_b200_params *params, const sasa_b200_outputs *d_out,
                                       const sasa_b200_outputs *d_out_isolated, void *stream);
 
+/* Exposed-point masks: which sphere points of every atom are solvent-accessible (the dot surface), from the same pass as the
+ * counts.  exposed holds W = (n_points + 31) / 32 u32 words per atom, atoms in batch order (the indexing of counts): bit b of
+ * word w of atom i is set exactly when point 32 w + b -- in the order of sasa_b200_sphere_points -- is exposed; bits at or
+ * above n_points are zero, and the popcount of atom i's row equals counts[i].  out / d_out are bit for bit what
+ * sasa_b200_batch_run_host / _device give for the same input (every field nullable); every n_points, simd_lanes, id_class and
+ * flag the plain run accepts is accepted.  exposed == NULL with atoms in the batch, or a buffer size (n_atoms * W * 4 bytes)
+ * that overflows size_t: SASA_B200_ERR_INVALID_ARGUMENT.  Non-finite input: SASA_B200_ERR_NON_FINITE with zero mask rows for
+ * that structure.  The host form uses the per-chunk pipeline; the device form behaves like sasa_b200_batch_run_device
+ * (stream-ordered, errors via sasa_b200_batch_sync). */
+SASA_B200_API int sasa_b200_batch_run_masks_host(sasa_b200_batch *batch, const float *xyzr, const uint32_t *id_class,
+                                   const sasa_b200_params *params, const sasa_b200_outputs *out,
+                                   uint32_t *exposed, sasa_b200_stats *stats /* nullable */);
+SASA_B200_API int sasa_b200_batch_run_masks_device(sasa_b200_batch *batch, const float *d_xyzr, const uint32_t *d_id_class,
+                                     const sasa_b200_params *params, const sasa_b200_outputs *d_out,
+                                     uint32_t *d_exposed, void *stream);
+
 /* MD-trajectory form (what mdsasa-bolt feeds calculate_sasa_internal per frame): a batch
  * created with S = n_frames equal-sized structures; xyz holds n_frames * n_atoms_per_frame
  * * 3 floats, radii n_atoms_per_frame floats shared by every frame (12 B/atom/frame on the

@@ -6,10 +6,12 @@ Engine / Batch wrapper (``engine``) and a mirror of the reference's public inter
 (``api``: ``calculate_sasa_internal``, ``SASAOptions`` ...).  There is no CPU fallback.
 """
 from .api import (Atom, AtomLevel, ChainLevel, ChainResult, ProteinLevel, ProteinResult, ResidueLevel,  # noqa: F401
-                  ResidueResult, SASACalcError, SASAOptions, calculate_sasa_internal, default_engine)
+                  ResidueResult, SASACalcError, SASAOptions, SurfaceResult, calculate_sasa_internal, default_engine,
+                  surface_points)
 from .engine import Batch, BatchResult, Engine, SasaB200Error  # noqa: F401
 from .structure import read_structure  # noqa: F401
 
 __all__ = ["Atom", "AtomLevel", "ResidueLevel", "ChainLevel", "ProteinLevel", "ChainResult", "ResidueResult",
-           "ProteinResult", "SASACalcError", "SASAOptions", "calculate_sasa_internal", "default_engine", "Engine",
+           "ProteinResult", "SASACalcError", "SASAOptions", "SurfaceResult", "calculate_sasa_internal", "default_engine",
+           "surface_points", "Engine",
            "Batch", "BatchResult", "SasaB200Error", "read_structure"]

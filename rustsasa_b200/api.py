@@ -12,7 +12,8 @@ Same names, argument meaning and error behaviour as the crate (rust-sasa 0.9.2):
 The numeric core is the C ABI (include/sasa_b200.h); there is no CPU path here.
 ``process_many`` is the batched form the CLI's directory mode (src/main.rs:342-480) maps onto.
 ``process_interface`` adds buried surface area: every structure in the complex and with each chain group standing alone,
-from one grouped batch call.
+from one grouped batch call.  ``process_surface`` and ``surface_points`` give the dot surface: the solvent-accessible test
+points themselves, from the exposed-point masks of the same batch call.
 """
 from __future__ import annotations
 
@@ -76,6 +77,15 @@ class InterfaceResult:
     buried_area: float
 
 
+@dataclass
+class SurfaceResult:
+    """One structure of ``SASAOptions.process_surface``: the level's result, the exposed test points (M, 3) float32 and for
+    each point the index of its atom in the order of an atom-level result (M,) int64."""
+    result: Any
+    points: np.ndarray
+    atom_index: np.ndarray
+
+
 class AtomLevel:
     name = "atom"
 
@@ -105,6 +115,20 @@ def calculate_sasa_internal(atoms, probe_radius: float = 1.4, n_points: int = 10
     xyzr = np.array([[a.position[0], a.position[1], a.position[2], a.radius] for a in atoms], dtype=np.float32)
     ids = np.array([a.id & 0xFFFFFFFFFFFFFFFF for a in atoms], dtype=np.uint64)
     return eng.calculate_sasa_internal(xyzr, ids, probe_radius, n_points, threads)
+
+
+def surface_points(xyzr, exposed, n_points: int, probe_radius: float = 1.4):
+    """The dot surface from exposed-point masks: for every set bit b of word w of atom i (``Batch.run_masks_host``'s
+    ``exposed``, (N, W) uint32) the point centre_i + (r_i + probe) * p_(32 w + b), in float32 with the engine's sphere points.
+    Returns (points (M, 3) float32, atom (M,) int64), atom-major and in point order within an atom."""
+    xyzr = np.ascontiguousarray(xyzr, np.float32).reshape(-1, 4)
+    exposed = np.ascontiguousarray(exposed, np.uint32).reshape(xyzr.shape[0], -1)
+    bits = np.unpackbits(exposed.view(np.uint8), axis=1, bitorder="little")[:, :n_points]
+    atom, k = np.nonzero(bits)
+    sphere = Engine.sphere_points(n_points)
+    r = xyzr[atom, 3] + np.float32(probe_radius)
+    points = xyzr[atom, :3] + r[:, None] * sphere[k]
+    return points.astype(np.float32, copy=False), atom.astype(np.int64)
 
 
 def _dense_classes(ids: np.ndarray) -> Optional[np.ndarray]:
@@ -165,6 +189,12 @@ class SASAOptions:
         src/main.rs:447-453)."""
         return self._run_many(structures, engine, None)
 
+    def process_surface(self, structures: Sequence[Structure], engine: Optional[Engine] = None) -> List:
+        """The dot surface: per structure a :class:`SurfaceResult` with the level's result and the solvent-accessible test
+        points, both from ONE batch call with exposed-point masks.  A structure whose extraction fails is reported as its
+        ``SASACalcError``, as in ``process_many``."""
+        return self._run_many(structures, engine, None, surface=True)
+
     def process_interface(self, structures: Sequence[Structure], chain_groups: Optional[Sequence[str]] = None,
                           engine: Optional[Engine] = None) -> List:
         """Buried surface area: per structure an :class:`InterfaceResult` with the level's result in the complex and
@@ -188,7 +218,8 @@ class SASAOptions:
             out[i] = label[c]
         return out
 
-    def _run_many(self, structures: Sequence[Structure], engine: Optional[Engine], chain_groups: Optional[List[str]]) -> List:
+    def _run_many(self, structures: Sequence[Structure], engine: Optional[Engine], chain_groups: Optional[List[str]],
+                  surface: bool = False) -> List:
         eng = engine or default_engine()
         packed: List[Optional[PackedStructure]] = []
         results: List = [None] * len(structures)
@@ -220,7 +251,9 @@ class SASAOptions:
         batch = Batch(eng, struct_off, seg_be if seg_be.shape[0] else None, seg_off if seg_be.shape[0] else None,
                       polar if seg_be.shape[0] else None)
         try:
-            if chain_groups is None:
+            if surface:
+                res = batch.run_masks_host(xyzr, id_class, self.probe_radius, self.n_points, want=want)
+            elif chain_groups is None:
                 res = batch.run_host(xyzr, id_class, self.probe_radius, self.n_points, want=want)
             else:   # the protein totals give the buried area: always requested
                 group = np.concatenate([self._chain_groups(packed[i].atom_chain, chain_groups) for i in good])
@@ -245,7 +278,11 @@ class SASAOptions:
             return ProteinResult(float(t[0]), float(t[1]), float(t[2]))
 
         for k, i in enumerate(good):
-            if chain_groups is None:
+            if surface:
+                a0, a1 = int(struct_off[k]), int(struct_off[k + 1])
+                pts, atom = surface_points(xyzr[a0:a1], res.exposed[a0:a1], self.n_points, self.probe_radius)
+                results[i] = SurfaceResult(level_result(res, k, packed[i]), pts, atom)
+            elif chain_groups is None:
                 results[i] = level_result(res, k, packed[i])
             else:
                 results[i] = InterfaceResult(level_result(cpx, k, packed[i]), level_result(iso, k, packed[i]),

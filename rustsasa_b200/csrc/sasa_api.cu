@@ -115,7 +115,7 @@ struct sasa_b200_ctx {
     LargeWorkspace large;
     cudaEvent_t ev_large = nullptr;
     bool large_used = false;
-    bool attr_done[8][8] = {};   // [kernel configuration][instantiation]: shared-memory attribute set (at first launch)
+    bool attr_done[8][12] = {};  // [kernel configuration][instantiation]: shared-memory attribute set (at first launch)
     // jobs: one per host-buffer run in flight (submit / wait); recycled, so events and the pinned status word are made once
     std::vector<sasa_b200_job *> free_jobs;
     cudaEvent_t ev_tail[kStreams] = {};   // end of the previous job on each copy stream (the next job's first stream waits on them)
@@ -223,6 +223,7 @@ int get_points(sasa_b200_ctx *ctx, uint32_t n, const Points **out) {
 // per-CTA budget that lets `minb` CTAs share one SM (228 KB per SM, 1 KB reserved per CTA, 227 KB per CTA max).
 typedef void (*SmallKernel)(const KParams);
 typedef void (*GroupKernel)(const KParams, const GroupParams);
+typedef void (*MaskKernel)(const KParams, const MaskParams);
 struct Proto {
     int nt, minb;
     uint32_t cmax;
@@ -230,6 +231,7 @@ struct Proto {
     SmallKernel fn[6];   // index = has_cls + 2 * tight (tight: n_points <= 128, no statistics / forced streaming)
                          //         + 2 more when the tight kernel compiled for 3 body slots applies (65..96 body points)
     GroupKernel fng[2];  // grouped runs (n_points <= 128), index = has_cls
+    MaskKernel fnm[4];   // exposed-point masks, index = has_cls + 2 * tight (same shared memory as the plain kernels)
 };
 #define SASA_PROTO(NT, MINB, CMAX)                                                                                     \
     Proto { NT, MINB, CMAX, { max_atoms(NT, MINB, CMAX, false), max_atoms(NT, MINB, CMAX, true),                       \
@@ -237,7 +239,9 @@ struct Proto {
             { sasa_small_kernel<NT, MINB, false, CMAX>, sasa_small_kernel<NT, MINB, true, CMAX>,                       \
               sasa_tight_kernel<NT, MINB, false, CMAX, 0>, sasa_tight_kernel<NT, MINB, true, CMAX, 0>,                 \
               sasa_tight_kernel<NT, MINB, false, CMAX, 3>, sasa_tight_kernel<NT, MINB, true, CMAX, 3> },               \
-            { sasa_tight_groups_kernel<NT, MINB, false, CMAX>, sasa_tight_groups_kernel<NT, MINB, true, CMAX> } }
+            { sasa_tight_groups_kernel<NT, MINB, false, CMAX>, sasa_tight_groups_kernel<NT, MINB, true, CMAX> },           \
+            { sasa_small_masks_kernel<NT, MINB, false, CMAX>, sasa_small_masks_kernel<NT, MINB, true, CMAX>,               \
+              sasa_tight_masks_kernel<NT, MINB, false, CMAX>, sasa_tight_masks_kernel<NT, MINB, true, CMAX> } }
 // 0-2 keep 32 warps resident per SM (64 registers/thread); 3-4 keep 24 warps (85 registers/thread)
 #ifndef SASA_ALL_PROTOS   // the shipped build instantiates the two default configurations only (half the build time and library
                          // size); -DSASA_ALL_PROTOS adds the three tuning configurations selectable with SASA_B200_CFGS
@@ -557,9 +561,10 @@ int check_params(sasa_b200_ctx *ctx, const sasa_b200_params *p) {
 // Enqueue every kernel of one chunk: the first fused launch on `st`, the others on sibling streams forked from and
 // joined back into `st` (so the caller still sees one stream-ordered unit of work).  Large-structure pipelines stay
 // on `st`.
-// gp: grouped runs (group labels and isolated outputs), else null.
+// gp: grouped runs (group labels and isolated outputs), else null.  mp: exposed-point masks, else null.
 int enqueue_chunk(sasa_b200_batch *b, int variant, const Chunk &ch, const KParams &base, cudaStream_t st,
-                  uint32_t *launches, const uint32_t *order_override = nullptr, const GroupParams *gp = nullptr) {
+                  uint32_t *launches, const uint32_t *order_override = nullptr, const GroupParams *gp = nullptr,
+                  const MaskParams *mp = nullptr) {
     sasa_b200_ctx *ctx = b->ctx;
     int n_small = 0;
     for (const Launch &L : ch.launches) n_small += L.cfg >= 0;
@@ -579,7 +584,7 @@ int enqueue_chunk(sasa_b200_batch *b, int variant, const Chunk &ch, const KParam
         if (L.cfg < 0 || all_large) {
             if (ctx->large_used) CU_TRY(ctx, cudaStreamWaitEvent(st, ctx->ev_large, 0));
             int rc = large_enqueue(ctx->sm_count, ctx->large, kp, &b->h_order[variant][L.order_off], L.n_work,
-                                   b->h_off.data(), b->h_seg_off.empty() ? nullptr : b->h_seg_off.data(), st, launches, 0, 1, gp);
+                                   b->h_off.data(), b->h_seg_off.empty() ? nullptr : b->h_seg_off.data(), st, launches, 0, 1, gp, mp);
             if (rc != 0) return fail(ctx, rc, "large-structure path failed: %s", cudaGetErrorString(cudaGetLastError()));
             CU_TRY(ctx, cudaEventRecord(ctx->ev_large, st));
             ctx->large_used = true;
@@ -596,12 +601,17 @@ int enqueue_chunk(sasa_b200_batch *b, int variant, const Chunk &ch, const KParam
             ls = ctx->side[small_idx - 1];
             CU_TRY(ctx, cudaStreamWaitEvent(ls, ctx->ev_fork, 0));
         }
-        void *args[] = {(void *)&kp, (void *)gp};
+        void *args[] = {(void *)&kp, mp ? (void *)mp : (void *)gp};
         const bool tight = kp.n_points <= 128 && (kp.flags & 3u) == 0;
         const uint32_t body = std::min(kp.n_points, kp.n_body);
-        // (attribute slots 6 / 7: the grouped kernels)
-        const int which = grouped ? 6 + (has_cls ? 1 : 0) : (has_cls ? 1 : 0) + (tight ? (SASA_OPT_NSLT && body > 64 && body <= 96 ? 4 : 2) : 0);
-        const void *fn = grouped ? (const void *)kProtos[c.proto].fng[has_cls ? 1 : 0] : (const void *)kProtos[c.proto].fn[which];
+        // (attribute slots 6 / 7: the grouped kernels; 8-11: the masked kernels)
+        const int mwhich = (has_cls ? 1 : 0) + (tight ? 2 : 0);
+        const int which = grouped ? 6 + (has_cls ? 1 : 0)
+                          : mp    ? 8 + mwhich
+                                  : (has_cls ? 1 : 0) + (tight ? (SASA_OPT_NSLT && body > 64 && body <= 96 ? 4 : 2) : 0);
+        const void *fn = grouped ? (const void *)kProtos[c.proto].fng[has_cls ? 1 : 0]
+                         : mp    ? (const void *)kProtos[c.proto].fnm[mwhich]
+                                 : (const void *)kProtos[c.proto].fn[which];
         if (!ctx->attr_done[c.proto][which]) {
             cudaError_t ea = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
             if (ea != cudaSuccess)
@@ -915,14 +925,27 @@ static int prepare_groups(sasa_b200_batch *b, const uint32_t *group, const sasa_
     return SASA_B200_OK;
 }
 
+// Checks of the masked entry points (after check_params): a mask buffer for every atom whose size fits a size_t.
+static int check_masks(sasa_b200_batch *b, const uint32_t *exposed, const sasa_b200_params *params) {
+    if (!exposed && b->n_atoms) return fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "exposed is NULL");
+    if (b->n_atoms && mask_words(params->n_points) > SIZE_MAX / 4 / b->n_atoms)
+        return fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "the mask buffer (%zu atoms x %u words) overflows size_t", b->n_atoms,
+                    mask_words(params->n_points));
+    return SASA_B200_OK;
+}
+
+// d_iso: grouped runs; masked: d_exposed receives the exposed-point masks (one of the two at most).
 static int run_device_impl(sasa_b200_batch *b, const float *d_xyzr, const uint32_t *d_id_class, const uint32_t *d_group,
-                           const sasa_b200_params *params, const sasa_b200_outputs *d_out, const sasa_b200_outputs *d_iso, void *stream) {
+                           const sasa_b200_params *params, const sasa_b200_outputs *d_out, const sasa_b200_outputs *d_iso, void *stream,
+                           bool masked = false, uint32_t *d_exposed = nullptr) {
     if (!b) return SASA_B200_ERR_INVALID_ARGUMENT;
     sasa_b200_ctx *ctx = b->ctx;
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (!d_out || (!d_xyzr && b->n_atoms)) return fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "d_xyzr / d_out is NULL");
     int rc = check_params(ctx, params);
     if (rc) return rc;
+    if (masked && (rc = check_masks(b, d_exposed, params)) != 0) return rc;
+    const MaskParams mp{d_exposed};
     const bool grouped = d_iso != nullptr;
     const int variant = (d_id_class ? 1 : 0) + 2 + (grouped ? 4 : 0);
     CU_TRY(ctx, cudaSetDevice(ctx->device));
@@ -942,7 +965,8 @@ static int run_device_impl(sasa_b200_batch *b, const float *d_xyzr, const uint32
     if (b->n_counters[variant])
         CU_TRY(ctx, cudaMemsetAsync(b->d_counters, 0, b->n_counters[variant] * sizeof(uint32_t), st));
     for (const Chunk &ch : b->plan[variant])
-        if ((rc = enqueue_chunk(b, variant, ch, base, st, &b->launches_last, nullptr, grouped ? &gp : nullptr)) != 0) return rc;
+        if ((rc = enqueue_chunk(b, variant, ch, base, st, &b->launches_last, nullptr, grouped ? &gp : nullptr, masked ? &mp : nullptr)) != 0)
+            return rc;
     return SASA_B200_OK;
 }
 
@@ -956,6 +980,11 @@ int sasa_b200_batch_run_groups_device(sasa_b200_batch *b, const float *d_xyzr, c
                                       const sasa_b200_outputs *d_out_isolated, void *stream) {
     if (b && !d_out_isolated) return fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "d_out_isolated is NULL");
     return run_device_impl(b, d_xyzr, d_id_class, d_group, params, d_out, d_out_isolated, stream);
+}
+
+int sasa_b200_batch_run_masks_device(sasa_b200_batch *b, const float *d_xyzr, const uint32_t *d_id_class, const sasa_b200_params *params,
+                                     const sasa_b200_outputs *d_out, uint32_t *d_exposed, void *stream) {
+    return run_device_impl(b, d_xyzr, d_id_class, nullptr, params, d_out, nullptr, stream, true, d_exposed);
 }
 
 int sasa_b200_batch_sync(sasa_b200_batch *b, sasa_b200_stats *stats) {
@@ -1012,7 +1041,8 @@ static int job_abort(sasa_b200_ctx *ctx, sasa_b200_job *j, int rc) {
 static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *xyz3, const float *radii,
                             const uint32_t *id_class, const sasa_b200_params *params, const sasa_b200_outputs *out,
                             sasa_b200_job **out_job, const uint8_t *ridx = nullptr, size_t n_palette = 0,
-                            const uint32_t *group = nullptr, const sasa_b200_outputs *out_iso = nullptr) {
+                            const uint32_t *group = nullptr, const sasa_b200_outputs *out_iso = nullptr, bool masked = false,
+                            uint32_t *exposed = nullptr) {
     sasa_b200_ctx *ctx = b->ctx;
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (!out || !out_job) return fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "out / out_job is NULL");
@@ -1021,8 +1051,10 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
     if (b->in_flight) return fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "this batch already has a run in flight: wait for it first");
     int rc = check_params(ctx, params);
     if (rc) return rc;
+    if (masked && (rc = check_masks(b, exposed, params)) != 0) return rc;
     CU_TRY(ctx, cudaSetDevice(ctx->device));
     const size_t N = b->n_atoms, S = b->S, G = b->n_seg;
+    const size_t W = mask_words(params->n_points);
     const bool grouped = out_iso != nullptr;   // sasa_b200_batch_run_groups_host: per-chunk pipeline only
     const int variant = (id_class ? 1 : 0) + (grouped ? 4 : 0);
     if (grouped && (rc = prepare_groups(b, group, params, out_iso, variant)) != 0) return rc;
@@ -1063,6 +1095,7 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
     const size_t o_iatom = o;  o += (grouped && out_iso->atom_sasa) ? al(N * 4) : 0;
     const size_t o_iseg = o;   o += (grouped && out_iso->seg_sasa && G) ? al(G * 4) : 0;
     const size_t o_iprot = o;  o += (grouped && out_iso->protein) ? al(S * 12) : 0;
+    const size_t o_mask = o;   o += masked ? al(N * W * 4) : 0;
     cudaStream_t s0 = ctx->streams[0];
     // the previous job may still be running on the sibling streams: this job's first stream starts behind all of them
     if (ctx->tail_valid)
@@ -1101,6 +1134,7 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
         gp.seg = (out_iso->seg_sasa && G) ? reinterpret_cast<float *>(base_p + o_iseg) : nullptr;
         gp.protein = out_iso->protein ? reinterpret_cast<float *>(base_p + o_iprot) : nullptr;
     }
+    const MaskParams mp{masked ? reinterpret_cast<uint32_t *>(base_p + o_mask) : nullptr};
     // ---- gated single-launch pipeline ----------------------------------------------------------------------------------
     // Thirteen launches of 148 persistent CTAs cost the pipelined run 0.25 ms over the same work as ONE launch (CTA start-ups
     // with a cold first structure, per-chunk instead of batch-wide queue; DESIGN.md section 6).  When every chunk of the plan is one
@@ -1110,7 +1144,7 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
     // there is no D2H stage to order behind individual chunks.  Needs outputs the device can address (pinned / registered
     // host memory) of moderate size; anything else takes the per-chunk launches below.
     static const bool gated_env = [] { const char *e = getenv("SASA_B200_GATED"); return !e || atoi(e) != 0; }();
-    bool gated = gated_env && variant < 2 && !b->h_gorder[variant].empty();
+    bool gated = gated_env && variant < 2 && !masked && !b->h_gorder[variant].empty();
     if (gated) {
         const size_t out_bytes = (out->counts ? N * 4 : 0) + (out->atom_sasa ? N * 4 : 0) + ((out->seg_sasa && G) ? G * 4 : 0) +
                                  (out->protein ? S * 12 : 0);
@@ -1224,7 +1258,8 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
             cudaEventRecord(e, st);
             trace_ev.push_back(e);
         }
-        if ((rc = enqueue_chunk(b, variant, ch, kbase, st, &job->launches, nullptr, grouped ? &gp : nullptr)) != 0) return job_abort(ctx, job, rc);
+        if ((rc = enqueue_chunk(b, variant, ch, kbase, st, &job->launches, nullptr, grouped ? &gp : nullptr, masked ? &mp : nullptr)) != 0)
+            return job_abort(ctx, job, rc);
         if (trace_chunks) {
             cudaEvent_t e;
             cudaEventCreate(&e);
@@ -1235,6 +1270,8 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
             J_TRY(cudaMemcpyAsync(out->counts + ch.a0, base_p + o_cnt + ch.a0 * 4, na * 4, cudaMemcpyDeviceToHost, st));
         if (na && out->atom_sasa)
             J_TRY(cudaMemcpyAsync(out->atom_sasa + ch.a0, base_p + o_atom + ch.a0 * 4, na * 4, cudaMemcpyDeviceToHost, st));
+        if (na && masked)
+            J_TRY(cudaMemcpyAsync(exposed + ch.a0 * W, base_p + o_mask + ch.a0 * W * 4, na * W * 4, cudaMemcpyDeviceToHost, st));
         if (out->seg_sasa && ch.g1 > ch.g0)
             J_TRY(cudaMemcpyAsync(out->seg_sasa + ch.g0, base_p + o_seg + ch.g0 * 4, (ch.g1 - ch.g0) * 4, cudaMemcpyDeviceToHost, st));
         if (out->protein && ch.s1 > ch.s0)
@@ -1366,6 +1403,15 @@ int sasa_b200_batch_run_groups_host(sasa_b200_batch *b, const float *xyzr, const
     if (!out_isolated) return fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "out_isolated is NULL");
     sasa_b200_job *job = nullptr;
     int rc = submit_host_impl(b, xyzr, nullptr, nullptr, id_class, params, out, &job, nullptr, 0, group, out_isolated);
+    if (rc) return rc;
+    return wait_job_impl(job, stats);
+}
+
+int sasa_b200_batch_run_masks_host(sasa_b200_batch *b, const float *xyzr, const uint32_t *id_class, const sasa_b200_params *params,
+                                   const sasa_b200_outputs *out, uint32_t *exposed, sasa_b200_stats *stats) {
+    if (!b) return SASA_B200_ERR_INVALID_ARGUMENT;
+    sasa_b200_job *job = nullptr;
+    int rc = submit_host_impl(b, xyzr, nullptr, nullptr, id_class, params, out, &job, nullptr, 0, nullptr, nullptr, true, exposed);
     if (rc) return rc;
     return wait_job_impl(job, stats);
 }

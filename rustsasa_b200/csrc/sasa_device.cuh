@@ -110,6 +110,17 @@ struct GroupAtoms {
     }
 };
 
+// Exposed-point masks (sasa_b200_batch_run_masks_*), a kernel argument of its own next to KParams: mask_words(n_points) u32 per
+// atom in batch order, bit b of word w set when point 32 w + b is exposed.  Every routine writes an atom's whole row with the
+// lanes w < W of its warp (one coalesced store), so no row is left unwritten and the buffer needs no zero-fill.
+struct MaskParams {
+    uint32_t *exposed;
+};
+__host__ __device__ constexpr uint32_t mask_words(uint32_t n_points) { return (n_points + 31u) / 32u; }
+__device__ __forceinline__ uint32_t *mask_row(const MaskParams &mp, uint32_t n_points, size_t atom) {
+    return mp.exposed + atom * mask_words(n_points);
+}
+
 struct Grid {
     float minx, miny, minz, inv_c;
     int nx, ny, nz, e;
@@ -136,6 +147,28 @@ __device__ __forceinline__ unsigned lanemask_lt() {
     unsigned m;
     asm("mov.u32 %0, %%lanemask_lt;" : "=r"(m));
     return m;
+}
+
+// Bits of the points that exist in word w of a mask row.
+__device__ __forceinline__ unsigned mask_valid(int n_points, int w) {
+    const int left = n_points - 32 * w;
+    return left >= 32 ? 0xffffffffu : (left > 0 ? (0xffffffffu >> (32 - left)) : 0u);
+}
+// Mask row of a point set of at most 128 points from the warp-uniform coverage words c0..c3 (all ones: a covered atom, zeros).
+__device__ __forceinline__ void mask_store4(uint32_t *row, int n_points, unsigned c0, unsigned c1, unsigned c2, unsigned c3) {
+    const int lane = lane_id();
+    if (lane < (int)mask_words((uint32_t)n_points))
+        row[lane] = mask_valid(n_points, lane) & ~(lane == 0 ? c0 : lane == 1 ? c1 : lane == 2 ? c2 : c3);
+}
+// A mask row of zeros (every point occluded).
+__device__ __forceinline__ void mask_zero(uint32_t *row, int n_points) {
+    const int W = (int)mask_words((uint32_t)n_points);
+    for (int w = lane_id(); w < W; w += 32) row[w] = 0u;
+}
+// The mask rows of atoms [a0, a0 + N) zeroed by the threads of a block (a structure with non-finite input).
+__device__ __forceinline__ void mask_zero_rows(const MaskParams &mp, uint32_t n_points, size_t a0, size_t N, size_t tid, size_t nth) {
+    const size_t W = mask_words(n_points);
+    for (size_t i = tid; i < N * W; i += nth) mp.exposed[a0 * W + i] = 0u;
 }
 
 __device__ __forceinline__ int cell_coord(float x, float mn, float inv_c, int n) {
@@ -228,11 +261,13 @@ __device__ __forceinline__ int row_lookup(const Rows &r, int idx) {
 // Streaming (list-free) evaluation of one atom: always correct for any density, used when
 // the neighbour list would overflow the per-warp staging area, when boundary statistics
 // are requested and as the in-kernel cross-check of the fast path.
-// Returns the exposed-point count; all lanes receive it.
+// Returns the exposed-point count; all lanes receive it.  HAS_MASK: the per-slot ballots are the
+// words of the atom's mask row `mrow`, stored by lanes 0-3 after every 128-point chunk.
 // ---------------------------------------------------------------------------------------
-template <typename AtomAcc, typename CellT, bool STATS>
+template <typename AtomAcc, typename CellT, bool STATS, bool HAS_MASK = false>
 __device__ float atom_streaming(const KParams &p, const Grid &g, const AtomAcc &atoms, const CellT *cell,
-                                const uint32_t *cls_sorted, int pos, float4 *ent, unsigned long long *boundary) {
+                                const uint32_t *cls_sorted, int pos, float4 *ent, unsigned long long *boundary,
+                                uint32_t *mrow = nullptr) {
     const int lane = lane_id();
     const float4 ai = atoms(pos);
     const float r = __fadd_rn(ai.w, p.probe);
@@ -286,11 +321,15 @@ __device__ float atom_streaming(const KParams &p, const Grid &g, const AtomAcc &
             }
             __syncwarp();
         }
+        unsigned word = 0u;   // HAS_MASK: lane s keeps the ballot of slot s
 #pragma unroll
         for (int s = 0; s < 4; ++s) {
-            exposed += (float)__popc(__ballot_sync(kFull, !occ[s]));
+            const unsigned live = __ballot_sync(kFull, !occ[s]);
+            exposed += (float)__popc(live);
+            if (HAS_MASK && lane == s) word = live;
             if (STATS) nbnd += __popc(__ballot_sync(kFull, bnd[s] && (p0 + 32u * s + lane < p.n_points)));
         }
+        if (HAS_MASK && lane < 4 && p0 / 32u + lane < mask_words(p.n_points)) mrow[p0 / 32u + lane] = word;
     }
     if (STATS && lane == 0 && nbnd) atomicAdd(boundary, (unsigned long long)nbnd);
     return exposed;

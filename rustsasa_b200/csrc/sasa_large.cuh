@@ -455,6 +455,18 @@ __device__ __noinline__ float large_cold_atom(const KParams &p, const Grid &g, c
     *streamed += 1;
     return atom_streaming<GlobalAtoms, uint32_t, false>(p, g, atoms, cells, nullptr, pos, ent, nullptr);
 }
+// The same for the masked kernels: the atom streams (atom_fast keeps no per-point result) and writes its mask row.
+__device__ __noinline__ float large_cold_atom_mask(const KParams &p, const Grid &g, const float4 *__restrict__ sorted,
+                                                   const uint32_t *__restrict__ cells, int pos, float4 *scratch, int *streamed,
+                                                   uint32_t *mrow) {
+    *streamed += 1;
+    return atom_streaming<GlobalAtoms, uint32_t, false, true>(p, g, GlobalAtoms{sorted}, cells, nullptr, pos, scratch, nullptr, mrow);
+}
+
+// Non-finite input of a masked run: the structure's mask rows are zeros, like its counts.
+__device__ __forceinline__ void large_blank_masks(const KParams &p, const MaskParams &mp, int N, uint32_t a0) {
+    mask_zero_rows(mp, p.n_points, a0, (size_t)N, (size_t)blockIdx.x * blockDim.x + threadIdx.x, (size_t)gridDim.x * blockDim.x);
+}
 
 #ifndef SASA_LARGE_TEX
 #define SASA_LARGE_TEX 16384  // structures of at least this many atoms read the cap table through the texture path in the 100-point cells
@@ -464,11 +476,12 @@ __device__ __noinline__ float large_cold_atom(const KParams &p, const Grid &g, c
 #ifndef SASA_OPT_ULARGE
 #define SASA_OPT_ULARGE 1
 #endif
-template <int NCHP, bool TEX = false>
-__global__ void __launch_bounds__(256, 4) large_cells_kernel(const KParams p, int N, uint32_t a0, LargeHeader *h,
-                                                             const float4 *__restrict__ sorted, const uint32_t *__restrict__ orig,
-                                                             const uint32_t *__restrict__ cells, const uint32_t *__restrict__ bstart,
-                                                             float *val, uint32_t rank, uint32_t n_ranks, uint32_t blk) {
+// HAS_MASK: every atom also writes its exposed-point mask row (mp); cold atoms stream.
+template <int NCHP, bool TEX, bool HAS_MASK>
+__device__ __forceinline__ void large_cells_body(const KParams &p, int N, uint32_t a0, LargeHeader *h, const float4 *__restrict__ sorted,
+                                                 const uint32_t *__restrict__ orig, const uint32_t *__restrict__ cells,
+                                                 const uint32_t *__restrict__ bstart, float *val, uint32_t rank, uint32_t n_ranks,
+                                                 uint32_t blk, const MaskParams &mp) {
     static_assert(kLCap * 16 >= kNbCap * 16 + kNbCap * 4 + 64, "the cold path's scratch must fit the staging strip");
     __shared__ __align__(16) float4 s_stage[8][kLCap];
     __shared__ __align__(16) uint32_t s_nbp[8][kLNb];
@@ -476,6 +489,7 @@ __global__ void __launch_bounds__(256, 4) large_cells_kernel(const KParams p, in
     __shared__ __align__(16) float4 s_ptab[NCHP == 1 ? 128 : 1];
     if (h->ncell == 0) {
         large_blank_outputs(p, N, a0);
+        if (HAS_MASK) large_blank_masks(p, mp, N, a0);
         return;
     }
     // the grid and the warp index on the uniform datapath (see SASA_OPT_UWARP / SASA_OPT_UGRID in sasa_tight.cuh).  Measured
@@ -523,6 +537,7 @@ __global__ void __launch_bounds__(256, 4) large_cells_kernel(const KParams p, in
             for (; pos < cell_end; ++pos) {
                 int cnt = -1;
                 float radius;
+                uint32_t *const mrow = HAS_MASK ? mask_row(mp, p.n_points, a0 + __ldg(orig + pos)) : nullptr;
                 if (total >= 0) {
                     const int self = self0 + (pos - cell_begin);
                     const float4 ai = st[self];
@@ -530,17 +545,19 @@ __global__ void __launch_bounds__(256, 4) large_cells_kernel(const KParams p, in
                     const int k = large_gather(st, total, self, ai, ai.w + reach0, nb);
                     if (k <= kLNb) {
                         if constexpr (NCHP == 1)
-                            cnt = cap_atom<TEX>(p.cap, StagedAtoms{st}, ai, p.probe, nb, k, s_ptab, (int)p.n_points, nbody, p.cap_tex);
+                            cnt = cap_atom<TEX, HAS_MASK>(p.cap, StagedAtoms{st}, ai, p.probe, nb, k, s_ptab, (int)p.n_points, nbody, p.cap_tex,
+                                                          mrow);
                         else
-                            cnt = capm_atom<NCHP, 9>(p.capm_in, p.capm_rg, p.capd, StagedAtoms{st}, ai, p.probe, nb, k, s_nbp[warp], p.pts4,
-                                                     (int)p.n_points, nbody);
+                            cnt = capm_atom<NCHP, 9, HAS_MASK>(p.capm_in, p.capm_rg, p.capd, StagedAtoms{st}, ai, p.probe, nb, k, s_nbp[warp],
+                                                               p.pts4, (int)p.n_points, nbody, mrow);
                         pairs += (unsigned)k;
                     }
                 }
                 if (cnt < 0) {   // too many candidates or neighbours for the strips: generic routines, then stage again
                     __syncwarp();
                     radius = __ldg(sorted + pos).w;
-                    cnt = (int)large_cold_atom(p, g, sorted, cells, pos, st, &streamed);
+                    cnt = HAS_MASK ? (int)large_cold_atom_mask(p, g, sorted, cells, pos, st, &streamed, mrow)
+                                   : (int)large_cold_atom(p, g, sorted, cells, pos, st, &streamed);
                     __syncwarp();
                     if (pos + 1 < cell_end) total = large_stage(g, cells, sorted, cx, cy, cz, st, self0);
                 }
@@ -555,19 +572,38 @@ __global__ void __launch_bounds__(256, 4) large_cells_kernel(const KParams p, in
     }
 }
 
+template <int NCHP, bool TEX = false>
+__global__ void __launch_bounds__(256, 4) large_cells_kernel(const KParams p, int N, uint32_t a0, LargeHeader *h,
+                                                             const float4 *__restrict__ sorted, const uint32_t *__restrict__ orig,
+                                                             const uint32_t *__restrict__ cells, const uint32_t *__restrict__ bstart,
+                                                             float *val, uint32_t rank, uint32_t n_ranks, uint32_t blk) {
+    large_cells_body<NCHP, TEX, false>(p, N, a0, h, sorted, orig, cells, bstart, val, rank, n_ranks, blk, MaskParams{});
+}
+
+template <int NCHP, bool TEX>
+__global__ void __launch_bounds__(256, 4) large_cells_masks_kernel(const KParams p, const MaskParams mp, int N, uint32_t a0, LargeHeader *h,
+                                                                   const float4 *__restrict__ sorted, const uint32_t *__restrict__ orig,
+                                                                   const uint32_t *__restrict__ cells, const uint32_t *__restrict__ bstart,
+                                                                   float *val, uint32_t blk) {
+    large_cells_body<NCHP, TEX, true>(p, N, a0, h, sorted, orig, cells, bstart, val, 0, 1, blk, mp);
+}
+
 // Generic atoms kernel: id classes, statistics flags, n_points > 1024.  One warp per atom; warps claim work blocks like the
 // cells kernel.  Only the atoms of blocks owned by `rank` are evaluated (n_ranks = 1: all).
-__global__ void __launch_bounds__(256, 2) large_atoms_kernel(const KParams p, int N, uint32_t a0, LargeHeader *h,
-                                                             const float4 *__restrict__ sorted, const uint32_t *__restrict__ orig,
-                                                             const uint32_t *__restrict__ cls_sorted, const uint32_t *__restrict__ cells,
-                                                             const uint32_t *__restrict__ bstart, float *val, uint32_t rank,
-                                                             uint32_t n_ranks, uint32_t blk) {
+// HAS_MASK: every atom also writes its exposed-point mask row (mp); atoms that would take atom_fast (id classes above 128
+// points, n_points > 1024) stream.
+template <bool HAS_MASK>
+__device__ __forceinline__ void large_atoms_body(const KParams &p, int N, uint32_t a0, LargeHeader *h, const float4 *__restrict__ sorted,
+                                                 const uint32_t *__restrict__ orig, const uint32_t *__restrict__ cls_sorted,
+                                                 const uint32_t *__restrict__ cells, const uint32_t *__restrict__ bstart, float *val,
+                                                 uint32_t rank, uint32_t n_ranks, uint32_t blk, const MaskParams &mp) {
     __shared__ __align__(16) float4 s_ent[8 * kNbCap];
     __shared__ uint32_t s_cand[8 * kNbCap];       // u32 candidate positions; reused as the u16 survivor queue
     static_assert(kNbCap * 2 >= kQueueCap, "survivor queue must fit the candidate list");
     __shared__ __align__(16) float4 s_ptab[128];
     if (h->ncell == 0) {
         large_blank_outputs(p, N, a0);
+        if (HAS_MASK) large_blank_masks(p, mp, N, a0);
         return;
     }
     const Grid g = h->grid;
@@ -601,7 +637,8 @@ __global__ void __launch_bounds__(256, 2) large_atoms_kernel(const KParams p, in
             const float4 ai = atoms(pos);
             float cnt;
             int k = -1;
-            if (!force_stream && !stats) {
+            uint32_t *const mrow = HAS_MASK ? mask_row(mp, p.n_points, a0 + orig[pos]) : nullptr;
+            if (!force_stream && !stats && (!HAS_MASK || use_cap)) {
                 const int cx = cell_coord(ai.x, g.minx, g.inv_c, g.nx), cy = cell_coord(ai.y, g.miny, g.inv_c, g.ny),
                           cz = cell_coord(ai.z, g.minz, g.inv_c, g.nz);
                 const int cid = (cz * g.ny + cy) * g.nx + cx;
@@ -610,7 +647,7 @@ __global__ void __launch_bounds__(256, 2) large_atoms_kernel(const KParams p, in
                                   : gather_candidates(p, g, atoms, cells, cls_sorted, pos, ai, w_cand);
             }
             if (k >= 0 && use_cap) {
-                cnt = (float)cap_atom(p.cap, atoms, ai, p.probe, w_cand, k, s_ptab, (int)p.n_points, nbody);
+                cnt = (float)cap_atom<false, HAS_MASK>(p.cap, atoms, ai, p.probe, w_cand, k, s_ptab, (int)p.n_points, nbody, 0ull, mrow);
                 pairs += (unsigned)k;
             } else if (k >= 0) {
                 const float r = __fadd_rn(ai.w, p.probe);
@@ -618,8 +655,8 @@ __global__ void __launch_bounds__(256, 2) large_atoms_kernel(const KParams p, in
                 cnt = atom_fast(p, w_ent, k, nfront, reinterpret_cast<uint16_t *>(w_cand), s_pts);
                 pairs += (unsigned)k;
             } else {
-                cnt = stats ? atom_streaming<GlobalAtoms, uint32_t, true>(p, g, atoms, cells, cls_sorted, pos, w_ent, p.stat)
-                            : atom_streaming<GlobalAtoms, uint32_t, false>(p, g, atoms, cells, cls_sorted, pos, w_ent, p.stat);
+                cnt = stats ? atom_streaming<GlobalAtoms, uint32_t, true, HAS_MASK>(p, g, atoms, cells, cls_sorted, pos, w_ent, p.stat, mrow)
+                            : atom_streaming<GlobalAtoms, uint32_t, false, HAS_MASK>(p, g, atoms, cells, cls_sorted, pos, w_ent, p.stat, mrow);
                 streamed += 1;
             }
             large_store(p, lane, a0 + orig[pos], orig[pos], val, atom_area(ai.w, p.probe, cnt, p.inv_n), (uint32_t)cnt);
@@ -630,6 +667,21 @@ __global__ void __launch_bounds__(256, 2) large_atoms_kernel(const KParams p, in
         if (pairs) atomicAdd(p.stat + 1, pairs);
         if (streamed) atomicAdd(p.stat + 2, streamed);
     }
+}
+
+__global__ void __launch_bounds__(256, 2) large_atoms_kernel(const KParams p, int N, uint32_t a0, LargeHeader *h,
+                                                             const float4 *__restrict__ sorted, const uint32_t *__restrict__ orig,
+                                                             const uint32_t *__restrict__ cls_sorted, const uint32_t *__restrict__ cells,
+                                                             const uint32_t *__restrict__ bstart, float *val, uint32_t rank,
+                                                             uint32_t n_ranks, uint32_t blk) {
+    large_atoms_body<false>(p, N, a0, h, sorted, orig, cls_sorted, cells, bstart, val, rank, n_ranks, blk, MaskParams{});
+}
+
+__global__ void __launch_bounds__(256, 2) large_atoms_masks_kernel(const KParams p, const MaskParams mp, int N, uint32_t a0, LargeHeader *h,
+                                                                   const float4 *__restrict__ sorted, const uint32_t *__restrict__ orig,
+                                                                   const uint32_t *__restrict__ cls_sorted, const uint32_t *__restrict__ cells,
+                                                                   const uint32_t *__restrict__ bstart, float *val, uint32_t blk) {
+    large_atoms_body<true>(p, N, a0, h, sorted, orig, cls_sorted, cells, bstart, val, 0, 1, blk, mp);
 }
 
 // One atom of the grouped atoms kernel with the list-based or streaming routines: neighbours cand[0, k) (k < 0: too many,
@@ -918,10 +970,12 @@ inline int large_reserve(LargeWorkspace &w, uint32_t n_atoms) {
 // atoms (+ the level sums when asked for).  `order` / `off` are host arrays.  range_n > 1 selects the atom-range split
 // (BASELINE cfg5): the cell list is built for the whole structure, only the work blocks owned by `range_rank` are
 // evaluated, and no sums are produced.  Grouped runs (gp set; no atom-range split, no flags) go through
-// large_groups_kernel and produce the level sums of both value vectors.
+// large_groups_kernel and produce the level sums of both value vectors.  Masked runs (mp set; no atom-range split) take the
+// masked instantiations of the cells / atoms kernels.
 inline int large_enqueue(int sm_count, LargeWorkspace &w, const KParams &kp, const uint32_t *order, uint32_t n_work,
                          const uint32_t *off, const uint32_t *seg_off, cudaStream_t st, uint32_t *launches,
-                         uint32_t range_rank = 0, uint32_t range_n = 1, const GroupParams *gp = nullptr) {
+                         uint32_t range_rank = 0, uint32_t range_n = 1, const GroupParams *gp = nullptr,
+                         const MaskParams *mp = nullptr) {
     for (uint32_t q = 0; q < n_work; ++q) {
         const uint32_t sid = order[q];
         const uint32_t a0 = off[sid];
@@ -962,18 +1016,27 @@ inline int large_enqueue(int sm_count, LargeWorkspace &w, const KParams &kp, con
         } else if (!cls && (kp.flags & 3u) == 0 && table) {
             const int ga = std::max(1, std::min((owned + 8 * (int)blk - 1) / (8 * (int)blk), sm_count * 4));
             // chunked tables are always laid out for eight chunks (the fused kernel shares them): one instantiation
-#define SASA_LARGE_CELLS(NCHP, TEX) large_cells_kernel<NCHP, TEX><<<ga, 256, 0, st>>>(kp, N, a0, w.hdr, w.sorted, w.orig, w.cells, w.bstart, w.val, range_rank, range_n, blk)
+#define SASA_LARGE_CELLS(NCHP, TEX)                                                                                                   \
+    if (mp) large_cells_masks_kernel<NCHP, TEX><<<ga, 256, 0, st>>>(kp, *mp, N, a0, w.hdr, w.sorted, w.orig, w.cells, w.bstart, w.val, blk); \
+    else large_cells_kernel<NCHP, TEX><<<ga, 256, 0, st>>>(kp, N, a0, w.hdr, w.sorted, w.orig, w.cells, w.bstart, w.val, range_rank, range_n, blk)
             if (kp.n_points <= 128) {
-                if (SASA_CAP_TEX && SASA_LARGE_TEX > 0 && kp.cap_tex && N >= SASA_LARGE_TEX) SASA_LARGE_CELLS(1, true);
-                else SASA_LARGE_CELLS(1, false);
+                if (SASA_CAP_TEX && SASA_LARGE_TEX > 0 && kp.cap_tex && N >= SASA_LARGE_TEX) {
+                    SASA_LARGE_CELLS(1, true);
+                } else {
+                    SASA_LARGE_CELLS(1, false);
+                }
             } else {
                 SASA_LARGE_CELLS(8, false);
             }
 #undef SASA_LARGE_CELLS
         } else {
             const int ga = std::max(1, std::min((owned + 8 * (int)blk - 1) / (8 * (int)blk), sm_count * 2));
-            large_atoms_kernel<<<ga, 256, 0, st>>>(kp, N, a0, w.hdr, w.sorted, w.orig, cls ? w.cls_sorted : nullptr, w.cells, w.bstart,
-                                                   w.val, range_rank, range_n, blk);
+            if (mp)
+                large_atoms_masks_kernel<<<ga, 256, 0, st>>>(kp, *mp, N, a0, w.hdr, w.sorted, w.orig, cls ? w.cls_sorted : nullptr, w.cells,
+                                                             w.bstart, w.val, blk);
+            else
+                large_atoms_kernel<<<ga, 256, 0, st>>>(kp, N, a0, w.hdr, w.sorted, w.orig, cls ? w.cls_sorted : nullptr, w.cells, w.bstart,
+                                                       w.val, range_rank, range_n, blk);
         }
         *launches += 5;
         // level sums (not in the atom-range split, where the per-atom values of the other ranks are missing); the `rank`

@@ -483,9 +483,10 @@ __device__ __forceinline__ bool claim_prefetched(const KParams &p, int *misc, ui
 
 // ---------------------------------------------------------------------------------------------------------
 // Generic fused kernel: any n_points (128-point chunks), boundary statistics, forced streaming.
+// HAS_MASK: every atom also writes its exposed-point mask row (mp); atoms that would take atom_fast (n_points > 1024) stream.
 // ---------------------------------------------------------------------------------------------------------
-template <int NT, int MINB, bool HAS_CLS, uint32_t CMAX>
-__global__ void __launch_bounds__(NT, MINB) sasa_small_kernel(const KParams p) {
+template <int NT, int MINB, bool HAS_CLS, uint32_t CMAX, bool HAS_MASK>
+__device__ __forceinline__ void small_kernel_body(const KParams &p, const MaskParams &mp) {
     extern __shared__ __align__(16) unsigned char smem[];
     constexpr uint32_t NMAX = max_atoms(NT, MINB, CMAX, HAS_CLS);
     const SmemView V = smem_view<NT, HAS_CLS, NMAX, CMAX>(smem);
@@ -502,7 +503,10 @@ __global__ void __launch_bounds__(NT, MINB) sasa_small_kernel(const KParams p) {
     while (claim_structure(p, V.misc, sid, a0, N)) {
         Grid g;
         int ncell;
-        if (!structure_setup<NT, HAS_CLS, CMAX>(p, V, sid, a0, N, g, ncell)) continue;
+        if (!structure_setup<NT, HAS_CLS, CMAX>(p, V, sid, a0, N, g, ncell)) {
+            if (HAS_MASK) mask_zero_rows(mp, p.n_points, a0, (size_t)N, threadIdx.x, NT);
+            continue;
+        }
 
         // ---- per-atom work: warps pull runs of consecutive cell-sorted atoms from a shared counter ----------
         const SmemAtoms atoms{V.atom};
@@ -521,7 +525,8 @@ __global__ void __launch_bounds__(NT, MINB) sasa_small_kernel(const KParams p) {
                 const float4 ai = V.atom[pos];
                 int cnt;
                 int k = -1;
-                if (!force_stream && !stats) {
+                uint32_t *const mrow = HAS_MASK ? mask_row(mp, p.n_points, a0 + V.orig[pos]) : nullptr;
+                if (!force_stream && !stats && (!HAS_MASK || p.capm_in)) {
                     if (pos >= cell_end) {
                         const int cx = cell_coord(ai.x, g.minx, g.inv_c, g.nx), cy = cell_coord(ai.y, g.miny, g.inv_c, g.ny),
                                   cz = cell_coord(ai.z, g.minz, g.inv_c, g.nz);
@@ -535,8 +540,8 @@ __global__ void __launch_bounds__(NT, MINB) sasa_small_kernel(const KParams p) {
                 if (k >= 0 && p.capm_in) {
                     // 128 < n_points <= 1024: the chunked cap table (sasa_cap.cuh) on the shared-memory atoms; the entry strip
                     // serves as the packed (bin, index) scratch
-                    cnt = capm_atom<8, 13>(p.capm_in, p.capm_rg, p.capd, atoms, ai, p.probe, w_cand, k, reinterpret_cast<uint32_t *>(w_ent),
-                                           p.pts4, (int)p.n_points, (int)min(p.n_points, p.n_body));
+                    cnt = capm_atom<8, 13, HAS_MASK>(p.capm_in, p.capm_rg, p.capd, atoms, ai, p.probe, w_cand, k, reinterpret_cast<uint32_t *>(w_ent),
+                                                     p.pts4, (int)p.n_points, (int)min(p.n_points, p.n_body), mrow);
                     pairs += (unsigned)k;
                 } else if (k >= 0) {
                     const float r = __fadd_rn(ai.w, p.probe);
@@ -544,8 +549,8 @@ __global__ void __launch_bounds__(NT, MINB) sasa_small_kernel(const KParams p) {
                     cnt = (int)atom_fast(p, w_ent, k, nfront, w_cand, s_pts);
                     pairs += (unsigned)k;
                 } else {
-                    cnt = (int)(stats ? atom_streaming<SmemAtoms, uint16_t, true>(p, g, atoms, V.cell, V.cls, pos, w_ent, p.stat)
-                                      : atom_streaming<SmemAtoms, uint16_t, false>(p, g, atoms, V.cell, V.cls, pos, w_ent, p.stat));
+                    cnt = (int)(stats ? atom_streaming<SmemAtoms, uint16_t, true, HAS_MASK>(p, g, atoms, V.cell, V.cls, pos, w_ent, p.stat, mrow)
+                                      : atom_streaming<SmemAtoms, uint16_t, false, HAS_MASK>(p, g, atoms, V.cell, V.cls, pos, w_ent, p.stat, mrow));
                     streamed += 1;
                 }
                 if (lane == 0) V.val[V.orig[pos]] = (float)cnt;
@@ -559,6 +564,17 @@ __global__ void __launch_bounds__(NT, MINB) sasa_small_kernel(const KParams p) {
         __syncthreads();
         structure_outputs<NT>(p, V, sid, a0, N, smem + kOffWarpBlocks);
     }
+}
+
+template <int NT, int MINB, bool HAS_CLS, uint32_t CMAX>
+__global__ void __launch_bounds__(NT, MINB) sasa_small_kernel(const KParams p) {
+    small_kernel_body<NT, MINB, HAS_CLS, CMAX, false>(p, MaskParams{});
+}
+
+// Exposed-point masks: the plain run's outputs plus every atom's mask row (n_points > 128, statistics, forced streaming).
+template <int NT, int MINB, bool HAS_CLS, uint32_t CMAX>
+__global__ void __launch_bounds__(NT, MINB) sasa_small_masks_kernel(const KParams p, const MaskParams mp) {
+    small_kernel_body<NT, MINB, HAS_CLS, CMAX, true>(p, mp);
 }
 
 }  // namespace sasa

@@ -461,26 +461,29 @@ __device__ __forceinline__ int tight_atom(const KParams &p, const float4 *ent, i
 // forced a coarser grid) take the generic per-atom gather and the generic chunked evaluation; atoms with more
 // than kNbCap neighbours (denser than any protein) the list-free streaming routine.  Returns the exposed-point
 // count and adds the atom's list length to misc[6] (pairs), or 1 to misc[7] (streamed atoms).
-template <bool HAS_CLS, class Atoms>
+// HAS_MASK: every cold atom streams (atom_fast keeps no per-point result) and writes its mask row `mrow`.
+template <bool HAS_CLS, class Atoms, bool HAS_MASK = false>
 __device__ __forceinline__ int tight_cold_eval(const float *px, const float *py, const float *pz, uint32_t n_points, uint32_t n_body,
                                                float probe, float near2, int m_min, int m_max, Grid g, const Atoms &atoms,
                                                const uint16_t *s_cell, const uint32_t *s_cls, const float4 *s_pts, int pos,
-                                               float4 *ent, uint16_t *cand, int *misc) {
+                                               float4 *ent, uint16_t *cand, int *misc, uint32_t *mrow = nullptr) {
     KParams q;
     q.px = px; q.py = py; q.pz = pz;
     q.n_points = n_points; q.n_body = n_body; q.probe = probe;
     q.near2 = near2; q.m_min = m_min; q.m_max = m_max; q.bcast_min = 16;
     const uint32_t *cls = HAS_CLS ? s_cls : nullptr;
-    const float4 ai = atoms(pos);
-    const int k = gather_candidates(q, g, atoms, s_cell, cls, pos, ai, cand);
-    if (k >= 0) {
-        const float r = __fadd_rn(ai.w, probe);
-        const int nfront = build_entries(q, atoms, ai, __fmul_rn(r, r), __fmul_rn(2.0f, r), cand, k, ent);
-        if (lane_id() == 0) atomicAdd(&misc[6], k);
-        return (int)atom_fast(q, ent, k, nfront, cand, s_pts);
+    if (!HAS_MASK) {
+        const float4 ai = atoms(pos);
+        const int k = gather_candidates(q, g, atoms, s_cell, cls, pos, ai, cand);
+        if (k >= 0) {
+            const float r = __fadd_rn(ai.w, probe);
+            const int nfront = build_entries(q, atoms, ai, __fmul_rn(r, r), __fmul_rn(2.0f, r), cand, k, ent);
+            if (lane_id() == 0) atomicAdd(&misc[6], k);
+            return (int)atom_fast(q, ent, k, nfront, cand, s_pts);
+        }
     }
     if (lane_id() == 0) atomicAdd(&misc[7], 1);
-    return (int)atom_streaming<Atoms, uint16_t, false>(q, g, atoms, s_cell, cls, pos, ent, nullptr);
+    return (int)atom_streaming<Atoms, uint16_t, false, HAS_MASK>(q, g, atoms, s_cell, cls, pos, ent, nullptr, mrow);
 }
 template <bool HAS_CLS>
 __device__ __noinline__ int tight_cold_atom(const float *px, const float *py, const float *pz, uint32_t n_points, uint32_t n_body,
@@ -489,6 +492,14 @@ __device__ __noinline__ int tight_cold_atom(const float *px, const float *py, co
                                             float4 *ent, uint16_t *cand, int *misc) {
     return tight_cold_eval<HAS_CLS>(px, py, pz, n_points, n_body, probe, near2, m_min, m_max, g, SmemAtoms{s_atom}, s_cell, s_cls,
                                     s_pts, pos, ent, cand, misc);
+}
+// The same for the masked kernel: the atom streams and writes its mask row.
+template <bool HAS_CLS>
+__device__ __noinline__ int tight_cold_atom_mask(const float *px, const float *py, const float *pz, uint32_t n_points, uint32_t n_body,
+                                                 float probe, Grid g, const float4 *s_atom, const uint16_t *s_cell, const uint32_t *s_cls,
+                                                 int pos, float4 *ent, int *misc, uint32_t *mrow) {
+    return tight_cold_eval<HAS_CLS, SmemAtoms, true>(px, py, pz, n_points, n_body, probe, 0.0f, 0, 0, g, SmemAtoms{s_atom}, s_cell, s_cls,
+                                                     nullptr, pos, ent, nullptr, misc, mrow);
 }
 // The same with the atom's group standing alone (grouped runs): atoms of other groups are invisible.
 template <bool HAS_CLS>
@@ -504,8 +515,10 @@ __device__ __noinline__ int tight_cold_atom_iso(const float *px, const float *py
 // 16-lane builds, 96 body points), or 0 to choose per launch among 1..4.
 // HAS_GRP: grouped run -- every atom is evaluated in the complex and with its group standing alone (the cap path in one pass,
 // cap_atom_groups; the cold path twice), and the output stage runs once per value array.
-template <int NT, int MINB, bool HAS_CLS, uint32_t CMAX, int NSLT, bool HAS_GRP>
-__device__ __forceinline__ void tight_kernel_body(const KParams &p, const GroupParams &gp) {
+// HAS_MASK: every atom also writes its exposed-point mask row (mp); cold atoms stream.
+template <int NT, int MINB, bool HAS_CLS, uint32_t CMAX, int NSLT, bool HAS_GRP, bool HAS_MASK = false>
+__device__ __forceinline__ void tight_kernel_body(const KParams &p, const GroupParams &gp, const MaskParams &mp = MaskParams{}) {
+    static_assert(!(HAS_GRP && HAS_MASK), "grouped runs write no masks");
     extern __shared__ __align__(16) unsigned char smem[];
     constexpr int NW = NT / 32;
     constexpr uint32_t NMAX = max_atoms(NT, MINB, CMAX, HAS_CLS, HAS_GRP);
@@ -547,7 +560,10 @@ __device__ __forceinline__ void tight_kernel_body(const KParams &p, const GroupP
 #if SASA_OPT_NEXT
         if (warp == 0) claim_next_and_prefetch(p, V.misc);   // every structure, also after a rejected one
 #endif
-        if (!ok) continue;
+        if (!ok) {
+            if (HAS_MASK) mask_zero_rows(mp, p.n_points, a0, (size_t)N, threadIdx.x, NT);
+            continue;
+        }
 #if SASA_OPT_USTRUCT
         sid = uniform_u32(sid); a0 = uniform_u32(a0); N = uniform_i32(N);
 #endif
@@ -634,8 +650,10 @@ __device__ __forceinline__ void tight_kernel_body(const KParams &p, const GroupP
                         int ka, kb;
                         tight_gather2(V.atom, w_list, total, pos, pos + 1, aa, ab, aa.w + reach0, ab.w + reach0, w_cand, w_cand2, ka, kb);
                         if (ka > kNbCap || kb > kNbCap) break;   // dense neighbourhood: the one-atom path below sorts it out
-                        const int ca = cap_atom<SASA_CAP_TEX != 0>(p.cap, SmemAtoms{V.atom}, aa, p.probe, w_cand, ka, V.ptab, (int)p.n_points, nbody, p.cap_tex);
-                        const int cb = cap_atom<SASA_CAP_TEX != 0>(p.cap, SmemAtoms{V.atom}, ab, p.probe, w_cand2, kb, V.ptab, (int)p.n_points, nbody, p.cap_tex);
+                        uint32_t *const ra = HAS_MASK ? mask_row(mp, p.n_points, a0 + V.orig[pos]) : nullptr;
+                        uint32_t *const rb = HAS_MASK ? mask_row(mp, p.n_points, a0 + V.orig[pos + 1]) : nullptr;
+                        const int ca = cap_atom<SASA_CAP_TEX != 0, HAS_MASK>(p.cap, SmemAtoms{V.atom}, aa, p.probe, w_cand, ka, V.ptab, (int)p.n_points, nbody, p.cap_tex, ra);
+                        const int cb = cap_atom<SASA_CAP_TEX != 0, HAS_MASK>(p.cap, SmemAtoms{V.atom}, ab, p.probe, w_cand2, kb, V.ptab, (int)p.n_points, nbody, p.cap_tex, rb);
                         pairs += (unsigned)(ka + kb);
                         if (lane < 2) V.val[(int)V.orig[pos + lane]] = (float)(lane ? cb : ca);
                         __syncwarp();
@@ -654,13 +672,15 @@ __device__ __forceinline__ void tight_kernel_body(const KParams &p, const GroupP
                     int k = total >= 0 ? tight_gather<HAS_CLS>(V.atom, V.cls, w_list, total, pos, ai, ai.w + reach0, w_nb)
                                        : kNbCap + 1;
                     int cnt_iso = 0;
+                    uint32_t *const mrow = HAS_MASK ? mask_row(mp, p.n_points, a0 + V.orig[pos]) : nullptr;
                     if (k <= kNbCap) {
 #if SASA_OPT_CAP
                         if (HAS_GRP)
                             cnt = cap_atom_groups<SASA_CAP_TEX != 0>(p.cap, SmemAtoms{V.atom}, ai, p.probe, w_nb, k, V.grp, V.grp[pos], V.ptab,
                                                                      (int)p.n_points, nbody, p.cap_tex, &cnt_iso);
                         else
-                            cnt = cap_atom<SASA_CAP_TEX != 0>(p.cap, SmemAtoms{V.atom}, ai, p.probe, w_nb, k, V.ptab, (int)p.n_points, nbody, p.cap_tex);
+                            cnt = cap_atom<SASA_CAP_TEX != 0, HAS_MASK>(p.cap, SmemAtoms{V.atom}, ai, p.probe, w_nb, k, V.ptab, (int)p.n_points, nbody,
+                                                                        p.cap_tex, mrow);
 #else
                         static_assert(!HAS_GRP, "grouped runs need the cap path");
                         const float r = __fadd_rn(ai.w, p.probe);
@@ -673,6 +693,9 @@ __device__ __forceinline__ void tight_kernel_body(const KParams &p, const GroupP
                         else cnt = tight_atom<1>(p, w_ent, k, nfront, V.ptab, w_cand, nbody, tail_sh);
 #endif
                         pairs += (unsigned)k;
+                    } else if (HAS_MASK) {
+                        cnt = tight_cold_atom_mask<HAS_CLS>(p.px, p.py, p.pz, p.n_points, p.n_body, p.probe, g, V.atom, V.cell, V.cls, pos,
+                                                            w_ent, V.misc, mrow);
                     } else {
                         cnt = tight_cold_atom<HAS_CLS>(p.px, p.py, p.pz, p.n_points, p.n_body, p.probe, p.near2, p.m_min, p.m_max,
                                                        g, V.atom, V.cell, V.cls, V.ptab, pos, w_ent, w_cand, V.misc);
@@ -714,6 +737,12 @@ __device__ __forceinline__ void tight_kernel_body(const KParams &p, const GroupP
 template <int NT, int MINB, bool HAS_CLS, uint32_t CMAX, int NSLT>
 __global__ void __launch_bounds__(NT, MINB) sasa_tight_kernel(const KParams p) {
     tight_kernel_body<NT, MINB, HAS_CLS, CMAX, NSLT, false>(p, GroupParams{});
+}
+
+// Exposed-point masks (n_points <= 128): the plain run's outputs plus every atom's mask row.
+template <int NT, int MINB, bool HAS_CLS, uint32_t CMAX>
+__global__ void __launch_bounds__(NT, MINB) sasa_tight_masks_kernel(const KParams p, const MaskParams mp) {
+    tight_kernel_body<NT, MINB, HAS_CLS, CMAX, 0, false, true>(p, GroupParams{}, mp);
 }
 
 // Grouped runs (n_points <= 128): complex and isolated outputs of every structure in one pass.

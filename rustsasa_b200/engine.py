@@ -80,6 +80,7 @@ class BatchResult:
     seg_sasa: Optional[np.ndarray] = None
     protein: Optional[np.ndarray] = None   # (S, 3): global, polar, non-polar
     stats: Optional[dict] = None
+    exposed: Optional[np.ndarray] = None   # (n_atoms, W) uint32 exposed-point masks (run_masks_host), W = ceil(n_points / 32)
 
 
 class Engine:
@@ -260,6 +261,34 @@ class Batch:
         prm = self._params(probe_radius, n_points, simd_lanes, flags)
         self.engine._check(self._L.sasa_b200_batch_run_device(self._h, _ptr(d_xyzr), _ptr(d_id_class), C.byref(prm),
                                                              C.byref(outs), _stream(stream)))
+
+    def run_masks_host(self, xyzr, id_class=None, probe_radius=1.4, n_points=100, simd_lanes=8, flags=0,
+                       want=("counts", "atom", "seg", "protein")) -> BatchResult:
+        """run_host plus every atom's exposed-point mask in ``exposed``, an (n_atoms, W) uint32 array with W = ceil(n_points /
+        32): bit b of word w is set when point 32 w + b (the order of ``Engine.sphere_points``) is solvent-accessible."""
+        xyzr = _np(xyzr, np.float32, (-1, 4))
+        assert xyzr.shape[0] == self.n_atoms, "xyzr does not match struct_off"
+        id_class = _np(id_class, np.uint32)
+        res = self._host_outputs(want, "numpy")
+        res.exposed = np.zeros((self.n_atoms, (n_points + 31) // 32), np.uint32)
+        outs = _lib.Outputs(_ptr(res.counts), _ptr(res.atom_sasa), _ptr(res.seg_sasa), _ptr(res.protein))
+        prm = self._params(probe_radius, n_points, simd_lanes, flags)
+        st = _lib.Stats()
+        self.engine._check(self._L.sasa_b200_batch_run_masks_host(self._h, _ptr(xyzr), _ptr(id_class), C.byref(prm), C.byref(outs),
+                                                                 _ptr(res.exposed), C.byref(st)))
+        res.stats = st.as_dict()
+        return res
+
+    def run_masks_device(self, d_xyzr, d_exposed, d_id_class=None, probe_radius=1.4, n_points=100, simd_lanes=8, flags=0,
+                         counts=None, atom_sasa=None, seg_sasa=None, protein=None, stream=None):
+        """run_device plus the exposed-point masks into ``d_exposed``, a torch CUDA tensor of n_atoms * ceil(n_points / 32)
+        32-bit words (e.g. int32 of shape (n_atoms, W)); enqueues on `stream` and returns without synchronising."""
+        if d_exposed is not None:
+            assert d_exposed.numel() * d_exposed.element_size() >= self.n_atoms * ((n_points + 31) // 32) * 4, "d_exposed is too small"
+        outs = _lib.Outputs(_ptr(counts), _ptr(atom_sasa), _ptr(seg_sasa), _ptr(protein))
+        prm = self._params(probe_radius, n_points, simd_lanes, flags)
+        self.engine._check(self._L.sasa_b200_batch_run_masks_device(self._h, _ptr(d_xyzr), _ptr(d_id_class), C.byref(prm),
+                                                                   C.byref(outs), _ptr(d_exposed), _stream(stream)))
 
     def run_groups_host(self, xyzr, group, id_class=None, probe_radius=1.4, n_points=100, simd_lanes=8, flags=0,
                         want=("counts", "atom", "seg", "protein")):
