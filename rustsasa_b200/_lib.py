@@ -10,7 +10,7 @@ import ctypes as C
 import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("SASA_B200_LIB") or os.path.join(HERE, "libsasa_b200.so")   # env override: tuning variants
+LIB_PATH = os.environ.get("SASA_B200_LIB") or os.path.join(HERE, "libsasa_b200.so")   # env override: another build of the library
 
 OK, ERR_INVALID_ARGUMENT, ERR_CUDA, ERR_OUT_OF_MEMORY, ERR_NON_FINITE, ERR_UNSUPPORTED = range(6)
 FLAG_BOUNDARY_STATS = 1

@@ -22,12 +22,11 @@ def needs_build() -> bool:
     return any(os.path.getmtime(d) > t for d in DEPS)
 
 
-def build(force: bool = False, verbose: bool = False, defines=(), out: str = OUT) -> str:
-    """defines / out: build a tuning variant (e.g. defines=("-DSASA_FETCH=1",), out=".../libsasa_b200_f1.so")."""
-    if not force and out == OUT and not needs_build():
+def build(force: bool = False, verbose: bool = False) -> str:
+    if not force and not needs_build():
         return OUT
     nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-    cmd = [nvcc] + NVCC_FLAGS + list(defines) + (["-Xptxas", "-v"] if verbose else []) + ["-o", out, SRC]
+    cmd = [nvcc] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-o", OUT, SRC]
     env = dict(os.environ)
     env.pop("CC", None)
     env.pop("CXX", None)
@@ -36,7 +35,7 @@ def build(force: bool = False, verbose: bool = False, defines=(), out: str = OUT
         print(r.stdout)
     if r.returncode != 0:
         raise RuntimeError("nvcc failed:\n" + r.stdout)
-    return out
+    return OUT
 
 
 HOST_DIR = os.path.join(HERE, "csrc", "host")

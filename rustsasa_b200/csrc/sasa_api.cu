@@ -39,12 +39,42 @@ thread_local std::string g_create_error;
 struct Points {
     float *d = nullptr;    // 3*n floats: x[n] y[n] z[n]
     uint4 *cap = nullptr;  // cap table (sasa_cap.cuh), n <= 128 only
-    cudaTextureObject_t cap_tex = 0;   // the same table as a linear uint4 texture (SASA_CAP_TEX)
+    cudaTextureObject_t cap_tex = 0;   // the same table as a linear uint4 texture (the fused kernel reads it through the texture pipe)
     // 128 < n <= 1024: the points as float4 and the chunked cap table (inner / ring masks in separate arrays)
     float4 *d4 = nullptr;
     uint4 *capm_in = nullptr, *capm_rg = nullptr;
     CapDims capd = {};
 };
+
+// The fused kernels of one shared-memory configuration, by attribute slot (kernel_slot).
+constexpr int kKernelSlots = 10;
+struct Proto {
+    int nt, minb;
+    uint32_t cmax;
+    uint32_t cap[4];                 // max_atoms(...), index = has_cls + 2 * grouped
+    const void *fn[kKernelSlots];
+};
+// Slots: plain runs has_cls + 2 * tight, masked runs 4 + the same (tight: n_points <= 128, no statistics / forced streaming),
+// grouped runs 8 + has_cls (always tight: they take no flags, and with n_points > 128 they take the large-structure path).
+int kernel_slot(bool grouped, bool masked, bool has_cls, bool tight) {
+    return grouped ? 8 + (has_cls ? 1 : 0) : (masked ? 4 : 0) + (has_cls ? 1 : 0) + (tight ? 2 : 0);
+}
+#define SASA_PROTO(NT, MINB, CMAX)                                                                                     \
+    Proto { NT, MINB, CMAX, { max_atoms(NT, MINB, CMAX, false), max_atoms(NT, MINB, CMAX, true),                       \
+                              max_atoms(NT, MINB, CMAX, false, true), max_atoms(NT, MINB, CMAX, true, true) },         \
+            { (const void *)sasa_small_kernel<NT, MINB, false, CMAX>, (const void *)sasa_small_kernel<NT, MINB, true, CMAX>, \
+              (const void *)sasa_tight_kernel<NT, MINB, false, CMAX>, (const void *)sasa_tight_kernel<NT, MINB, true, CMAX>, \
+              (const void *)sasa_small_masks_kernel<NT, MINB, false, CMAX>,                                            \
+              (const void *)sasa_small_masks_kernel<NT, MINB, true, CMAX>,                                             \
+              (const void *)sasa_tight_masks_kernel<NT, MINB, false, CMAX>,                                            \
+              (const void *)sasa_tight_masks_kernel<NT, MINB, true, CMAX>,                                             \
+              (const void *)sasa_tight_groups_kernel<NT, MINB, false, CMAX>,                                           \
+              (const void *)sasa_tight_groups_kernel<NT, MINB, true, CMAX> } }
+// Shared-memory configurations of the fused kernel.  nmax is derived from the per-CTA budget that lets `minb` CTAs share one SM
+// (228 KB per SM, 1 KB reserved per CTA, 227 KB per CTA max); both keep 32 warps resident per SM (64 registers/thread).
+const Proto kProtos[] = {SASA_PROTO(512, 2, 8192), SASA_PROTO(1024, 1, 16384)};
+#undef SASA_PROTO
+constexpr int kNumProtos = sizeof(kProtos) / sizeof(kProtos[0]);
 
 struct SmallCfg {
     int nt, minb;
@@ -54,10 +84,9 @@ struct SmallCfg {
     int proto;
 };
 
-#ifndef SASA_STREAMS
-#define SASA_STREAMS 3   // streams of the pipelined host entry points.  cfg2 end to end, device-side span (tools/exp_e2e.py, one B200): 2 streams
-#endif                   // 5.92 ms, 3: 5.26 ms, 4: 5.29 ms, 6: 5.37 ms (5.00 ms as one device-resident launch)
-constexpr int kStreams = SASA_STREAMS;
+// Streams of the pipelined host entry points.  cfg2 end to end, device-side span (tools/exp_e2e.py, one B200): 2 streams 5.92 ms,
+// 3: 5.26 ms, 4: 5.29 ms, 6: 5.37 ms (5.00 ms as one device-resident launch).
+constexpr int kStreams = 3;
 constexpr size_t kChunkAtoms = 1000000;
 constexpr size_t kMaxGatedChunks = 1024;              // chunks of one gated single-launch run (more: the per-chunk launches)
 constexpr size_t kGatedMaxOutBytes = 32u << 20;        // outputs above this go through device memory and D2H copies
@@ -115,7 +144,7 @@ struct sasa_b200_ctx {
     LargeWorkspace large;
     cudaEvent_t ev_large = nullptr;
     bool large_used = false;
-    bool attr_done[8][12] = {};  // [kernel configuration][instantiation]: shared-memory attribute set (at first launch)
+    bool attr_done[kNumProtos][kKernelSlots] = {};  // shared-memory attribute set (at a kernel's first launch)
     // jobs: one per host-buffer run in flight (submit / wait); recycled, so events and the pinned status word are made once
     std::vector<sasa_b200_job *> free_jobs;
     cudaEvent_t ev_tail[kStreams] = {};   // end of the previous job on each copy stream (the next job's first stream waits on them)
@@ -178,25 +207,18 @@ int get_points(sasa_b200_ctx *ctx, uint32_t n, const Points **out) {
             cap_build_table(n, h.data(), h.data() + n, h.data() + 2 * (size_t)n, t.data());
             CU_TRY(ctx, cudaMalloc(&P.cap, t.size() * sizeof(uint32_t)));
             CU_TRY(ctx, cudaMemcpy(P.cap, t.data(), t.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
-#if SASA_CAP_TEX
-            {
-                cudaResourceDesc rd = {};
-                rd.resType = cudaResourceTypeLinear;
-                rd.res.linear.devPtr = P.cap;
-                rd.res.linear.desc = cudaCreateChannelDesc<uint4>();
-                rd.res.linear.sizeInBytes = t.size() * sizeof(uint32_t);
-                cudaTextureDesc td = {};
-                td.readMode = cudaReadModeElementType;
-                CU_TRY(ctx, cudaCreateTextureObject(&P.cap_tex, &rd, &td, nullptr));
-            }
-#endif
+            cudaResourceDesc rd = {};
+            rd.resType = cudaResourceTypeLinear;
+            rd.res.linear.devPtr = P.cap;
+            rd.res.linear.desc = cudaCreateChannelDesc<uint4>();
+            rd.res.linear.sizeInBytes = t.size() * sizeof(uint32_t);
+            cudaTextureDesc td = {};
+            td.readMode = cudaReadModeElementType;
+            CU_TRY(ctx, cudaCreateTextureObject(&P.cap_tex, &rd, &td, nullptr));
         } else if (n <= 1024) {   // chunked table for the large-structure path (sasa_cap.cuh, capm_atom)
-            static const int grid_n = [] {
-                const char *e = getenv("SASA_B200_CAPM_N");   // tuning aid: direction bins per axis (even)
-                const int v = e ? atoi(e) : 64;
-                return v >= 8 && v <= 256 && v % 2 == 0 ? v : 64;
-            }();
-            P.capd = cap_dims(grid_n, kCapmL, 8);   // always eight chunk slots: capm_atom<8> serves every 128 < n <= 1024
+            // 64 direction bins per axis: a 96^2 / 128^2 grid measured 1.55 / 1.54 ms against 1.60 ms on cfg5 (run r02l) for
+            // 2.3x / 4x the table.  Always eight chunk slots: capm_atom<8> serves every 128 < n <= 1024.
+            P.capd = cap_dims(64, kCapmL, 8);
             const size_t words = cap_multi_words(P.capd);
             std::vector<uint32_t> tin(words), trg(words);
             cap_build_table_multi(n, h.data(), h.data() + n, h.data() + 2 * (size_t)n, P.capd, tin.data(), trg.data());
@@ -219,60 +241,19 @@ int get_points(sasa_b200_ctx *ctx, uint32_t n, const Points **out) {
     return SASA_B200_OK;
 }
 
-// Shared-memory configurations of the fused kernel, smallest atom capacity first.  nmax is derived from the
-// per-CTA budget that lets `minb` CTAs share one SM (228 KB per SM, 1 KB reserved per CTA, 227 KB per CTA max).
-typedef void (*SmallKernel)(const KParams);
-typedef void (*GroupKernel)(const KParams, const GroupParams);
-typedef void (*MaskKernel)(const KParams, const MaskParams);
-struct Proto {
-    int nt, minb;
-    uint32_t cmax;
-    uint32_t cap[4];     // max_atoms(...), index = has_cls + 2 * grouped
-    SmallKernel fn[6];   // index = has_cls + 2 * tight (tight: n_points <= 128, no statistics / forced streaming)
-                         //         + 2 more when the tight kernel compiled for 3 body slots applies (65..96 body points)
-    GroupKernel fng[2];  // grouped runs (n_points <= 128), index = has_cls
-    MaskKernel fnm[4];   // exposed-point masks, index = has_cls + 2 * tight (same shared memory as the plain kernels)
-};
-#define SASA_PROTO(NT, MINB, CMAX)                                                                                     \
-    Proto { NT, MINB, CMAX, { max_atoms(NT, MINB, CMAX, false), max_atoms(NT, MINB, CMAX, true),                       \
-                              max_atoms(NT, MINB, CMAX, false, true), max_atoms(NT, MINB, CMAX, true, true) },         \
-            { sasa_small_kernel<NT, MINB, false, CMAX>, sasa_small_kernel<NT, MINB, true, CMAX>,                       \
-              sasa_tight_kernel<NT, MINB, false, CMAX, 0>, sasa_tight_kernel<NT, MINB, true, CMAX, 0>,                 \
-              sasa_tight_kernel<NT, MINB, false, CMAX, 3>, sasa_tight_kernel<NT, MINB, true, CMAX, 3> },               \
-            { sasa_tight_groups_kernel<NT, MINB, false, CMAX>, sasa_tight_groups_kernel<NT, MINB, true, CMAX> },           \
-            { sasa_small_masks_kernel<NT, MINB, false, CMAX>, sasa_small_masks_kernel<NT, MINB, true, CMAX>,               \
-              sasa_tight_masks_kernel<NT, MINB, false, CMAX>, sasa_tight_masks_kernel<NT, MINB, true, CMAX> } }
-// 0-2 keep 32 warps resident per SM (64 registers/thread); 3-4 keep 24 warps (85 registers/thread)
-#ifndef SASA_ALL_PROTOS   // the shipped build instantiates the two default configurations only (half the build time and library
-                         // size); -DSASA_ALL_PROTOS adds the three tuning configurations selectable with SASA_B200_CFGS
-#ifndef SASA_NT_MAIN
-#define SASA_NT_MAIN 1024
-#endif
-const Proto kProtos[] = {SASA_PROTO(512, 2, 8192), SASA_PROTO(512, 2, 8192), SASA_PROTO(SASA_NT_MAIN, 1, 16384),
-                         SASA_PROTO(512, 2, 8192), SASA_PROTO(SASA_NT_MAIN, 1, 16384)};
-#else
-const Proto kProtos[] = {SASA_PROTO(256, 4, 4096), SASA_PROTO(512, 2, 8192), SASA_PROTO(1024, 1, 16384),
-                         SASA_PROTO(384, 2, 8192), SASA_PROTO(768, 1, 16384)};
-#endif
-const char *kDefaultCfgs = "12";
-constexpr int kNumProtos = sizeof(kProtos) / sizeof(kProtos[0]);
-
+// The configurations of the context, smallest atom capacity first.
 int build_cfgs(sasa_b200_ctx *ctx) {
-    const char *only = getenv("SASA_B200_CFGS");   // e.g. "34": choose the configurations (tuning aid)
-    if (!only || !*only) only = kDefaultCfgs;
     for (int i = 0; i < kNumProtos; ++i) {
         const Proto &pr = kProtos[i];
-        if (!strchr(only, '0' + i)) continue;
         SmallCfg c{pr.nt, pr.minb, {pr.cap[0], pr.cap[1], pr.cap[2], pr.cap[3]}, pr.cmax, {0, 0, 0, 0}, i};
         for (int v = 0; v < 4; ++v) c.smem[v] = small_layout(c.cap[v], c.cmax, c.nt / 32, (v & 1) == 1, v >= 2).total;
         if (*std::min_element(c.cap, c.cap + 4) == 0 || *std::max_element(c.smem, c.smem + 4) > ctx->smem_optin)
             return fail(ctx, SASA_B200_ERR_UNSUPPORTED, "the fused kernels are laid out for 228 KB of shared memory per SM (B200); this device offers %zu per block",
                         ctx->smem_optin);
-        // (the MaxDynamicSharedMemorySize attribute is set at a kernel's first launch, enqueue_chunk: touching all thirty
-        // instantiations here made the driver load every one of them at context creation)
+        // (the MaxDynamicSharedMemorySize attribute is set at a kernel's first launch, enqueue_chunk: touching every
+        // instantiation here made the driver load every one of them at context creation)
         ctx->cfgs.push_back(c);
     }
-    if (ctx->cfgs.empty()) return fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "SASA_B200_CFGS selects no kernel configuration");
     std::sort(ctx->cfgs.begin(), ctx->cfgs.end(), [](const SmallCfg &a, const SmallCfg &b) { return a.cap[0] < b.cap[0]; });
     return SASA_B200_OK;
 }
@@ -327,19 +308,10 @@ struct sasa_b200_batch {
 
 namespace {
 
-// Queue of the gated single-launch pipeline: CHUNK-MAJOR -- the structures of chunk 0 largest-first, then those of chunk 1, ... --
-// so that a CTA only ever waits for the chunk the copy stream is working on and a slow copy (eight ranks sharing one host, pageable
-// input) degrades the run gracefully: everything that has arrived is worked on, the end is the last chunk's copy plus its work.
-// The builder can also simulate arrival against work and give every position the largest structure that has arrived
-// (SASA_B200_GATED_RATE = assumed ratio of copy to compute speed in atoms, > 0): after the copies are done the rest of the queue
-// is then in exact largest-first order, as in a device-resident run.  Measured on cfg2 with rate 1.25 (the real ratio is about 2
-// for the 13-byte wire format on one GPU): 5.21 -> 5.18 ms.  It is off by default because it is fragile: where the copies are
-// slower than assumed, large structures of chunks still to come sit at the head of the queue, the CTAs wait for them, and the small
-// structures of every chunk pile up behind the last copy.
-static double gated_rate() {
-    static const double r = [] { const char *e = getenv("SASA_B200_GATED_RATE"); return e ? atof(e) : 0.0; }();
-    return r;
-}
+// Queue of the gated single-launch pipeline: CHUNK-MAJOR -- the structures of chunk 0 largest-first (ties: lower index first),
+// then those of chunk 1, ... -- so that a CTA only ever waits for the chunk the copy stream is working on and a slow copy (eight
+// ranks sharing one host, pageable input) degrades the run gracefully: everything that has arrived is worked on, the end is the
+// last chunk's copy plus its work.
 void build_gated_order(sasa_b200_batch *b, int variant) {
     std::vector<uint32_t> &order = b->h_gorder[variant], &need = b->h_gneed[variant];
     order.clear();
@@ -350,32 +322,11 @@ void build_gated_order(sasa_b200_batch *b, int variant) {
     for (const Chunk &ch : plan)
         if (ch.launches.size() != 1 || ch.launches[0].cfg < 0 || ch.launches[0].cfg != cfg0) return;
     auto atoms_of = [&](uint32_t sidx) { return b->h_off[sidx + 1] - b->h_off[sidx]; };
-    std::vector<std::pair<uint32_t, uint32_t>> heap;   // (atoms, structure), max-heap; ties: lower structure index first
-    auto less = [](const std::pair<uint32_t, uint32_t> &x, const std::pair<uint32_t, uint32_t> &y) {
-        return x.first != y.first ? x.first < y.first : x.second > y.second;
-    };
-    std::vector<uint32_t> chunk_of(b->S, 0);
-    size_t next_chunk = 0;
-    double t = 0.0;
-    const double rate = gated_rate();
-    auto arrive = [&]() {
-        const Chunk &ch = plan[next_chunk];
-        for (uint32_t i = ch.s0; i < ch.s1; ++i) {
-            chunk_of[i] = (uint32_t)next_chunk;
-            heap.emplace_back(atoms_of(i), i);
-            std::push_heap(heap.begin(), heap.end(), less);
-        }
-        ++next_chunk;
-    };
-    arrive();
-    while (order.size() < b->S) {
-        while (next_chunk < plan.size() && (heap.empty() || (rate > 0.0 && (double)(plan[next_chunk].a1 - plan[0].a1) <= rate * t))) arrive();
-        std::pop_heap(heap.begin(), heap.end(), less);
-        const std::pair<uint32_t, uint32_t> top = heap.back();
-        heap.pop_back();
-        order.push_back(top.second);
-        need.push_back(chunk_of[top.second] + 1);
-        t += (double)top.first;
+    for (size_t c = 0; c < plan.size(); ++c) {
+        const size_t first = order.size();
+        for (uint32_t i = plan[c].s0; i < plan[c].s1; ++i) order.push_back(i);
+        std::stable_sort(order.begin() + first, order.end(), [&](uint32_t x, uint32_t y) { return atoms_of(x) > atoms_of(y); });
+        need.resize(order.size(), (uint32_t)(c + 1));
     }
 }
 
@@ -411,7 +362,7 @@ void build_plan(sasa_b200_batch *b, int variant) {
         ch.s0 = s;
         ch.a0 = b->h_off[s];
         // the first chunks are smaller so that the first kernel starts after a short copy (ramp 1/8, 1/4, 1/2, 1, 1, ...)
-        static const size_t ramp_levels = [] { const char *e = getenv("SASA_B200_RAMP"); return e ? (size_t)atoi(e) : (size_t)3; }();
+        constexpr size_t ramp_levels = 3;
         const size_t ramp = plan.size() < ramp_levels && chunk_atoms != ~(size_t)0 ? chunk_atoms >> (ramp_levels - plan.size()) : chunk_atoms;
         while (s < b->S && (b->h_off[s] - ch.a0 < ramp || s == ch.s0)) ++s;
         // equal-sized structures (MD frames) finish in lock step: cut the chunk at a whole number of waves of the
@@ -510,22 +461,13 @@ void fill_run_params(KParams *kp, const Points *pts, const sasa_b200_params &prm
     kp->n_body = (n / lanes) * lanes;
     kp->inv_n = 1.0f / (float)n;
     kp->probe = prm.probe_radius;
-    static const float near_a = [] {
-        const char *e = getenv("SASA_B200_NEAR");
-        return e ? (float)atof(e) : 4.0f;
-    }();
-    kp->near2 = near_a * near_a;
-    static const int bcast_min = [] {
-        const char *e = getenv("SASA_B200_BCAST_MIN");
-        return e ? atoi(e) : 16;
-    }();
-    kp->bcast_min = bcast_min;
-    static const int m_min = [] { const char *e = getenv("SASA_B200_M_MIN"); return e ? atoi(e) : 4; }();
-    static const int m_max = [] { const char *e = getenv("SASA_B200_M_MAX"); return e ? atoi(e) : 16; }();
-    kp->m_min = m_min;
-    kp->m_max = m_max;
-    static const uint32_t nocache = getenv("SASA_B200_NOCACHE") ? 4u : 0u;   // tuning aid
-    kp->flags = prm.flags | nocache;
+    // the two-phase point tests of the generic kernel (atom_fast): neighbours nearer than 4 A first, phase 1 against 4..16 of
+    // them, the broadcast form of phase 2 above 16 survivors
+    kp->near2 = 4.0f * 4.0f;
+    kp->bcast_min = 16;
+    kp->m_min = 4;
+    kp->m_max = 16;
+    kp->flags = prm.flags;
 }
 
 int make_kparams(sasa_b200_batch *b, const RunArgs &ra, KParams *kp) {
@@ -568,10 +510,9 @@ int enqueue_chunk(sasa_b200_batch *b, int variant, const Chunk &ch, const KParam
     sasa_b200_ctx *ctx = b->ctx;
     int n_small = 0;
     for (const Launch &L : ch.launches) n_small += L.cfg >= 0;
-    static const bool no_fork = getenv("SASA_B200_NO_FORK") != nullptr;   // tuning aid
     // device-resident runs only: in the pipelined host path the sibling streams would be shared by chunks in flight on
     // different copy streams and delay their D2H (measured: -5 % end to end), while the next chunk back-fills anyway
-    const bool fork = !no_fork && (variant & 2) && n_small > 1 && n_small <= sasa_b200_ctx::kSide + 1;
+    const bool fork = (variant & 2) && n_small > 1 && n_small <= sasa_b200_ctx::kSide + 1;
     if (fork) CU_TRY(ctx, cudaEventRecord(ctx->ev_fork, st));
     int small_idx = 0, forked = 0;
     // grouped runs with more than 128 points: no fused kernel, every structure takes the large-structure path
@@ -603,20 +544,13 @@ int enqueue_chunk(sasa_b200_batch *b, int variant, const Chunk &ch, const KParam
         }
         void *args[] = {(void *)&kp, mp ? (void *)mp : (void *)gp};
         const bool tight = kp.n_points <= 128 && (kp.flags & 3u) == 0;
-        const uint32_t body = std::min(kp.n_points, kp.n_body);
-        // (attribute slots 6 / 7: the grouped kernels; 8-11: the masked kernels)
-        const int mwhich = (has_cls ? 1 : 0) + (tight ? 2 : 0);
-        const int which = grouped ? 6 + (has_cls ? 1 : 0)
-                          : mp    ? 8 + mwhich
-                                  : (has_cls ? 1 : 0) + (tight ? (SASA_OPT_NSLT && body > 64 && body <= 96 ? 4 : 2) : 0);
-        const void *fn = grouped ? (const void *)kProtos[c.proto].fng[has_cls ? 1 : 0]
-                         : mp    ? (const void *)kProtos[c.proto].fnm[mwhich]
-                                 : (const void *)kProtos[c.proto].fn[which];
-        if (!ctx->attr_done[c.proto][which]) {
+        const int slot = kernel_slot(grouped, mp != nullptr, has_cls, tight);
+        const void *fn = kProtos[c.proto].fn[slot];
+        if (!ctx->attr_done[c.proto][slot]) {
             cudaError_t ea = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
             if (ea != cudaSuccess)
                 return fail(ctx, SASA_B200_ERR_CUDA, "cudaFuncSetAttribute(MaxDynamicSharedMemorySize=%zu) failed: %s", smem, cudaGetErrorString(ea));
-            ctx->attr_done[c.proto][which] = true;
+            ctx->attr_done[c.proto][slot] = true;
         }
         cudaError_t e = cudaLaunchKernel(fn, dim3(grid), dim3(c.nt), args, smem, ls);
         if (e != cudaSuccess) return fail(ctx, SASA_B200_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(e));
@@ -1143,8 +1077,7 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
     // (wait_ready, sasa_small.cuh), and the kernel writes its results straight into the caller's page-locked buffers --
     // there is no D2H stage to order behind individual chunks.  Needs outputs the device can address (pinned / registered
     // host memory) of moderate size; anything else takes the per-chunk launches below.
-    static const bool gated_env = [] { const char *e = getenv("SASA_B200_GATED"); return !e || atoi(e) != 0; }();
-    bool gated = gated_env && variant < 2 && !masked && !b->h_gorder[variant].empty();
+    bool gated = variant < 2 && !masked && !b->h_gorder[variant].empty();
     if (gated) {
         const size_t out_bytes = (out->counts ? N * 4 : 0) + (out->atom_sasa ? N * 4 : 0) + ((out->seg_sasa && G) ? G * 4 : 0) +
                                  (out->protein ? S * 12 : 0);
@@ -1191,10 +1124,6 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
     J_TRY(cudaEventRecord(job->ev0, s0));
     for (int i = 1; i < kStreams; ++i) J_TRY(cudaStreamWaitEvent(ctx->streams[i], job->ev0, 0));
     size_t ci = 0;
-    // SASA_B200_TRACE_CHUNKS=1 (debugging aid): events around every chunk's kernels; the run is synchronised and the start / end
-    // of each chunk relative to the job's first event printed to stderr
-    static const bool trace_chunks = getenv("SASA_B200_TRACE_CHUNKS") != nullptr;
-    std::vector<cudaEvent_t> trace_ev;
     // the large-structure workspace is shared by all chunks: keep such batches on a single stream
     const int nstreams = b->max_large_v[variant] || (grouped && params->n_points > 128) ? 1 : kStreams;
     if (gated) {
@@ -1252,20 +1181,8 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
             if (id_class) J_TRY(cudaMemcpyAsync(base_p + o_cls + ch.a0 * 4, id_class + ch.a0, na * 4, cudaMemcpyHostToDevice, st));
             if (grouped) J_TRY(cudaMemcpyAsync(base_p + o_grp + ch.a0 * 4, group + ch.a0, na * 4, cudaMemcpyHostToDevice, st));
         }
-        if (trace_chunks) {
-            cudaEvent_t e;
-            cudaEventCreate(&e);
-            cudaEventRecord(e, st);
-            trace_ev.push_back(e);
-        }
         if ((rc = enqueue_chunk(b, variant, ch, kbase, st, &job->launches, nullptr, grouped ? &gp : nullptr, masked ? &mp : nullptr)) != 0)
             return job_abort(ctx, job, rc);
-        if (trace_chunks) {
-            cudaEvent_t e;
-            cudaEventCreate(&e);
-            cudaEventRecord(e, st);
-            trace_ev.push_back(e);
-        }
         if (na && out->counts)
             J_TRY(cudaMemcpyAsync(out->counts + ch.a0, base_p + o_cnt + ch.a0 * 4, na * 4, cudaMemcpyDeviceToHost, st));
         if (na && out->atom_sasa)
@@ -1297,20 +1214,6 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
     ctx->tail_valid = true;
     J_TRY(cudaMemcpyAsync(job->h_status, d_status, 32, cudaMemcpyDeviceToHost, s0));
     J_TRY(cudaEventRecord(job->ev1, s0));
-    if (trace_chunks) {
-        cudaEventSynchronize(job->ev1);
-        float t_end = 0.f;
-        cudaEventElapsedTime(&t_end, job->ev0, job->ev1);
-        fprintf(stderr, "[sasa_b200] chunk trace (ms after the job's first event; whole job %.3f):", t_end);
-        for (size_t i = 0; i + 1 < trace_ev.size(); i += 2) {
-            float a = 0.f, z = 0.f;
-            cudaEventElapsedTime(&a, job->ev0, trace_ev[i]);
-            cudaEventElapsedTime(&z, job->ev0, trace_ev[i + 1]);
-            fprintf(stderr, " [%zu: %.3f-%.3f, %zu atoms]", i / 2, a, z, (size_t)(b->plan[variant][i / 2].a1 - b->plan[variant][i / 2].a0));
-        }
-        fprintf(stderr, "\n");
-        for (cudaEvent_t e : trace_ev) cudaEventDestroy(e);
-    }
     J_TRY(cudaFreeAsync(job->d_arena, s0));
     job->d_arena = nullptr;
 #undef J_TRY

@@ -62,8 +62,8 @@ struct KParams {
     // sphere points (SoA) and run parameters
     const float *px, *py, *pz;
     const uint4 *cap;             // cap table of this point set (sasa_cap.cuh), n_points <= 128 only; else null
-    unsigned long long cap_tex;   // the same table as a linear texture of uint4 (SASA_CAP_TEX: the fused kernel fetches its bins through
-                                  // the texture pipe, off the LSU data pipe that carries the shared-memory traffic); 0: none
+    unsigned long long cap_tex;   // the same table as a linear texture of uint4 (the fused kernel fetches its bins through the
+                                  // texture pipe, off the LSU data pipe that carries the shared-memory traffic); 0: none
     const uint4 *capm_in, *capm_rg;   // chunked cap table (inner / ring masks), 128 < n_points <= 1024; else null
     const float4 *pts4;           // the points as float4 (chunked cap path)
     CapDims capd;
@@ -126,18 +126,9 @@ struct Grid {
     int nx, ny, nz, e;
 };
 
-#ifndef SASA_OPT_LANEID
-#define SASA_OPT_LANEID 0      // 1: the lane index from %laneid (one S2R) instead of threadIdx.x & 31 (S2R + LOP3) wherever ptxas
-#endif                        // rematerialises it -- measured: 6 instructions per atom fewer but 1 % slower (r04b: 1,848 vs 1,868), off
-__device__ __forceinline__ int lane_id() {
-#if SASA_OPT_LANEID
-    unsigned l;
-    asm("mov.u32 %0, %%laneid;" : "=r"(l));
-    return (int)l;
-#else
-    return threadIdx.x & 31;
-#endif
-}
+// threadIdx.x & 31 rather than %laneid: the special register saves 6 instructions per atom where ptxas rematerialises the
+// lane index but measured 1 % slower (r04b: 1,848 vs 1,868 M atoms/s)
+__device__ __forceinline__ int lane_id() { return threadIdx.x & 31; }
 // A warp-uniform value routed through a warp reduction: REDUX writes a UNIFORM register, so ptxas may keep the value (and
 // what is computed from it) on the uniform datapath instead of in one of the 64 vector registers of every thread.
 __device__ __forceinline__ unsigned uniform_u32(unsigned v) { return __reduce_max_sync(kFull, v); }
@@ -378,12 +369,6 @@ __device__ __forceinline__ int gather_candidates(const KParams &p, const Grid &g
 
 // Register cache of the flattened candidate list of one cell: window w of lane l is candidate 32*w + l.
 // All atoms of a cell share it, so consecutive atoms of the same cell skip rows_of / row_lookup altogether.
-#ifndef SASA_FETCH
-#define SASA_FETCH 4
-#endif
-#ifndef SASA_PRELOAD
-#define SASA_PRELOAD 0
-#endif
 constexpr int kCacheWin = 12;   // 384 candidates; denser neighbourhoods use the uncached gather
 template <typename IdxT>
 struct CandCache {

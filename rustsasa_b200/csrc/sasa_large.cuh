@@ -304,10 +304,6 @@ __device__ __forceinline__ void large_blank_outputs(const KParams &p, int N, uin
 // profiles/r02a_cfg4_large_atoms.txt), compacts the neighbours into an index list and hands it to the cap-table
 // occlusion: cap_atom for n_points <= 128, capm_atom (chunked table) above.
 // ---------------------------------------------------------------------------------------------------------------------
-#ifndef SASA_OPT_LHDR
-#define SASA_OPT_LHDR 1       // large_stage / large_gather: division-free row header, predicated scan and position stores, neighbour list
-#endif                        // without capacity tests (as SASA_OPT_HDR / FILLP / NOGUARD of the fused kernel): cfg4 0.187 -> 0.185 ms,
-                              // cfg5 1.648 -> 1.614 ms (gpurun_out r04l)
 constexpr int kLCap = 288;    // staged candidates per cell block (largest seen at protein density: 266)
 constexpr int kLNb = 128;     // neighbours per atom on the fast path (protein lists peak around 75)
 
@@ -318,17 +314,15 @@ struct StagedAtoms {
 
 // Candidate rows of cell (cx, cy, cz) -> st[0, total) as atoms, padded to a multiple of 32 with far-away sentinels.
 // Returns total (-1: more than kLCap) and the staged index of the first atom of the cell itself.
+// The division-free row header, the predicated scan and position stores (as in tight_fill_list) and the neighbour list without
+// capacity tests (large_gather) took cfg4 0.187 -> 0.185 ms, cfg5 1.648 -> 1.614 ms (run r04l).
 __device__ __forceinline__ int large_stage(const Grid &g, const uint32_t *__restrict__ cells, const float4 *__restrict__ sorted,
                                            int cx, int cy, int cz, float4 *st, int &self0) {
     const int lane = lane_id();
     const int w = 2 * g.e + 1;
-#if SASA_OPT_LHDR
-    // as in tight_fill_list (SASA_OPT_HDR): lane / w by multiplication (w is 3 or 5), scan with the shuffle's own predicate
+    // as in tight_fill_list: lane / w by multiplication (w is 3 or 5), scan with the shuffle's own predicate
     const int q = g.e == 2 ? (lane * 13) >> 6 : (lane * 11) >> 5;
     const int dy = lane - q * w - g.e, dz = q - g.e;
-#else
-    const int dy = lane % w - g.e, dz = lane / w - g.e;
-#endif
     const int y = cy + dy, z = cz + dz;
     int start = 0, len = 0;
     if (lane < w * w && y >= 0 && y < g.ny && z >= 0 && z < g.nz) {
@@ -338,18 +332,10 @@ __device__ __forceinline__ int large_stage(const Grid &g, const uint32_t *__rest
         len = (int)__ldg(cells + base + x1 + 1) - start;
     }
     int incl = len;
-#if SASA_OPT_LHDR
 #pragma unroll
     for (int d = 1; d < 32; d <<= 1)
         asm volatile("{\n .reg .pred p;\n .reg .b32 t;\n shfl.sync.up.b32 t|p, %0, %1, 0, 0xffffffff;\n @p add.s32 %0, %0, t;\n}"
                      : "+r"(incl) : "r"(d));
-#else
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-        const int t = __shfl_up_sync(kFull, incl, d);
-        if (lane >= d) incl += t;
-    }
-#endif
     const int total = __shfl_sync(kFull, incl, 31);
     // the cell's own row is lane e * w + e; its atoms sit (first atom of the cell - row start) into that row
     const int self_lane = g.e * w + g.e;
@@ -358,7 +344,6 @@ __device__ __forceinline__ int large_stage(const Grid &g, const uint32_t *__rest
     if (total > kLCap) return -1;
     const int maxlen = __reduce_max_sync(kFull, len);
     // positions first (parked in the .x slot of the destination), then one coalesced-by-row copy of the atoms themselves
-#if SASA_OPT_LHDR
     {
         uint32_t dsts = (uint32_t)__cvta_generic_to_shared(st + (incl - len));
         int v = start, left = len;
@@ -374,20 +359,6 @@ __device__ __forceinline__ int large_stage(const Grid &g, const uint32_t *__rest
             dsts += 64; v += 4; left -= 4;
         }
     }
-#else
-    {
-        int *dst = reinterpret_cast<int *>(st + (incl - len));
-        int v = start, left = len;
-#pragma unroll 1
-        for (int t = 0; t < maxlen; t += 4) {
-            if (left > 0) dst[0] = v;
-            if (left > 1) dst[4] = v + 1;
-            if (left > 2) dst[8] = v + 2;
-            if (left > 3) dst[12] = v + 3;
-            dst += 16; v += 4; left -= 4;
-        }
-    }
-#endif
     __syncwarp();
     const int padded = (total + 31) & ~31;
 #pragma unroll 2
@@ -417,10 +388,10 @@ __device__ __forceinline__ int large_gather(const float4 *st, int total, int sel
         const bool acc0 = (d0 <= c0 * c0) & (w0 + lane != self), acc1 = (d1 <= c1 * c1) & (w0 + 32 + lane != self);
         const unsigned m0 = __ballot_sync(kFull, acc0), m1 = __ballot_sync(kFull, acc1);
         const int at0 = k + __popc(m0 & lt);
-        if (SASA_OPT_LHDR ? acc0 : (acc0 & (at0 < kLNb))) nb[at0] = (uint16_t)(w0 + lane);
+        if (acc0) nb[at0] = (uint16_t)(w0 + lane);
         k += __popc(m0);
         const int at1 = k + __popc(m1 & lt);
-        if (SASA_OPT_LHDR ? acc1 : (acc1 & (at1 < kLNb))) nb[at1] = (uint16_t)(w0 + 32 + lane);
+        if (acc1) nb[at1] = (uint16_t)(w0 + 32 + lane);
         k += __popc(m1);
     }
     if (w0 < total) {
@@ -431,7 +402,7 @@ __device__ __forceinline__ int large_gather(const float4 *st, int total, int sel
         const bool acc0 = (d0 <= c0 * c0) & (w0 + lane != self);
         const unsigned m0 = __ballot_sync(kFull, acc0);
         const int at0 = k + __popc(m0 & lt);
-        if (SASA_OPT_LHDR ? acc0 : (acc0 & (at0 < kLNb))) nb[at0] = (uint16_t)(w0 + lane);
+        if (acc0) nb[at0] = (uint16_t)(w0 + lane);
         k += __popc(m0);
     }
     __syncwarp();
@@ -468,14 +439,6 @@ __device__ __forceinline__ void large_blank_masks(const KParams &p, const MaskPa
     mask_zero_rows(mp, p.n_points, a0, (size_t)N, (size_t)blockIdx.x * blockDim.x + threadIdx.x, (size_t)gridDim.x * blockDim.x);
 }
 
-#ifndef SASA_LARGE_TEX
-#define SASA_LARGE_TEX 16384  // structures of at least this many atoms read the cap table through the texture path in the 100-point cells
-#endif                        // kernel too (SASA_CAP_TEX; 0: never).  Measured (gpurun_out r05d): cfg4, 150 k atoms, 0.1846 -> 0.1776 ms; one
-                              // call on one small structure gets SLOWER (1,283 atoms 79 -> 92 us, 2,622 atoms 77 -> 84 us: a texture fetch
-                              // has the longer latency and these runs are latency-bound), 19 k / 32 k atoms 120 -> 119 / 160 -> 153 us
-#ifndef SASA_OPT_ULARGE
-#define SASA_OPT_ULARGE 1
-#endif
 // HAS_MASK: every atom also writes its exposed-point mask row (mp); cold atoms stream.
 template <int NCHP, bool TEX, bool HAS_MASK>
 __device__ __forceinline__ void large_cells_body(const KParams &p, int N, uint32_t a0, LargeHeader *h, const float4 *__restrict__ sorted,
@@ -485,20 +448,20 @@ __device__ __forceinline__ void large_cells_body(const KParams &p, int N, uint32
     static_assert(kLCap * 16 >= kNbCap * 16 + kNbCap * 4 + 64, "the cold path's scratch must fit the staging strip");
     __shared__ __align__(16) float4 s_stage[8][kLCap];
     __shared__ __align__(16) uint32_t s_nbp[8][kLNb];
-    __shared__ __align__(16) uint16_t s_nb[8][SASA_OPT_LHDR ? kLCap : kLNb];   // SASA_OPT_LHDR: room for every staged candidate, no capacity test in the gather
+    __shared__ __align__(16) uint16_t s_nb[8][kLCap];   // room for every staged candidate: no capacity test in the gather
     __shared__ __align__(16) float4 s_ptab[NCHP == 1 ? 128 : 1];
     if (h->ncell == 0) {
         large_blank_outputs(p, N, a0);
         if (HAS_MASK) large_blank_masks(p, mp, N, a0);
         return;
     }
-    // the grid and the warp index on the uniform datapath (see SASA_OPT_UWARP / SASA_OPT_UGRID in sasa_tight.cuh).  Measured
+    // the grid and the warp index on the uniform datapath (as in tight_kernel_body).  Measured
     // (gpurun_out r04e): cfg4 (NCHP = 1) 0.1875 -> 0.1854 ms, cfg5 (NCHP = 8) 1.65 -> 2.00 ms -- the chunked cap path has no
     // vector registers to spare for the extra moves -- so only the 100-point instance takes it
     Grid g = h->grid;
     const int lane = lane_id();
     int warp = threadIdx.x >> 5;
-    if (SASA_OPT_ULARGE && NCHP == 1) {
+    if (NCHP == 1) {
         g.minx = uniform_f32(g.minx); g.miny = uniform_f32(g.miny); g.minz = uniform_f32(g.minz); g.inv_c = uniform_f32(g.inv_c);
         g.nx = uniform_i32(g.nx); g.ny = uniform_i32(g.ny); g.nz = uniform_i32(g.nz); g.e = uniform_i32(g.e);
         warp = uniform_i32(warp);
@@ -1020,7 +983,12 @@ inline int large_enqueue(int sm_count, LargeWorkspace &w, const KParams &kp, con
     if (mp) large_cells_masks_kernel<NCHP, TEX><<<ga, 256, 0, st>>>(kp, *mp, N, a0, w.hdr, w.sorted, w.orig, w.cells, w.bstart, w.val, blk); \
     else large_cells_kernel<NCHP, TEX><<<ga, 256, 0, st>>>(kp, N, a0, w.hdr, w.sorted, w.orig, w.cells, w.bstart, w.val, range_rank, range_n, blk)
             if (kp.n_points <= 128) {
-                if (SASA_CAP_TEX && SASA_LARGE_TEX > 0 && kp.cap_tex && N >= SASA_LARGE_TEX) {
+                // Structures of at least kLargeTexAtoms atoms read the cap table through the texture path, as the fused kernel does.
+                // Measured (run r05d): cfg4, 150 k atoms, 0.1846 -> 0.1776 ms; one call on one small structure gets SLOWER
+                // (1,283 atoms 79 -> 92 us, 2,622 atoms 77 -> 84 us: a texture fetch has the longer latency and these runs are
+                // latency-bound), 19 k / 32 k atoms 120 -> 119 / 160 -> 153 us.
+                constexpr int kLargeTexAtoms = 16384;
+                if (kp.cap_tex && N >= kLargeTexAtoms) {
                     SASA_LARGE_CELLS(1, true);
                 } else {
                     SASA_LARGE_CELLS(1, false);

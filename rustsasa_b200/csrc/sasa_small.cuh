@@ -128,7 +128,7 @@ struct SmemView {
     float4 *atom;       // cell-sorted atoms; atom[N] is the far-away sentinel of the tight kernel
     float *red;         // block reduction scratch
     int *misc;          // [0] structure claimed by the CTA, [1] work counter of the per-atom loop, [2..5] the next structure
-                        // (claim_next_and_prefetch), [6..7] statistics, [8..15] the cell grid (store_grid / load_grid)
+                        // (claim_next_and_prefetch), [6..7] statistics, [8..15] the cell grid (store_grid)
     float *val;         // per-atom exposed-point count, then area, by ORIGINAL index
     uint16_t *cellid, *rank;   // alias val during the counting sort
     uint32_t *cls;      // id classes in sorted order (HAS_CLS)
@@ -169,18 +169,11 @@ __device__ __forceinline__ void stage_points(const KParams &p, float4 *ptab) {
     }
 }
 
-// The structure's cell grid parked in misc[8..15] for code that would rather re-read it than hold eight registers (the
-// tight kernel's cold-path experiments, SASA_OPT_GRIDLD; volatile: the loads must stay where they are written).
+// The structure's cell grid parked in misc[8..15].  Nothing reads it back any more; the stores stay because dropping them
+// changes the SASS of every fused kernel, which wants a measurement of its own.
 __device__ __forceinline__ void store_grid(int *misc, const Grid &g) {
     misc[8] = __float_as_int(g.minx); misc[9] = __float_as_int(g.miny); misc[10] = __float_as_int(g.minz);
     misc[11] = __float_as_int(g.inv_c); misc[12] = g.nx; misc[13] = g.ny; misc[14] = g.nz; misc[15] = g.e;
-}
-__device__ __forceinline__ Grid load_grid(const int *misc) {
-    const volatile int *m = misc;
-    Grid g;
-    g.minx = __int_as_float(m[8]); g.miny = __int_as_float(m[9]); g.minz = __int_as_float(m[10]);
-    g.inv_c = __int_as_float(m[11]); g.nx = m[12]; g.ny = m[13]; g.nz = m[14]; g.e = m[15];
-    return g;
 }
 
 // One structure from raw float4 atoms to a cell-sorted shared-memory copy: bounds / r_max / finiteness (one fused
@@ -320,32 +313,26 @@ __device__ __forceinline__ float seq_sum(const float *v, int n, float t) {
 
 // Per-atom counts -> areas (coalesced stores), then the level sums in the reference's order: replaces the
 // numeric part of process_atoms (src/options.rs:195-232, :292-315, :370-410) and simd_sum (src/utils.rs:14-22).
-// AREA_READY: val already holds areas and the counts have been written (tight kernel).
 // Every sum keeps the reference's order (bit-identical results) but only the two chains that ARE sequential run on a
 // single thread: residue / chain sums are one thread each; the ProteinLevel polar / non-polar totals -- running sums of
 // the residue sums in residue order (src/options.rs:376-403) -- take the residue sums from a shared-memory scratch
 // (`scratch`: the per-warp blocks, idle between structures) instead of recomputing them with dependent loads; the global
 // total (src/options.rs:404) is seq_sum over all atoms.  The two chains run concurrently on threads 0 and 32.
-template <int NT, bool AREA_READY = false>
+template <int NT>
 __device__ __forceinline__ void structure_outputs(const KParams &p, const SmemView &V, uint32_t sid, uint32_t a0, int N,
                                                   unsigned char *scratch) {
     const int tid = threadIdx.x;
     constexpr int kScratch = (int)(((size_t)(NT / 32) * kWarpBlockBytes / 5) & ~(size_t)3);   // 4 B sum + 1 B polar flag each
     float *const s_sum = reinterpret_cast<float *>(scratch);
     uint8_t *const s_pol = scratch + (size_t)kScratch * 4;
-    if (AREA_READY) {
-        if (p.out_atom)
-            for (int i = tid; i < N; i += NT) p.out_atom[a0 + i] = V.val[i];
-    } else {
-        for (int i = tid; i < N; i += NT) {
-            const float cnt = V.val[i];
-            const float area = atom_area(p.xyz3 ? load_radius3(p, a0, i) : __ldg(p.xyzr + a0 + i).w, p.probe, cnt, p.inv_n);
-            if (p.out_counts) p.out_counts[a0 + i] = (uint32_t)cnt;
-            if (p.out_atom) p.out_atom[a0 + i] = area;
-            V.val[i] = area;
-        }
-        __syncthreads();
+    for (int i = tid; i < N; i += NT) {
+        const float cnt = V.val[i];
+        const float area = atom_area(p.xyz3 ? load_radius3(p, a0, i) : __ldg(p.xyzr + a0 + i).w, p.probe, cnt, p.inv_n);
+        if (p.out_counts) p.out_counts[a0 + i] = (uint32_t)cnt;
+        if (p.out_atom) p.out_atom[a0 + i] = area;
+        V.val[i] = area;
     }
+    __syncthreads();
     if (p.seg_be) {
         const uint32_t g0 = p.struct_seg_off[sid], g1 = p.struct_seg_off[sid + 1];
         if (p.out_protein) {
@@ -511,7 +498,7 @@ __device__ __forceinline__ void small_kernel_body(const KParams &p, const MaskPa
         // ---- per-atom work: warps pull runs of consecutive cell-sorted atoms from a shared counter ----------
         const SmemAtoms atoms{V.atom};
         unsigned pairs = 0, streamed = 0;
-        constexpr int kFetch = SASA_FETCH;
+        constexpr int kFetch = 4;   // atoms per claim
         CandCache<uint16_t> cc;
         for (;;) {
             int base = 0;

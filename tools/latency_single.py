@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Latency of ONE structure through sasa_b200_calculate_sasa_internal (host buffers, synchronous) -- BASELINE config 1.
-usage (GPU box): latency_single.py [names...]     env SASA_B200_CFGS selects the fused configurations (tuning aid)"""
+usage (GPU box): latency_single.py [names...]"""
 import os
 import sys
 import time
@@ -24,5 +24,5 @@ for name in sys.argv[1:] or ["151L_H3.pdb", "example.cif", "4xfj", "1hbn", "1jz8
     for _ in range(reps):
         eng.calculate_sasa_internal(x, None, 1.4, 100, -1)
     dt = (time.perf_counter() - t0) / reps
-    print(f"CFGS={os.environ.get('SASA_B200_CFGS', 'default'):8s} {name:14s} {x.shape[0]:6d} atoms  {dt * 1e6:8.1f} us/call  "
+    print(f"{name:14s} {x.shape[0]:6d} atoms  {dt * 1e6:8.1f} us/call  "
           f"{x.shape[0] / dt / 1e6:7.2f} M atoms/s", flush=True)

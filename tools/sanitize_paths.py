@@ -56,7 +56,7 @@ for n in (100, 960):
     sasa, counts = eng.calculate_sasa_internal(a.xyzr, None, 1.4, n, -1, want_counts=True)
     oo = orc.calculate_sasa_internal(a.xyzr, 1.4, n, threads=-1)
     check(f"one-structure call, large path, {n} points", np.array_equal(counts, oo["counts"]) and np.array_equal(sasa, oo["sasa"]))
-a17 = W.large_assembly(17000)   # >= SASA_LARGE_TEX atoms: the texture-path instance of the 100-point cells kernel
+a17 = W.large_assembly(17000)   # >= kLargeTexAtoms (16,384) atoms: the texture-path instance of the 100-point cells kernel
 sasa, counts = eng.calculate_sasa_internal(a17.xyzr, None, 1.4, 100, -1, want_counts=True)
 oo17 = orc.calculate_sasa_internal(a17.xyzr, 1.4, 100, threads=-1)
 check("one-structure call, large path with texture fetches, 100 points", np.array_equal(counts, oo17["counts"]) and np.array_equal(sasa, oo17["sasa"]))
