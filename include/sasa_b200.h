@@ -206,6 +206,27 @@ SASA_B200_API int sasa_b200_batch_run_masks_device(sasa_b200_batch *batch, const
                                      const sasa_b200_params *params, const sasa_b200_outputs *d_out,
                                      uint32_t *d_exposed, void *stream);
 
+/* Grouped runs with exposed-point masks: interface patches in one pass.
+ *   out / out_isolated  bit for bit what sasa_b200_batch_run_groups_* gives for the same input; every field nullable.
+ *   exposed             the layout of sasa_b200_batch_run_masks_*, and bit for bit that entry point's masks (the complex).
+ *   exposed_isolated    the same layout; atom i's row is its mask with its group standing alone (the engine's mask when the
+ *                       group's atoms run as their own structure).
+ * So popcount(exposed row i) == counts[i], popcount(exposed_isolated row i) == count_isolated[i], exposed[i] & ~exposed_isolated[i]
+ * == 0, and the points of atom i that other groups bury -- the interface patch -- are exposed_isolated[i] & ~exposed[i], with
+ * popcount count_isolated[i] - counts[i].  group == NULL, either mask pointer NULL with atoms in the batch, or a mask buffer
+ * size that overflows size_t: SASA_B200_ERR_INVALID_ARGUMENT; params->flags != 0: SASA_B200_ERR_UNSUPPORTED.  Non-finite input:
+ * SASA_B200_ERR_NON_FINITE with both output sets NaN-filled and both mask row sets zeroed for that structure.  The host form
+ * uses the per-chunk pipeline; the device form behaves like sasa_b200_batch_run_groups_device (stream-ordered, errors via
+ * sasa_b200_batch_sync). */
+SASA_B200_API int sasa_b200_batch_run_groups_masks_host(sasa_b200_batch *batch, const float *xyzr, const uint32_t *id_class,
+                                          const uint32_t *group, const sasa_b200_params *params, const sasa_b200_outputs *out,
+                                          const sasa_b200_outputs *out_isolated, uint32_t *exposed, uint32_t *exposed_isolated,
+                                          sasa_b200_stats *stats /* nullable */);
+SASA_B200_API int sasa_b200_batch_run_groups_masks_device(sasa_b200_batch *batch, const float *d_xyzr, const uint32_t *d_id_class,
+                                            const uint32_t *d_group, const sasa_b200_params *params, const sasa_b200_outputs *d_out,
+                                            const sasa_b200_outputs *d_out_isolated, uint32_t *d_exposed,
+                                            uint32_t *d_exposed_isolated, void *stream);
+
 /* MD-trajectory form (what mdsasa-bolt feeds calculate_sasa_internal per frame): a batch
  * created with S = n_frames equal-sized structures; xyz holds n_frames * n_atoms_per_frame
  * * 3 floats, radii n_atoms_per_frame floats shared by every frame (12 B/atom/frame on the

@@ -5,13 +5,14 @@ the thin Python host layer used by the tests and the benchmark: a ctypes binding
 Engine / Batch wrapper (``engine``) and a mirror of the reference's public interface for the path
 (``api``: ``calculate_sasa_internal``, ``SASAOptions`` ...).  There is no CPU fallback.
 """
-from .api import (Atom, AtomLevel, ChainLevel, ChainResult, ProteinLevel, ProteinResult, ResidueLevel,  # noqa: F401
-                  ResidueResult, SASACalcError, SASAOptions, SurfaceResult, calculate_sasa_internal, default_engine,
-                  surface_points)
+from .api import (Atom, AtomLevel, ChainLevel, ChainResult, InterfaceResult, InterfaceSurfaceResult,  # noqa: F401
+                  ProteinLevel, ProteinResult, ResidueLevel, ResidueResult, SASACalcError, SASAOptions, SurfaceResult,
+                  calculate_sasa_internal, default_engine, surface_points)
 from .engine import Batch, BatchResult, Engine, SasaB200Error  # noqa: F401
 from .structure import read_structure  # noqa: F401
 
 __all__ = ["Atom", "AtomLevel", "ResidueLevel", "ChainLevel", "ProteinLevel", "ChainResult", "ResidueResult",
-           "ProteinResult", "SASACalcError", "SASAOptions", "SurfaceResult", "calculate_sasa_internal", "default_engine",
+           "ProteinResult", "SASACalcError", "SASAOptions", "SurfaceResult", "InterfaceResult", "InterfaceSurfaceResult",
+           "calculate_sasa_internal", "default_engine",
            "surface_points", "Engine",
            "Batch", "BatchResult", "SasaB200Error", "read_structure"]

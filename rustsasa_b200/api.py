@@ -13,7 +13,8 @@ The numeric core is the C ABI (include/sasa_b200.h); there is no CPU path here.
 ``process_many`` is the batched form the CLI's directory mode (src/main.rs:342-480) maps onto.
 ``process_interface`` adds buried surface area: every structure in the complex and with each chain group standing alone,
 from one grouped batch call.  ``process_surface`` and ``surface_points`` give the dot surface: the solvent-accessible test
-points themselves, from the exposed-point masks of the same batch call.
+points themselves, from the exposed-point masks of the same batch call.  ``process_interface_surface`` gives both: the buried
+area and the interface patches, the test points that partner groups bury, from one grouped batch call with masks.
 """
 from __future__ import annotations
 
@@ -82,6 +83,16 @@ class SurfaceResult:
     """One structure of ``SASAOptions.process_surface``: the level's result, the exposed test points (M, 3) float32 and for
     each point the index of its atom in the order of an atom-level result (M,) int64."""
     result: Any
+    points: np.ndarray
+    atom_index: np.ndarray
+
+
+@dataclass
+class InterfaceSurfaceResult:
+    """One structure of ``SASAOptions.process_interface_surface``: the :class:`InterfaceResult` and the interface patches, the
+    test points exposed with the atom's group standing alone but buried in the complex, (M, 3) float32, with for each point
+    the index of its atom in the order of an atom-level result (M,) int64."""
+    interface: InterfaceResult
     points: np.ndarray
     atom_index: np.ndarray
 
@@ -204,6 +215,14 @@ class SASAOptions:
         whose extraction fails is reported as its ``SASACalcError``, as in ``process_many``."""
         return self._run_many(structures, engine, list(chain_groups) if chain_groups is not None else [])
 
+    def process_interface_surface(self, structures: Sequence[Structure], chain_groups: Optional[Sequence[str]] = None,
+                                  engine: Optional[Engine] = None) -> List:
+        """Interface patches: per structure an :class:`InterfaceSurfaceResult` with what ``process_interface`` gives for the
+        same arguments and the buried test points -- exposed with the atom's chain group standing alone, buried in the complex
+        -- all from ONE grouped batch call with exposed-point masks.  Chain grouping and error reporting are those of
+        ``process_interface``."""
+        return self._run_many(structures, engine, list(chain_groups) if chain_groups is not None else [], surface=True)
+
     @staticmethod
     def _chain_groups(atom_chain: np.ndarray, chain_groups: List[str]) -> np.ndarray:
         """Dense per-atom group labels of one structure."""
@@ -251,14 +270,13 @@ class SASAOptions:
         batch = Batch(eng, struct_off, seg_be if seg_be.shape[0] else None, seg_off if seg_be.shape[0] else None,
                       polar if seg_be.shape[0] else None)
         try:
-            if surface:
-                res = batch.run_masks_host(xyzr, id_class, self.probe_radius, self.n_points, want=want)
-            elif chain_groups is None:
-                res = batch.run_host(xyzr, id_class, self.probe_radius, self.n_points, want=want)
+            if chain_groups is None:
+                run = batch.run_masks_host if surface else batch.run_host
+                res = run(xyzr, id_class, self.probe_radius, self.n_points, want=want)
             else:   # the protein totals give the buried area: always requested
                 group = np.concatenate([self._chain_groups(packed[i].atom_chain, chain_groups) for i in good])
-                cpx, iso = batch.run_groups_host(xyzr, group, id_class, self.probe_radius, self.n_points,
-                                                 want=tuple(set(want) | {"protein"}))
+                run = batch.run_groups_masks_host if surface else batch.run_groups_host
+                cpx, iso = run(xyzr, group, id_class, self.probe_radius, self.n_points, want=tuple(set(want) | {"protein"}))
         finally:
             batch.close()
 
@@ -278,13 +296,18 @@ class SASAOptions:
             return ProteinResult(float(t[0]), float(t[1]), float(t[2]))
 
         for k, i in enumerate(good):
-            if surface:
-                a0, a1 = int(struct_off[k]), int(struct_off[k + 1])
+            a0, a1 = int(struct_off[k]), int(struct_off[k + 1])
+            if chain_groups is None and surface:
                 pts, atom = surface_points(xyzr[a0:a1], res.exposed[a0:a1], self.n_points, self.probe_radius)
                 results[i] = SurfaceResult(level_result(res, k, packed[i]), pts, atom)
             elif chain_groups is None:
                 results[i] = level_result(res, k, packed[i])
             else:
-                results[i] = InterfaceResult(level_result(cpx, k, packed[i]), level_result(iso, k, packed[i]),
-                                             float(iso.protein[k, 0]) - float(cpx.protein[k, 0]))
+                r = InterfaceResult(level_result(cpx, k, packed[i]), level_result(iso, k, packed[i]),
+                                    float(iso.protein[k, 0]) - float(cpx.protein[k, 0]))
+                if surface:
+                    buried = iso.exposed[a0:a1] & ~cpx.exposed[a0:a1]
+                    pts, atom = surface_points(xyzr[a0:a1], buried, self.n_points, self.probe_radius)
+                    r = InterfaceSurfaceResult(r, pts, atom)
+                results[i] = r
         return results

@@ -47,7 +47,7 @@ struct Points {
 };
 
 // The fused kernels of one shared-memory configuration, by attribute slot (kernel_slot).
-constexpr int kKernelSlots = 10;
+constexpr int kKernelSlots = 12;
 struct Proto {
     int nt, minb;
     uint32_t cmax;
@@ -55,9 +55,10 @@ struct Proto {
     const void *fn[kKernelSlots];
 };
 // Slots: plain runs has_cls + 2 * tight, masked runs 4 + the same (tight: n_points <= 128, no statistics / forced streaming),
-// grouped runs 8 + has_cls (always tight: they take no flags, and with n_points > 128 they take the large-structure path).
+// grouped runs 8 + has_cls and masked grouped runs 10 + has_cls (always tight: they take no flags, and with n_points > 128 they take
+// the large-structure path).
 int kernel_slot(bool grouped, bool masked, bool has_cls, bool tight) {
-    return grouped ? 8 + (has_cls ? 1 : 0) : (masked ? 4 : 0) + (has_cls ? 1 : 0) + (tight ? 2 : 0);
+    return grouped ? (masked ? 10 : 8) + (has_cls ? 1 : 0) : (masked ? 4 : 0) + (has_cls ? 1 : 0) + (tight ? 2 : 0);
 }
 #define SASA_PROTO(NT, MINB, CMAX)                                                                                     \
     Proto { NT, MINB, CMAX, { max_atoms(NT, MINB, CMAX, false), max_atoms(NT, MINB, CMAX, true),                       \
@@ -69,7 +70,9 @@ int kernel_slot(bool grouped, bool masked, bool has_cls, bool tight) {
               (const void *)sasa_tight_masks_kernel<NT, MINB, false, CMAX>,                                            \
               (const void *)sasa_tight_masks_kernel<NT, MINB, true, CMAX>,                                             \
               (const void *)sasa_tight_groups_kernel<NT, MINB, false, CMAX>,                                           \
-              (const void *)sasa_tight_groups_kernel<NT, MINB, true, CMAX> } }
+              (const void *)sasa_tight_groups_kernel<NT, MINB, true, CMAX>,                                            \
+              (const void *)sasa_tight_groups_masks_kernel<NT, MINB, false, CMAX>,                                     \
+              (const void *)sasa_tight_groups_masks_kernel<NT, MINB, true, CMAX> } }
 // Shared-memory configurations of the fused kernel.  nmax is derived from the per-CTA budget that lets `minb` CTAs share one SM
 // (228 KB per SM, 1 KB reserved per CTA, 227 KB per CTA max); both keep 32 warps resident per SM (64 registers/thread).
 const Proto kProtos[] = {SASA_PROTO(512, 2, 8192), SASA_PROTO(1024, 1, 16384)};
@@ -503,10 +506,11 @@ int check_params(sasa_b200_ctx *ctx, const sasa_b200_params *p) {
 // Enqueue every kernel of one chunk: the first fused launch on `st`, the others on sibling streams forked from and
 // joined back into `st` (so the caller still sees one stream-ordered unit of work).  Large-structure pipelines stay
 // on `st`.
-// gp: grouped runs (group labels and isolated outputs), else null.  mp: exposed-point masks, else null.
+// gp: grouped runs (group labels and isolated outputs), else null.  mp: exposed-point masks, else null.  mpi: the isolated
+// masks of a masked grouped run (gp and mp set), else null.
 int enqueue_chunk(sasa_b200_batch *b, int variant, const Chunk &ch, const KParams &base, cudaStream_t st,
                   uint32_t *launches, const uint32_t *order_override = nullptr, const GroupParams *gp = nullptr,
-                  const MaskParams *mp = nullptr) {
+                  const MaskParams *mp = nullptr, const MaskParams *mpi = nullptr) {
     sasa_b200_ctx *ctx = b->ctx;
     int n_small = 0;
     for (const Launch &L : ch.launches) n_small += L.cfg >= 0;
@@ -525,7 +529,7 @@ int enqueue_chunk(sasa_b200_batch *b, int variant, const Chunk &ch, const KParam
         if (L.cfg < 0 || all_large) {
             if (ctx->large_used) CU_TRY(ctx, cudaStreamWaitEvent(st, ctx->ev_large, 0));
             int rc = large_enqueue(ctx->sm_count, ctx->large, kp, &b->h_order[variant][L.order_off], L.n_work,
-                                   b->h_off.data(), b->h_seg_off.empty() ? nullptr : b->h_seg_off.data(), st, launches, 0, 1, gp, mp);
+                                   b->h_off.data(), b->h_seg_off.empty() ? nullptr : b->h_seg_off.data(), st, launches, 0, 1, gp, mp, mpi);
             if (rc != 0) return fail(ctx, rc, "large-structure path failed: %s", cudaGetErrorString(cudaGetLastError()));
             CU_TRY(ctx, cudaEventRecord(ctx->ev_large, st));
             ctx->large_used = true;
@@ -542,7 +546,8 @@ int enqueue_chunk(sasa_b200_batch *b, int variant, const Chunk &ch, const KParam
             ls = ctx->side[small_idx - 1];
             CU_TRY(ctx, cudaStreamWaitEvent(ls, ctx->ev_fork, 0));
         }
-        void *args[] = {(void *)&kp, mp ? (void *)mp : (void *)gp};
+        // (kernel arguments past the kernel's own are not read)
+        void *args[] = {(void *)&kp, gp ? (void *)gp : (void *)mp, (void *)mp, (void *)mpi};
         const bool tight = kp.n_points <= 128 && (kp.flags & 3u) == 0;
         const int slot = kernel_slot(grouped, mp != nullptr, has_cls, tight);
         const void *fn = kProtos[c.proto].fn[slot];
@@ -859,28 +864,30 @@ static int prepare_groups(sasa_b200_batch *b, const uint32_t *group, const sasa_
     return SASA_B200_OK;
 }
 
-// Checks of the masked entry points (after check_params): a mask buffer for every atom whose size fits a size_t.
-static int check_masks(sasa_b200_batch *b, const uint32_t *exposed, const sasa_b200_params *params) {
-    if (!exposed && b->n_atoms) return fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "exposed is NULL");
+// Checks of the masked entry points (after check_params): a mask buffer for every atom whose size fits a size_t.  name: the
+// buffer's argument name, for the error message.
+static int check_masks(sasa_b200_batch *b, const uint32_t *exposed, const sasa_b200_params *params, const char *name = "exposed") {
+    if (!exposed && b->n_atoms) return fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "%s is NULL", name);
     if (b->n_atoms && mask_words(params->n_points) > SIZE_MAX / 4 / b->n_atoms)
         return fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "the mask buffer (%zu atoms x %u words) overflows size_t", b->n_atoms,
                     mask_words(params->n_points));
     return SASA_B200_OK;
 }
 
-// d_iso: grouped runs; masked: d_exposed receives the exposed-point masks (one of the two at most).
+// d_iso: grouped runs; masked: d_exposed receives the exposed-point masks, and with d_iso d_exposed_iso the isolated ones.
 static int run_device_impl(sasa_b200_batch *b, const float *d_xyzr, const uint32_t *d_id_class, const uint32_t *d_group,
                            const sasa_b200_params *params, const sasa_b200_outputs *d_out, const sasa_b200_outputs *d_iso, void *stream,
-                           bool masked = false, uint32_t *d_exposed = nullptr) {
+                           bool masked = false, uint32_t *d_exposed = nullptr, uint32_t *d_exposed_iso = nullptr) {
     if (!b) return SASA_B200_ERR_INVALID_ARGUMENT;
     sasa_b200_ctx *ctx = b->ctx;
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (!d_out || (!d_xyzr && b->n_atoms)) return fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "d_xyzr / d_out is NULL");
     int rc = check_params(ctx, params);
     if (rc) return rc;
-    if (masked && (rc = check_masks(b, d_exposed, params)) != 0) return rc;
-    const MaskParams mp{d_exposed};
     const bool grouped = d_iso != nullptr;
+    if (masked && (rc = check_masks(b, d_exposed, params)) != 0) return rc;
+    if (masked && grouped && (rc = check_masks(b, d_exposed_iso, params, "exposed_isolated")) != 0) return rc;
+    const MaskParams mp{d_exposed}, mpi{d_exposed_iso};
     const int variant = (d_id_class ? 1 : 0) + 2 + (grouped ? 4 : 0);
     CU_TRY(ctx, cudaSetDevice(ctx->device));
     if (grouped && (rc = prepare_groups(b, d_group, params, d_iso, variant)) != 0) return rc;
@@ -899,7 +906,8 @@ static int run_device_impl(sasa_b200_batch *b, const float *d_xyzr, const uint32
     if (b->n_counters[variant])
         CU_TRY(ctx, cudaMemsetAsync(b->d_counters, 0, b->n_counters[variant] * sizeof(uint32_t), st));
     for (const Chunk &ch : b->plan[variant])
-        if ((rc = enqueue_chunk(b, variant, ch, base, st, &b->launches_last, nullptr, grouped ? &gp : nullptr, masked ? &mp : nullptr)) != 0)
+        if ((rc = enqueue_chunk(b, variant, ch, base, st, &b->launches_last, nullptr, grouped ? &gp : nullptr, masked ? &mp : nullptr,
+                                masked && grouped ? &mpi : nullptr)) != 0)
             return rc;
     return SASA_B200_OK;
 }
@@ -919,6 +927,14 @@ int sasa_b200_batch_run_groups_device(sasa_b200_batch *b, const float *d_xyzr, c
 int sasa_b200_batch_run_masks_device(sasa_b200_batch *b, const float *d_xyzr, const uint32_t *d_id_class, const sasa_b200_params *params,
                                      const sasa_b200_outputs *d_out, uint32_t *d_exposed, void *stream) {
     return run_device_impl(b, d_xyzr, d_id_class, nullptr, params, d_out, nullptr, stream, true, d_exposed);
+}
+
+int sasa_b200_batch_run_groups_masks_device(sasa_b200_batch *b, const float *d_xyzr, const uint32_t *d_id_class, const uint32_t *d_group,
+                                            const sasa_b200_params *params, const sasa_b200_outputs *d_out,
+                                            const sasa_b200_outputs *d_out_isolated, uint32_t *d_exposed, uint32_t *d_exposed_isolated,
+                                            void *stream) {
+    if (b && !d_out_isolated) return fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "d_out_isolated is NULL");
+    return run_device_impl(b, d_xyzr, d_id_class, d_group, params, d_out, d_out_isolated, stream, true, d_exposed, d_exposed_isolated);
 }
 
 int sasa_b200_batch_sync(sasa_b200_batch *b, sasa_b200_stats *stats) {
@@ -976,7 +992,7 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
                             const uint32_t *id_class, const sasa_b200_params *params, const sasa_b200_outputs *out,
                             sasa_b200_job **out_job, const uint8_t *ridx = nullptr, size_t n_palette = 0,
                             const uint32_t *group = nullptr, const sasa_b200_outputs *out_iso = nullptr, bool masked = false,
-                            uint32_t *exposed = nullptr) {
+                            uint32_t *exposed = nullptr, uint32_t *exposed_iso = nullptr) {
     sasa_b200_ctx *ctx = b->ctx;
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (!out || !out_job) return fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "out / out_job is NULL");
@@ -985,11 +1001,12 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
     if (b->in_flight) return fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "this batch already has a run in flight: wait for it first");
     int rc = check_params(ctx, params);
     if (rc) return rc;
+    const bool grouped = out_iso != nullptr;   // sasa_b200_batch_run_groups_host: per-chunk pipeline only
     if (masked && (rc = check_masks(b, exposed, params)) != 0) return rc;
+    if (masked && grouped && (rc = check_masks(b, exposed_iso, params, "exposed_isolated")) != 0) return rc;
     CU_TRY(ctx, cudaSetDevice(ctx->device));
     const size_t N = b->n_atoms, S = b->S, G = b->n_seg;
     const size_t W = mask_words(params->n_points);
-    const bool grouped = out_iso != nullptr;   // sasa_b200_batch_run_groups_host: per-chunk pipeline only
     const int variant = (id_class ? 1 : 0) + (grouped ? 4 : 0);
     if (grouped && (rc = prepare_groups(b, group, params, out_iso, variant)) != 0) return rc;
     const bool indexed = xyz3 != nullptr && ridx != nullptr;   // 13 B/atom: coordinates + a palette index per atom
@@ -1030,6 +1047,7 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
     const size_t o_iseg = o;   o += (grouped && out_iso->seg_sasa && G) ? al(G * 4) : 0;
     const size_t o_iprot = o;  o += (grouped && out_iso->protein) ? al(S * 12) : 0;
     const size_t o_mask = o;   o += masked ? al(N * W * 4) : 0;
+    const size_t o_imask = o;  o += (masked && grouped) ? al(N * W * 4) : 0;
     cudaStream_t s0 = ctx->streams[0];
     // the previous job may still be running on the sibling streams: this job's first stream starts behind all of them
     if (ctx->tail_valid)
@@ -1069,6 +1087,7 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
         gp.protein = out_iso->protein ? reinterpret_cast<float *>(base_p + o_iprot) : nullptr;
     }
     const MaskParams mp{masked ? reinterpret_cast<uint32_t *>(base_p + o_mask) : nullptr};
+    const MaskParams mpi{(masked && grouped) ? reinterpret_cast<uint32_t *>(base_p + o_imask) : nullptr};
     // ---- gated single-launch pipeline ----------------------------------------------------------------------------------
     // Thirteen launches of 148 persistent CTAs cost the pipelined run 0.25 ms over the same work as ONE launch (CTA start-ups
     // with a cold first structure, per-chunk instead of batch-wide queue; DESIGN.md section 6).  When every chunk of the plan is one
@@ -1181,7 +1200,8 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
             if (id_class) J_TRY(cudaMemcpyAsync(base_p + o_cls + ch.a0 * 4, id_class + ch.a0, na * 4, cudaMemcpyHostToDevice, st));
             if (grouped) J_TRY(cudaMemcpyAsync(base_p + o_grp + ch.a0 * 4, group + ch.a0, na * 4, cudaMemcpyHostToDevice, st));
         }
-        if ((rc = enqueue_chunk(b, variant, ch, kbase, st, &job->launches, nullptr, grouped ? &gp : nullptr, masked ? &mp : nullptr)) != 0)
+        if ((rc = enqueue_chunk(b, variant, ch, kbase, st, &job->launches, nullptr, grouped ? &gp : nullptr, masked ? &mp : nullptr,
+                                (masked && grouped) ? &mpi : nullptr)) != 0)
             return job_abort(ctx, job, rc);
         if (na && out->counts)
             J_TRY(cudaMemcpyAsync(out->counts + ch.a0, base_p + o_cnt + ch.a0 * 4, na * 4, cudaMemcpyDeviceToHost, st));
@@ -1204,6 +1224,8 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
             if (out_iso->protein && ch.s1 > ch.s0)
                 J_TRY(cudaMemcpyAsync(out_iso->protein + 3 * (size_t)ch.s0, base_p + o_iprot + 12 * (size_t)ch.s0,
                                       12 * (size_t)(ch.s1 - ch.s0), cudaMemcpyDeviceToHost, st));
+            if (na && masked)
+                J_TRY(cudaMemcpyAsync(exposed_iso + ch.a0 * W, base_p + o_imask + ch.a0 * W * 4, na * W * 4, cudaMemcpyDeviceToHost, st));
         }
     }
     // join the sibling streams into the first one, read the status words back, free the arena in stream order
@@ -1315,6 +1337,19 @@ int sasa_b200_batch_run_masks_host(sasa_b200_batch *b, const float *xyzr, const 
     if (!b) return SASA_B200_ERR_INVALID_ARGUMENT;
     sasa_b200_job *job = nullptr;
     int rc = submit_host_impl(b, xyzr, nullptr, nullptr, id_class, params, out, &job, nullptr, 0, nullptr, nullptr, true, exposed);
+    if (rc) return rc;
+    return wait_job_impl(job, stats);
+}
+
+int sasa_b200_batch_run_groups_masks_host(sasa_b200_batch *b, const float *xyzr, const uint32_t *id_class, const uint32_t *group,
+                                          const sasa_b200_params *params, const sasa_b200_outputs *out,
+                                          const sasa_b200_outputs *out_isolated, uint32_t *exposed, uint32_t *exposed_isolated,
+                                          sasa_b200_stats *stats) {
+    if (!b) return SASA_B200_ERR_INVALID_ARGUMENT;
+    if (!out_isolated) return fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "out_isolated is NULL");
+    sasa_b200_job *job = nullptr;
+    int rc = submit_host_impl(b, xyzr, nullptr, nullptr, id_class, params, out, &job, nullptr, 0, group, out_isolated, true, exposed,
+                              exposed_isolated);
     if (rc) return rc;
     return wait_job_impl(job, stats);
 }

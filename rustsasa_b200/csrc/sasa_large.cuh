@@ -665,17 +665,25 @@ __device__ __forceinline__ float large_eval_atom(const KParams &p, const Grid &g
 // Atoms kernel of grouped runs: every atom in the complex and with its group standing alone.  n_points <= 128: one pass with
 // cap_atom_groups over the complex neighbour list; otherwise (and for atoms with more than kNbCap neighbours) two evaluations,
 // the second with the atoms of other groups hidden (GroupAtoms).  Writes val (complex areas) and val_iso.
-__global__ void __launch_bounds__(256, 2) large_groups_kernel(const KParams p, const GroupParams gp, int N, uint32_t a0, LargeHeader *h,
-                                                              const float4 *__restrict__ sorted, const uint32_t *__restrict__ orig,
-                                                              const uint32_t *__restrict__ cls_sorted, const uint32_t *__restrict__ grp_sorted,
-                                                              const uint32_t *__restrict__ cells, const uint32_t *__restrict__ bstart,
-                                                              float *val, float *val_iso, uint32_t blk) {
+// HAS_MASK: every atom also writes its mask row in the complex (mp) and with its group standing alone (mpi).  The cap path
+// writes both from cap_atom_groups; every other atom (n_points > 128, more than kNbCap neighbours) streams both evaluations,
+// because atom_fast keeps no per-point result.
+template <bool HAS_MASK>
+__device__ __forceinline__ void large_groups_body(const KParams &p, const GroupParams &gp, int N, uint32_t a0, LargeHeader *h,
+                                                  const float4 *__restrict__ sorted, const uint32_t *__restrict__ orig,
+                                                  const uint32_t *__restrict__ cls_sorted, const uint32_t *__restrict__ grp_sorted,
+                                                  const uint32_t *__restrict__ cells, const uint32_t *__restrict__ bstart, float *val,
+                                                  float *val_iso, uint32_t blk, const MaskParams &mp, const MaskParams &mpi) {
     __shared__ __align__(16) float4 s_ent[8 * kNbCap];
     __shared__ uint32_t s_cand[8 * kNbCap];
     __shared__ __align__(16) float4 s_ptab[128];
     if (h->ncell == 0) {
         large_blank_outputs(p, N, a0);
         large_blank_outputs(iso_outputs(p, gp), N, a0);
+        if (HAS_MASK) {
+            large_blank_masks(p, mp, N, a0);
+            large_blank_masks(p, mpi, N, a0);
+        }
         return;
     }
     const Grid g = h->grid;
@@ -706,18 +714,30 @@ __global__ void __launch_bounds__(256, 2) large_groups_kernel(const KParams p, c
         for (int pos = (int)__ldg(bstart + b); pos < pend; ++pos) {
             const float4 ai = atoms(pos);
             const uint32_t gi = __ldg(grp_sorted + pos);
-            const int cx = cell_coord(ai.x, g.minx, g.inv_c, g.nx), cy = cell_coord(ai.y, g.miny, g.inv_c, g.ny),
-                      cz = cell_coord(ai.z, g.minz, g.inv_c, g.nz);
-            const int cid = (cz * g.ny + cy) * g.nx + cx;
-            if (cid != cc.cell) fill_cache(g, cells, cx, cy, cz, cid, cc);
-            const int k = cc.total >= 0 ? gather_cached(p, atoms, cls_sorted, pos, ai, cc, w_cand)
-                                        : gather_candidates(p, g, atoms, cells, cls_sorted, pos, ai, w_cand);
+            int k = -1;
+            if (!HAS_MASK || use_cap) {
+                const int cx = cell_coord(ai.x, g.minx, g.inv_c, g.nx), cy = cell_coord(ai.y, g.miny, g.inv_c, g.ny),
+                          cz = cell_coord(ai.z, g.minz, g.inv_c, g.nz);
+                const int cid = (cz * g.ny + cy) * g.nx + cx;
+                if (cid != cc.cell) fill_cache(g, cells, cx, cy, cz, cid, cc);
+                k = cc.total >= 0 ? gather_cached(p, atoms, cls_sorted, pos, ai, cc, w_cand)
+                                  : gather_candidates(p, g, atoms, cells, cls_sorted, pos, ai, w_cand);
+            }
+            uint32_t *const mrow = HAS_MASK ? mask_row(mp, p.n_points, a0 + orig[pos]) : nullptr;
+            uint32_t *const irow = HAS_MASK ? mask_row(mpi, p.n_points, a0 + orig[pos]) : nullptr;
             float cnt, cnt_iso;
             if (k >= 0) pairs += (unsigned)k;
             if (k >= 0 && use_cap) {
                 int iso;
-                cnt = (float)cap_atom_groups(p.cap, atoms, ai, p.probe, w_cand, k, grp_sorted, gi, s_ptab, (int)p.n_points, nbody, 0ull, &iso);
+                cnt = (float)cap_atom_groups<false, HAS_MASK>(p.cap, atoms, ai, p.probe, w_cand, k, grp_sorted, gi, s_ptab, (int)p.n_points,
+                                                              nbody, 0ull, &iso, mrow, irow);
                 cnt_iso = (float)iso;
+            } else if (HAS_MASK) {
+                cnt = atom_streaming<GlobalAtoms, uint32_t, false, true>(p, g, atoms, cells, cls_sorted, pos, w_ent, nullptr, mrow);
+                __syncwarp();
+                cnt_iso = atom_streaming<GroupAtoms<true>, uint32_t, false, true>(p, g, GroupAtoms<true>{sorted, grp_sorted, gi}, cells,
+                                                                                  cls_sorted, pos, w_ent, nullptr, irow);
+                streamed += 2;
             } else {
                 cnt = large_eval_atom(p, g, atoms, cells, cls_sorted, pos, ai, k, w_cand, w_ent, s_pts, streamed);
                 __syncwarp();
@@ -736,6 +756,24 @@ __global__ void __launch_bounds__(256, 2) large_groups_kernel(const KParams p, c
         if (pairs) atomicAdd(p.stat + 1, pairs);
         if (streamed) atomicAdd(p.stat + 2, streamed);
     }
+}
+
+__global__ void __launch_bounds__(256, 2) large_groups_kernel(const KParams p, const GroupParams gp, int N, uint32_t a0, LargeHeader *h,
+                                                              const float4 *__restrict__ sorted, const uint32_t *__restrict__ orig,
+                                                              const uint32_t *__restrict__ cls_sorted, const uint32_t *__restrict__ grp_sorted,
+                                                              const uint32_t *__restrict__ cells, const uint32_t *__restrict__ bstart,
+                                                              float *val, float *val_iso, uint32_t blk) {
+    large_groups_body<false>(p, gp, N, a0, h, sorted, orig, cls_sorted, grp_sorted, cells, bstart, val, val_iso, blk, MaskParams{},
+                             MaskParams{});
+}
+
+__global__ void __launch_bounds__(256, 2) large_groups_masks_kernel(const KParams p, const GroupParams gp, const MaskParams mp,
+                                                                    const MaskParams mpi, int N, uint32_t a0, LargeHeader *h,
+                                                                    const float4 *__restrict__ sorted, const uint32_t *__restrict__ orig,
+                                                                    const uint32_t *__restrict__ cls_sorted,
+                                                                    const uint32_t *__restrict__ grp_sorted, const uint32_t *__restrict__ cells,
+                                                                    const uint32_t *__restrict__ bstart, float *val, float *val_iso, uint32_t blk) {
+    large_groups_body<true>(p, gp, N, a0, h, sorted, orig, cls_sorted, grp_sorted, cells, bstart, val, val_iso, blk, mp, mpi);
 }
 
 __device__ __forceinline__ float warp_sum_range(const float *v, uint32_t b, uint32_t e) {
@@ -934,11 +972,11 @@ inline int large_reserve(LargeWorkspace &w, uint32_t n_atoms) {
 // (BASELINE cfg5): the cell list is built for the whole structure, only the work blocks owned by `range_rank` are
 // evaluated, and no sums are produced.  Grouped runs (gp set; no atom-range split, no flags) go through
 // large_groups_kernel and produce the level sums of both value vectors.  Masked runs (mp set; no atom-range split) take the
-// masked instantiations of the cells / atoms kernels.
+// masked instantiations of the cells / atoms kernels; masked grouped runs (gp, mp and mpi set) large_groups_masks_kernel.
 inline int large_enqueue(int sm_count, LargeWorkspace &w, const KParams &kp, const uint32_t *order, uint32_t n_work,
                          const uint32_t *off, const uint32_t *seg_off, cudaStream_t st, uint32_t *launches,
                          uint32_t range_rank = 0, uint32_t range_n = 1, const GroupParams *gp = nullptr,
-                         const MaskParams *mp = nullptr) {
+                         const MaskParams *mp = nullptr, const MaskParams *mpi = nullptr) {
     for (uint32_t q = 0; q < n_work; ++q) {
         const uint32_t sid = order[q];
         const uint32_t a0 = off[sid];
@@ -973,8 +1011,12 @@ inline int large_enqueue(int sm_count, LargeWorkspace &w, const KParams &kp, con
         if (gp) {
             large_scatter_groups_kernel<<<gc, 256, 0, st>>>(gp->grp + a0, N, w.hdr, w.cells, w.cellid, w.rank, w.grp_sorted);
             const int ga = std::max(1, std::min((N + 8 * (int)blk - 1) / (8 * (int)blk), sm_count * 2));
-            large_groups_kernel<<<ga, 256, 0, st>>>(kp, *gp, N, a0, w.hdr, w.sorted, w.orig, cls ? w.cls_sorted : nullptr, w.grp_sorted, w.cells,
-                                                    w.bstart, w.val, w.val_iso, blk);
+            if (mp)
+                large_groups_masks_kernel<<<ga, 256, 0, st>>>(kp, *gp, *mp, *mpi, N, a0, w.hdr, w.sorted, w.orig, cls ? w.cls_sorted : nullptr,
+                                                              w.grp_sorted, w.cells, w.bstart, w.val, w.val_iso, blk);
+            else
+                large_groups_kernel<<<ga, 256, 0, st>>>(kp, *gp, N, a0, w.hdr, w.sorted, w.orig, cls ? w.cls_sorted : nullptr, w.grp_sorted,
+                                                        w.cells, w.bstart, w.val, w.val_iso, blk);
             *launches += 1;
         } else if (!cls && (kp.flags & 3u) == 0 && table) {
             const int ga = std::max(1, std::min((owned + 8 * (int)blk - 1) / (8 * (int)blk), sm_count * 4));

@@ -212,13 +212,22 @@ __device__ __noinline__ int tight_cold_atom_iso(const float *px, const float *py
     return tight_cold_eval<HAS_CLS>(px, py, pz, n_points, n_body, probe, near2, m_min, m_max, g, GroupAtoms<false>{s_atom, s_grp, s_grp[pos]},
                                     s_cell, s_cls, s_pts, pos, ent, cand, misc);
 }
+// The isolated evaluation of a masked grouped run: the atom streams with its group standing alone and writes its isolated row.
+template <bool HAS_CLS>
+__device__ __noinline__ int tight_cold_atom_iso_mask(const float *px, const float *py, const float *pz, uint32_t n_points, uint32_t n_body,
+                                                     float probe, Grid g, const float4 *s_atom, const uint32_t *s_grp, const uint16_t *s_cell,
+                                                     const uint32_t *s_cls, int pos, float4 *ent, int *misc, uint32_t *irow) {
+    return tight_cold_eval<HAS_CLS, GroupAtoms<false>, true>(px, py, pz, n_points, n_body, probe, 0.0f, 0, 0, g,
+                                                             GroupAtoms<false>{s_atom, s_grp, s_grp[pos]}, s_cell, s_cls, nullptr, pos, ent,
+                                                             nullptr, misc, irow);
+}
 
 // HAS_GRP: grouped run -- every atom is evaluated in the complex and with its group standing alone (the cap path in one pass,
 // cap_atom_groups; the cold path twice), and the output stage runs once per value array.
-// HAS_MASK: every atom also writes its exposed-point mask row (mp); cold atoms stream.
+// HAS_MASK: every atom also writes its exposed-point mask row (mp); cold atoms stream.  With HAS_GRP also its isolated row (mpi).
 template <int NT, int MINB, bool HAS_CLS, uint32_t CMAX, bool HAS_GRP, bool HAS_MASK = false>
-__device__ __forceinline__ void tight_kernel_body(const KParams &p, const GroupParams &gp, const MaskParams &mp = MaskParams{}) {
-    static_assert(!(HAS_GRP && HAS_MASK), "grouped runs write no masks");
+__device__ __forceinline__ void tight_kernel_body(const KParams &p, const GroupParams &gp, const MaskParams &mp = MaskParams{},
+                                                  const MaskParams &mpi = MaskParams{}) {
     extern __shared__ __align__(16) unsigned char smem[];
     constexpr int NW = NT / 32;
     constexpr uint32_t NMAX = max_atoms(NT, MINB, CMAX, HAS_CLS, HAS_GRP);
@@ -252,6 +261,7 @@ __device__ __forceinline__ void tight_kernel_body(const KParams &p, const GroupP
         if (warp == 0) claim_next_and_prefetch(p, V.misc);   // every structure, also after a rejected one
         if (!ok) {
             if (HAS_MASK) mask_zero_rows(mp, p.n_points, a0, (size_t)N, threadIdx.x, NT);
+            if (HAS_GRP && HAS_MASK) mask_zero_rows(mpi, p.n_points, a0, (size_t)N, threadIdx.x, NT);
             continue;
         }
         // the structure's cell grid (eight CTA-uniform values) in uniform registers
@@ -320,10 +330,11 @@ __device__ __forceinline__ void tight_kernel_body(const KParams &p, const GroupP
                                        : kNbCap + 1;
                     int cnt_iso = 0;
                     uint32_t *const mrow = HAS_MASK ? mask_row(mp, p.n_points, a0 + V.orig[pos]) : nullptr;
+                    uint32_t *const irow = HAS_GRP && HAS_MASK ? mask_row(mpi, p.n_points, a0 + V.orig[pos]) : nullptr;
                     if (k <= kNbCap) {
                         if (HAS_GRP)
-                            cnt = cap_atom_groups<true>(p.cap, SmemAtoms{V.atom}, ai, p.probe, w_nba, k, V.grp, V.grp[pos], V.ptab,
-                                                        (int)p.n_points, nbody, p.cap_tex, &cnt_iso);
+                            cnt = cap_atom_groups<true, HAS_MASK>(p.cap, SmemAtoms{V.atom}, ai, p.probe, w_nba, k, V.grp, V.grp[pos], V.ptab,
+                                                                  (int)p.n_points, nbody, p.cap_tex, &cnt_iso, mrow, irow);
                         else
                             cnt = cap_atom<true, HAS_MASK>(p.cap, SmemAtoms{V.atom}, ai, p.probe, w_nba, k, V.ptab, (int)p.n_points, nbody,
                                                            p.cap_tex, mrow);
@@ -331,6 +342,9 @@ __device__ __forceinline__ void tight_kernel_body(const KParams &p, const GroupP
                     } else if (HAS_MASK) {
                         cnt = tight_cold_atom_mask<HAS_CLS>(p.px, p.py, p.pz, p.n_points, p.n_body, p.probe, g, V.atom, V.cell, V.cls, pos,
                                                             w_ent, V.misc, mrow);
+                        if (HAS_GRP)
+                            cnt_iso = tight_cold_atom_iso_mask<HAS_CLS>(p.px, p.py, p.pz, p.n_points, p.n_body, p.probe, g, V.atom, V.grp,
+                                                                        V.cell, V.cls, pos, w_ent, V.misc, irow);
                     } else {
                         cnt = tight_cold_atom<HAS_CLS>(p.px, p.py, p.pz, p.n_points, p.n_body, p.probe, p.near2, p.m_min, p.m_max,
                                                        g, V.atom, V.cell, V.cls, V.ptab, pos, w_ent, w_cand, V.misc);
@@ -378,6 +392,14 @@ __global__ void __launch_bounds__(NT, MINB) sasa_tight_masks_kernel(const KParam
 template <int NT, int MINB, bool HAS_CLS, uint32_t CMAX>
 __global__ void __launch_bounds__(NT, MINB) sasa_tight_groups_kernel(const KParams p, const GroupParams gp) {
     tight_kernel_body<NT, MINB, HAS_CLS, CMAX, true>(p, gp);
+}
+
+// Grouped runs with exposed-point masks (n_points <= 128): the grouped run's outputs plus every atom's mask row in the complex
+// (mp) and with its group standing alone (mpi).
+template <int NT, int MINB, bool HAS_CLS, uint32_t CMAX>
+__global__ void __launch_bounds__(NT, MINB) sasa_tight_groups_masks_kernel(const KParams p, const GroupParams gp, const MaskParams mp,
+                                                                           const MaskParams mpi) {
+    tight_kernel_body<NT, MINB, HAS_CLS, CMAX, true, true>(p, gp, mp, mpi);
 }
 
 }  // namespace sasa

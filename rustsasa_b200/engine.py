@@ -80,7 +80,8 @@ class BatchResult:
     seg_sasa: Optional[np.ndarray] = None
     protein: Optional[np.ndarray] = None   # (S, 3): global, polar, non-polar
     stats: Optional[dict] = None
-    exposed: Optional[np.ndarray] = None   # (n_atoms, W) uint32 exposed-point masks (run_masks_host), W = ceil(n_points / 32)
+    exposed: Optional[np.ndarray] = None   # (n_atoms, W) uint32 exposed-point masks (run_masks_host, run_groups_masks_host),
+                                           # W = ceil(n_points / 32)
 
 
 class Engine:
@@ -309,30 +310,69 @@ class Batch:
         cpx.stats = iso.stats = st.as_dict()
         return cpx, iso
 
+    def _device_outputs(self, want, dev) -> BatchResult:
+        import torch
+        r = BatchResult()
+        if "counts" in want:
+            r.counts = torch.zeros(self.n_atoms, dtype=torch.int32, device=dev)
+        if "atom" in want:
+            r.atom_sasa = torch.zeros(self.n_atoms, dtype=torch.float32, device=dev)
+        if "seg" in want and self.n_seg:
+            r.seg_sasa = torch.zeros(self.n_seg, dtype=torch.float32, device=dev)
+        if "protein" in want:
+            r.protein = torch.zeros((max(self.S, 0), 3), dtype=torch.float32, device=dev)
+        return r
+
     def run_groups_device(self, d_xyzr, d_group, d_id_class=None, probe_radius=1.4, n_points=100, simd_lanes=8, flags=0,
                           want=("counts", "atom", "seg", "protein"), stream=None):
         """run_groups_host on torch CUDA tensors: allocates the outputs on the input's device, enqueues on `stream` (None =
         torch's current stream) and returns (complex, isolated) BatchResults of tensors without synchronising."""
-        import torch
-        dev = d_xyzr.device
-
-        def outputs():
-            r = BatchResult()
-            if "counts" in want:
-                r.counts = torch.zeros(self.n_atoms, dtype=torch.int32, device=dev)
-            if "atom" in want:
-                r.atom_sasa = torch.zeros(self.n_atoms, dtype=torch.float32, device=dev)
-            if "seg" in want and self.n_seg:
-                r.seg_sasa = torch.zeros(self.n_seg, dtype=torch.float32, device=dev)
-            if "protein" in want:
-                r.protein = torch.zeros((max(self.S, 0), 3), dtype=torch.float32, device=dev)
-            return r
-        cpx, iso = outputs(), outputs()
+        cpx, iso = self._device_outputs(want, d_xyzr.device), self._device_outputs(want, d_xyzr.device)
         outs = [_lib.Outputs(_ptr(r.counts), _ptr(r.atom_sasa), _ptr(r.seg_sasa), _ptr(r.protein)) for r in (cpx, iso)]
         prm = self._params(probe_radius, n_points, simd_lanes, flags)
         self.engine._check(self._L.sasa_b200_batch_run_groups_device(self._h, _ptr(d_xyzr), _ptr(d_id_class), _ptr(d_group),
                                                                     C.byref(prm), C.byref(outs[0]), C.byref(outs[1]),
                                                                     _stream(stream)))
+        return cpx, iso
+
+    def run_groups_masks_host(self, xyzr, group, id_class=None, probe_radius=1.4, n_points=100, simd_lanes=8, flags=0,
+                              want=("counts", "atom", "seg", "protein")):
+        """run_groups_host plus the exposed-point masks of both evaluations: complex.exposed is run_masks_host's mask, and
+        isolated.exposed every atom's mask with its group standing alone, each (n_atoms, W) uint32.  The interface patch -- the
+        points of atom i that other groups bury -- is ``isolated.exposed[i] & ~complex.exposed[i]``."""
+        xyzr = _np(xyzr, np.float32, (-1, 4))
+        assert xyzr.shape[0] == self.n_atoms, "xyzr does not match struct_off"
+        group = _np(group, np.uint32)
+        assert group is None or group.shape[0] == self.n_atoms, "group does not match struct_off"
+        id_class = _np(id_class, np.uint32)
+        cpx, iso = self._host_outputs(want, "numpy"), self._host_outputs(want, "numpy")
+        for r in (cpx, iso):
+            r.exposed = np.zeros((self.n_atoms, (n_points + 31) // 32), np.uint32)
+        outs = [_lib.Outputs(_ptr(r.counts), _ptr(r.atom_sasa), _ptr(r.seg_sasa), _ptr(r.protein)) for r in (cpx, iso)]
+        prm = self._params(probe_radius, n_points, simd_lanes, flags)
+        st = _lib.Stats()
+        self.engine._check(self._L.sasa_b200_batch_run_groups_masks_host(
+            self._h, _ptr(xyzr), _ptr(id_class), _ptr(group), C.byref(prm), C.byref(outs[0]), C.byref(outs[1]), _ptr(cpx.exposed),
+            _ptr(iso.exposed), C.byref(st)))
+        cpx.stats = iso.stats = st.as_dict()
+        return cpx, iso
+
+    def run_groups_masks_device(self, d_xyzr, d_group, d_exposed, d_exposed_isolated, d_id_class=None, probe_radius=1.4,
+                                n_points=100, simd_lanes=8, flags=0, want=("counts", "atom", "seg", "protein"), stream=None):
+        """run_groups_device plus the masks of both evaluations into ``d_exposed`` (complex) and ``d_exposed_isolated``, torch
+        CUDA tensors of n_atoms * ceil(n_points / 32) 32-bit words each.  Returns (complex, isolated) BatchResults of tensors,
+        with ``exposed`` set to the two mask tensors, without synchronising."""
+        W = (n_points + 31) // 32
+        for m in (d_exposed, d_exposed_isolated):
+            if m is not None:
+                assert m.numel() * m.element_size() >= self.n_atoms * W * 4, "mask tensor is too small"
+        cpx, iso = self._device_outputs(want, d_xyzr.device), self._device_outputs(want, d_xyzr.device)
+        cpx.exposed, iso.exposed = d_exposed, d_exposed_isolated
+        outs = [_lib.Outputs(_ptr(r.counts), _ptr(r.atom_sasa), _ptr(r.seg_sasa), _ptr(r.protein)) for r in (cpx, iso)]
+        prm = self._params(probe_radius, n_points, simd_lanes, flags)
+        self.engine._check(self._L.sasa_b200_batch_run_groups_masks_device(
+            self._h, _ptr(d_xyzr), _ptr(d_id_class), _ptr(d_group), C.byref(prm), C.byref(outs[0]), C.byref(outs[1]),
+            _ptr(d_exposed), _ptr(d_exposed_isolated), _stream(stream)))
         return cpx, iso
 
     def run_atom_range_device(self, d_xyzr, rank: int, n_ranks: int, d_id_class=None, probe_radius=1.4, n_points=100,

@@ -52,6 +52,31 @@ def other_group_fraction(d, group, probe, n_sample):
     return hit / max(tot, 1)
 
 
+def plane_groups(struct_off, xyzr, seed):
+    """Two groups per structure: the sides of a random plane through its centroid."""
+    rng = np.random.default_rng(seed)
+    group = np.empty(xyzr.shape[0], np.uint32)
+    for s in range(len(struct_off) - 1):
+        a0, a1 = int(struct_off[s]), int(struct_off[s + 1])
+        x = xyzr[a0:a1, :3].astype(np.float64)
+        nrm = rng.normal(size=3)
+        group[a0:a1] = ((x - x.mean(axis=0)) @ nrm > 0.0).astype(np.uint32)
+    return group
+
+
+def split_order(struct_off, group):
+    """The two-run baseline's rebuilt batch: per structure the atoms of group 0, then those of group 1, each a structure of its
+    own.  Returns (perm, split_off): rebuilt atom k is original atom perm[k]."""
+    perm, split_off = [], [0]
+    for s in range(len(struct_off) - 1):
+        a0, a1 = int(struct_off[s]), int(struct_off[s + 1])
+        for g in (0, 1):
+            idx = a0 + np.nonzero(group[a0:a1] == g)[0]
+            perm.append(idx)
+            split_off.append(split_off[-1] + idx.size)
+    return np.concatenate(perm), np.asarray(split_off, np.uint64)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--structures", type=int, default=4400)
@@ -63,24 +88,9 @@ def main():
     from rustsasa_b200 import Engine, workloads as W
     probe, n_points = 1.4, 100
     d = W.proteome_batch(args.structures, seed=W.SEED)
-    rng = np.random.default_rng(W.SEED + 17)
     S, N = len(d.struct_off) - 1, d.n_atoms
-    group = np.empty(N, np.uint32)
-    for s in range(S):
-        a0, a1 = int(d.struct_off[s]), int(d.struct_off[s + 1])
-        x = d.xyzr[a0:a1, :3].astype(np.float64)
-        nrm = rng.normal(size=3)
-        group[a0:a1] = ((x - x.mean(axis=0)) @ nrm > 0.0).astype(np.uint32)
-    # (c)'s rebuilt batch: per structure the atoms of group 0, then those of group 1, each a structure of its own
-    perm, split_off = [], [0]
-    for s in range(S):
-        a0, a1 = int(d.struct_off[s]), int(d.struct_off[s + 1])
-        for g in (0, 1):
-            idx = a0 + np.nonzero(group[a0:a1] == g)[0]
-            perm.append(idx)
-            split_off.append(split_off[-1] + idx.size)
-    perm = np.concatenate(perm)
-    split_off = np.asarray(split_off, np.uint64)
+    group = plane_groups(d.struct_off, d.xyzr, W.SEED + 17)
+    perm, split_off = split_order(d.struct_off, group)   # (c)'s rebuilt batch
 
     eng = Engine(0)
     b = eng.batch(d.struct_off, d.seg_be, d.struct_seg_off, d.seg_polar)
