@@ -235,6 +235,26 @@ SASA_B200_API int sasa_b200_batch_run_frames_host(sasa_b200_batch *batch, const 
                                     const sasa_b200_params *params, const sasa_b200_outputs *out,
                                     sasa_b200_stats *stats /* nullable */);
 
+/* Grouped runs of MD frames: buried surface area per frame along a trajectory, in the 12-byte frames form.  The batch, xyz
+ * and radii are exactly as in sasa_b200_batch_run_frames_host; group holds n_atoms_per_frame labels shared by every frame
+ * (only equality within a frame matters).  They cross the wire once per run and are expanded on the device, so a frame costs
+ * 12 B/atom on the wire as in the plain frames form.
+ *   out           bit for bit what sasa_b200_batch_run_frames_host gives for the same input; every field nullable.
+ *   out_isolated  bit for bit what sasa_b200_batch_run_groups_host gives for the same coordinates packed as float4 with the
+ *                 labels tiled over the frames; every field nullable.
+ * xyz, radii or group NULL with atoms in the batch, out_isolated NULL, or frames of unequal size: SASA_B200_ERR_INVALID_ARGUMENT;
+ * params->flags != 0: SASA_B200_ERR_UNSUPPORTED.  Non-finite input: SASA_B200_ERR_NON_FINITE with both output sets NaN-filled
+ * for that frame only.  Uses the per-chunk pipeline of the host entry points.  submit / sasa_b200_job_wait split the run like
+ * sasa_b200_batch_submit_host: the buffers belong to the run until the wait returns, and a batch carries one run at a time. */
+SASA_B200_API int sasa_b200_batch_run_groups_frames_host(sasa_b200_batch *batch, const float *xyz, const float *radii,
+                                           const uint32_t *group, const sasa_b200_params *params,
+                                           const sasa_b200_outputs *out, const sasa_b200_outputs *out_isolated,
+                                           sasa_b200_stats *stats /* nullable */);
+SASA_B200_API int sasa_b200_batch_submit_groups_frames_host(sasa_b200_batch *batch, const float *xyz, const float *radii,
+                                              const uint32_t *group, const sasa_b200_params *params,
+                                              const sasa_b200_outputs *out, const sasa_b200_outputs *out_isolated,
+                                              sasa_b200_job **out_job);
+
 /* Indexed-radius form: 13 bytes per atom on the wire instead of 16.  Proteins use a handful of distinct radii (ProtOr,
  * radii/protor.config, has ten), so the extraction step (build_atoms_and_mapping, src/options.rs:81-116) can emit
  * coordinates as 3 floats per atom plus ONE BYTE per atom indexing a palette of at most 256 radii.  With eight GPUs pulling

@@ -7,12 +7,12 @@ Engine / Batch wrapper (``engine``) and a mirror of the reference's public inter
 """
 from .api import (Atom, AtomLevel, ChainLevel, ChainResult, InterfaceResult, InterfaceSurfaceResult,  # noqa: F401
                   ProteinLevel, ProteinResult, ResidueLevel, ResidueResult, SASACalcError, SASAOptions, SurfaceResult,
-                  calculate_sasa_internal, default_engine, surface_points)
+                  TrajectoryInterfaceResult, calculate_sasa_internal, default_engine, surface_points, trajectory_interface)
 from .engine import Batch, BatchResult, Engine, SasaB200Error  # noqa: F401
 from .structure import read_structure  # noqa: F401
 
 __all__ = ["Atom", "AtomLevel", "ResidueLevel", "ChainLevel", "ProteinLevel", "ChainResult", "ResidueResult",
            "ProteinResult", "SASACalcError", "SASAOptions", "SurfaceResult", "InterfaceResult", "InterfaceSurfaceResult",
-           "calculate_sasa_internal", "default_engine",
-           "surface_points", "Engine",
+           "TrajectoryInterfaceResult", "calculate_sasa_internal", "default_engine",
+           "surface_points", "trajectory_interface", "Engine",
            "Batch", "BatchResult", "SasaB200Error", "read_structure"]

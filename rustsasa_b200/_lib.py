@@ -27,7 +27,7 @@ EXPORTS = [
     "sasa_b200_device_count", "sasa_b200_batch_run_indexed_host", "sasa_b200_batch_submit_indexed_host",
     "sasa_b200_batch_run_atom_range_peers_device", "sasa_b200_batch_run_groups_host", "sasa_b200_batch_run_groups_device",
     "sasa_b200_batch_run_masks_host", "sasa_b200_batch_run_masks_device", "sasa_b200_batch_run_groups_masks_host",
-    "sasa_b200_batch_run_groups_masks_device",
+    "sasa_b200_batch_run_groups_masks_device", "sasa_b200_batch_run_groups_frames_host", "sasa_b200_batch_submit_groups_frames_host",
 ]
 
 
@@ -90,6 +90,10 @@ def load() -> C.CDLL:
                                                         vp, vp, C.POINTER(Stats)]
     L.sasa_b200_batch_run_groups_masks_device.argtypes = [vp, vp, vp, vp, C.POINTER(Params), C.POINTER(Outputs), C.POINTER(Outputs),
                                                           vp, vp, vp]
+    L.sasa_b200_batch_run_groups_frames_host.argtypes = [vp, vp, vp, vp, C.POINTER(Params), C.POINTER(Outputs), C.POINTER(Outputs),
+                                                         C.POINTER(Stats)]
+    L.sasa_b200_batch_submit_groups_frames_host.argtypes = [vp, vp, vp, vp, C.POINTER(Params), C.POINTER(Outputs), C.POINTER(Outputs),
+                                                            C.POINTER(vp)]
     L.sasa_b200_batch_submit_host.argtypes = [vp, vp, vp, C.POINTER(Params), C.POINTER(Outputs), C.POINTER(vp)]
     L.sasa_b200_batch_submit_frames_host.argtypes = [vp, vp, vp, C.POINTER(Params), C.POINTER(Outputs), C.POINTER(vp)]
     L.sasa_b200_job_wait.argtypes = [vp, C.POINTER(Stats)]

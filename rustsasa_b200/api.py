@@ -97,6 +97,18 @@ class InterfaceSurfaceResult:
     atom_index: np.ndarray
 
 
+@dataclass
+class TrajectoryInterfaceResult:
+    """``trajectory_interface``: per frame the protein totals (global, polar, non-polar) in the complex and with every group
+    standing alone, (F, 3) float32 each, the buried area isolated - complex of the global totals (F,), and with residue ranges
+    given, the segment sums (F, G) of both."""
+    complex: np.ndarray
+    isolated: np.ndarray
+    buried: np.ndarray
+    complex_seg: Optional[np.ndarray] = None
+    isolated_seg: Optional[np.ndarray] = None
+
+
 class AtomLevel:
     name = "atom"
 
@@ -140,6 +152,93 @@ def surface_points(xyzr, exposed, n_points: int, probe_radius: float = 1.4):
     r = xyzr[atom, 3] + np.float32(probe_radius)
     points = xyzr[atom, :3] + r[:, None] * sphere[k]
     return points.astype(np.float32, copy=False), atom.astype(np.int64)
+
+
+# Page-locked staging of one block of trajectory_interface's frames (two blocks are staged at once).
+_TRAJECTORY_STAGING_BYTES = 256 << 20
+
+
+def trajectory_interface(xyz, radii, group, seg_be=None, seg_polar=None, probe_radius: float = 1.4, n_points: int = 100,
+                         frames_per_call: Optional[int] = None, engine: Optional[Engine] = None) -> TrajectoryInterfaceResult:
+    """Buried surface area along an MD trajectory.  ``xyz`` (F, N, 3) frames (any array, a numpy memmap included: blocks of
+    frames are copied into page-locked staging), ``radii`` (N,) and ``group`` (N,) labels shared by every frame; ``seg_be``
+    (G, 2) residue ranges within a frame and ``seg_polar`` (G,) their polar flags, both optional.
+
+    Frames go through ``Batch.submit_groups_frames_host`` in blocks of ``frames_per_call`` (default: the whole trajectory when
+    it fits 256 MB of staging, else as many frames as do).  Two batches alternate, so the next block is staged and submitted
+    before the current one is waited for: the host copy of block k + 1 and its transfer overlap the kernels of block k, and a
+    trajectory of any length runs with bounded memory.  The results equal one ``run_groups_frames_host`` over all frames bit
+    for bit."""
+    eng = engine or default_engine()
+    if not isinstance(xyz, np.ndarray):
+        xyz = np.asarray(xyz, np.float32)
+    if xyz.ndim != 3 or xyz.shape[2] != 3:
+        raise ValueError(f"xyz must be (F, N, 3), got {xyz.shape}")
+    F, N = int(xyz.shape[0]), int(xyz.shape[1])
+    radii = np.ascontiguousarray(radii, np.float32).reshape(-1)
+    group = np.ascontiguousarray(group, np.uint32).reshape(-1)
+    if radii.shape[0] != N or group.shape[0] != N:
+        raise ValueError(f"radii and group need one value per atom of a frame ({N}), got {radii.shape[0]} and {group.shape[0]}")
+    seg = None if seg_be is None else np.ascontiguousarray(seg_be, np.uint32).reshape(-1, 2)
+    pol = None if seg_polar is None or seg is None else np.ascontiguousarray(seg_polar, np.uint8).reshape(-1)
+    G = 0 if seg is None else seg.shape[0]
+    if frames_per_call is None:
+        frames_per_call = max(1, _TRAJECTORY_STAGING_BYTES // max(1, N * 12))
+    B = max(1, min(int(frames_per_call), F))
+    want = ("protein", "seg") if G else ("protein",)
+    out = TrajectoryInterfaceResult(np.zeros((F, 3), np.float32), np.zeros((F, 3), np.float32), np.zeros(F, np.float32),
+                                    np.zeros((F, G), np.float32) if G else None, np.zeros((F, G), np.float32) if G else None)
+    if F == 0:
+        return out
+
+    class _Slot:   # one batch of `fb` frames with its staging and page-locked outputs
+        def __init__(self, fb):
+            self.fb = fb
+            topo = (np.tile(seg, (fb, 1)), (np.arange(fb + 1) * G).astype(np.uint64),
+                    None if pol is None else np.tile(pol, fb)) if G else (None, None, None)
+            self.batch = Batch(eng, (np.arange(fb + 1) * N).astype(np.uint64), *topo)
+            self.stage = eng.pinned_empty((fb, N, 3), np.float32)
+            self.res = (self.batch._host_outputs(want, "pinned"), self.batch._host_outputs(want, "pinned"))
+
+    slots = {}
+
+    def slot_for(k, fb):
+        key = (k % 2, fb)
+        if key not in slots:
+            slots[key] = _Slot(fb)
+        return slots[key]
+
+    blocks = [(f0, min(f0 + B, F)) for f0 in range(0, F, B)]
+
+    def submit(k):
+        f0, f1 = blocks[k]
+        s = slot_for(k, f1 - f0)
+        np.copyto(s.stage, xyz[f0:f1], casting="same_kind")
+        return s, s.batch.submit_groups_frames_host(s.stage, radii, group, probe_radius, n_points, want=want, result=s.res)
+
+    pending = None
+    try:
+        pending = submit(0)
+        for k in range(len(blocks)):
+            s, job = pending
+            pending = submit(k + 1) if k + 1 < len(blocks) else None
+            cpx, iso = job.wait()
+            f0, f1 = blocks[k]
+            out.complex[f0:f1] = cpx.protein
+            out.isolated[f0:f1] = iso.protein
+            if G:
+                out.complex_seg[f0:f1] = cpx.seg_sasa.reshape(f1 - f0, G)
+                out.isolated_seg[f0:f1] = iso.seg_sasa.reshape(f1 - f0, G)
+    finally:
+        if pending is not None:   # an error left a block in flight: its buffers stay alive until it is done
+            try:
+                pending[1].wait()
+            except Exception:
+                pass
+        for s in slots.values():
+            s.batch.close()
+    out.buried[:] = out.isolated[:, 0] - out.complex[:, 0]
+    return out
 
 
 def _dense_classes(ids: np.ndarray) -> Optional[np.ndarray]:

@@ -1021,6 +1021,9 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
                 return fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "run_frames needs equal-sized structures");
     }
     if (indexed && (n_palette == 0 || n_palette > 256)) return fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "the radius palette holds 1..256 entries");
+    // grouped MD form: `group` holds the fN labels of one frame, shared by every frame; they cross the wire once and are
+    // expanded on the device chunk by chunk (expand_frame_labels_kernel)
+    const bool frame_labels = frames && grouped;
     const Points *pts = nullptr;
     if ((rc = get_points(ctx, params->n_points, &pts)) != 0) return rc;
     sasa_b200_job *job = job_acquire(ctx);
@@ -1042,6 +1045,7 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
     const size_t o_seg = o;    o += (out->seg_sasa && G) ? al(G * 4) : 0;
     const size_t o_prot = o;   o += out->protein ? al(S * 12) : 0;
     const size_t o_grp = o;    o += grouped ? al(N * 4) : 0;
+    const size_t o_lab = o;    o += frame_labels ? al(fN * 4) : 0;
     const size_t o_icnt = o;   o += (grouped && out_iso->counts) ? al(N * 4) : 0;
     const size_t o_iatom = o;  o += (grouped && out_iso->atom_sasa) ? al(N * 4) : 0;
     const size_t o_iseg = o;   o += (grouped && out_iso->seg_sasa && G) ? al(G * 4) : 0;
@@ -1131,7 +1135,8 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
     // structures on the large-structure path still expand to float4 first
     // (per plan: round 1 asked "any plan", so a 5,001-atom frame -- fused without id classes, large path with them -- lost both
     // the fused unpack and the three-stream overlap: cfg3 ran 18.4 ms end to end where the kernels take 12.9 ms)
-    const bool fused_frames = frames && b->max_large_v[variant] == 0;
+    // (grouped runs with n_points > 128 take the large-structure path for every structure, whatever the plan says)
+    const bool fused_frames = frames && b->max_large_v[variant] == 0 && !(grouped && params->n_points > 128);
     if (fused_frames) {
         kbase.xyz3 = reinterpret_cast<const float *>(base_p + o_xyz3);
         kbase.radii = reinterpret_cast<const float *>(base_p + o_rad);
@@ -1140,6 +1145,7 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
     J_TRY(cudaMemsetAsync(d_status, 0, 128, s0));   // status words + the ready counter of the gated pipeline (at +64 bytes)
     if (b->n_counters[variant]) J_TRY(cudaMemsetAsync(b->d_counters, 0, b->n_counters[variant] * sizeof(uint32_t), s0));
     if (frames && fN) J_TRY(cudaMemcpyAsync(base_p + o_rad, radii, fN * 4, cudaMemcpyHostToDevice, s0));
+    if (frame_labels && fN) J_TRY(cudaMemcpyAsync(base_p + o_lab, group, fN * 4, cudaMemcpyHostToDevice, s0));
     J_TRY(cudaEventRecord(job->ev0, s0));
     for (int i = 1; i < kStreams; ++i) J_TRY(cudaStreamWaitEvent(ctx->streams[i], job->ev0, 0));
     size_t ci = 0;
@@ -1198,7 +1204,14 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
                 J_TRY(cudaMemcpyAsync(base_p + o_xyzr + ch.a0 * 16, xyzr + ch.a0 * 4, na * 16, cudaMemcpyHostToDevice, st));
             }
             if (id_class) J_TRY(cudaMemcpyAsync(base_p + o_cls + ch.a0 * 4, id_class + ch.a0, na * 4, cudaMemcpyHostToDevice, st));
-            if (grouped) J_TRY(cudaMemcpyAsync(base_p + o_grp + ch.a0 * 4, group + ch.a0, na * 4, cudaMemcpyHostToDevice, st));
+            if (frame_labels) {
+                expand_frame_labels_kernel<<<(unsigned)((na + 255) / 256), 256, 0, st>>>(
+                    reinterpret_cast<const uint32_t *>(base_p + o_lab), reinterpret_cast<uint32_t *>(base_p + o_grp) + ch.a0, (uint32_t)na,
+                    (uint32_t)fN, (uint32_t)(ch.a0 % fN));
+                ++job->launches;
+            } else if (grouped) {
+                J_TRY(cudaMemcpyAsync(base_p + o_grp + ch.a0 * 4, group + ch.a0, na * 4, cudaMemcpyHostToDevice, st));
+            }
         }
         if ((rc = enqueue_chunk(b, variant, ch, kbase, st, &job->launches, nullptr, grouped ? &gp : nullptr, masked ? &mp : nullptr,
                                 (masked && grouped) ? &mpi : nullptr)) != 0)
@@ -1328,6 +1341,24 @@ int sasa_b200_batch_run_groups_host(sasa_b200_batch *b, const float *xyzr, const
     if (!out_isolated) return fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "out_isolated is NULL");
     sasa_b200_job *job = nullptr;
     int rc = submit_host_impl(b, xyzr, nullptr, nullptr, id_class, params, out, &job, nullptr, 0, group, out_isolated);
+    if (rc) return rc;
+    return wait_job_impl(job, stats);
+}
+
+int sasa_b200_batch_submit_groups_frames_host(sasa_b200_batch *b, const float *xyz, const float *radii, const uint32_t *group,
+                                              const sasa_b200_params *params, const sasa_b200_outputs *out,
+                                              const sasa_b200_outputs *out_isolated, sasa_b200_job **out_job) {
+    if (!b) return SASA_B200_ERR_INVALID_ARGUMENT;
+    if (!out_isolated) return fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "out_isolated is NULL");
+    if (b->n_atoms && (!xyz || !radii)) return fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "xyz / radii is NULL");
+    return submit_host_impl(b, nullptr, xyz, radii, nullptr, params, out, out_job, nullptr, 0, group, out_isolated);
+}
+
+int sasa_b200_batch_run_groups_frames_host(sasa_b200_batch *b, const float *xyz, const float *radii, const uint32_t *group,
+                                           const sasa_b200_params *params, const sasa_b200_outputs *out,
+                                           const sasa_b200_outputs *out_isolated, sasa_b200_stats *stats) {
+    sasa_b200_job *job = nullptr;
+    int rc = sasa_b200_batch_submit_groups_frames_host(b, xyz, radii, group, params, out, out_isolated, &job);
     if (rc) return rc;
     return wait_job_impl(job, stats);
 }

@@ -929,6 +929,14 @@ __global__ void __launch_bounds__(256) pack_frames_kernel(const float *__restric
     out[i] = make_float4(xyz[3 * (size_t)i], xyz[3 * (size_t)i + 1], xyz[3 * (size_t)i + 2], __ldg(radii + a));
 }
 
+// labels[atom] shared by every frame -> one label per atom of the chunk (grouped runs of MD frames); `phase` as above.
+__global__ void __launch_bounds__(256) expand_frame_labels_kernel(const uint32_t *__restrict__ labels, uint32_t *__restrict__ out,
+                                                                  uint32_t n, uint32_t per_frame, uint32_t phase) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    out[i] = __ldg(labels + (phase + i) % per_frame);
+}
+
 // xyz[atom][3] + one palette index per atom -> float4 {x, y, z, palette[index]}.
 __global__ void __launch_bounds__(256) pack_indexed_kernel(const float *__restrict__ xyz, const uint8_t *__restrict__ ridx,
                                                            const float *__restrict__ palette, float4 *__restrict__ out, uint32_t n) {

@@ -310,6 +310,45 @@ class Batch:
         cpx.stats = iso.stats = st.as_dict()
         return cpx, iso
 
+    def _groups_frames_args(self, xyz, radii, group):
+        xyz = _np(xyz, np.float32, (-1, 3))
+        radii = _np(radii, np.float32)
+        group = _np(group, np.uint32)
+        assert xyz.shape[0] == self.n_atoms, "xyz does not match struct_off"
+        assert group is None or radii is None or group.shape == radii.shape, "group and radii hold one value per atom of a frame"
+        return xyz, radii, group
+
+    def run_groups_frames_host(self, xyz, radii, group, probe_radius=1.4, n_points=100, simd_lanes=8, flags=0,
+                               want=("protein",), result=None):
+        """Grouped run in the MD form: xyz (F, N, 3) float32, radii (N,) and group (N,) labels shared by every frame.  Returns
+        (complex, isolated) BatchResults: complex is run_frames_host's result, isolated what run_groups_host gives with the
+        labels tiled over the frames.  Buried area per frame = isolated - complex.  `result`: a (complex, isolated) pair of
+        BatchResults to write into instead of new arrays."""
+        xyz, radii, group = self._groups_frames_args(xyz, radii, group)
+        cpx, iso = result if result is not None else (self._host_outputs(want, "numpy"), self._host_outputs(want, "numpy"))
+        outs = [_lib.Outputs(_ptr(r.counts), _ptr(r.atom_sasa), _ptr(r.seg_sasa), _ptr(r.protein)) for r in (cpx, iso)]
+        prm = self._params(probe_radius, n_points, simd_lanes, flags)
+        st = _lib.Stats()
+        self.engine._check(self._L.sasa_b200_batch_run_groups_frames_host(self._h, _ptr(xyz), _ptr(radii), _ptr(group), C.byref(prm),
+                                                                         C.byref(outs[0]), C.byref(outs[1]), C.byref(st)))
+        cpx.stats = iso.stats = st.as_dict()
+        return cpx, iso
+
+    def submit_groups_frames_host(self, xyz, radii, group, probe_radius=1.4, n_points=100, simd_lanes=8, flags=0,
+                                  want=("protein",), result=None) -> "Job":
+        """Asynchronous run_groups_frames_host: returns at once with a Job whose ``wait()`` returns (complex, isolated).  The
+        outputs are page-locked; xyz should be too (``Engine.pinned_empty``), and the inputs must stay alive until wait
+        returns."""
+        xyz, radii, group = self._groups_frames_args(xyz, radii, group)
+        res = result if result is not None else (self._host_outputs(want, "pinned"), self._host_outputs(want, "pinned"))
+        outs = [_lib.Outputs(_ptr(r.counts), _ptr(r.atom_sasa), _ptr(r.seg_sasa), _ptr(r.protein)) for r in res]
+        prm = self._params(probe_radius, n_points, simd_lanes, flags)
+        h = C.c_void_p()
+        self.engine._check(self._L.sasa_b200_batch_submit_groups_frames_host(self._h, _ptr(xyz), _ptr(radii), _ptr(group),
+                                                                            C.byref(prm), C.byref(outs[0]), C.byref(outs[1]),
+                                                                            C.byref(h)))
+        return Job(self, h, tuple(res), (xyz, radii, group))
+
     def _device_outputs(self, want, dev) -> BatchResult:
         import torch
         r = BatchResult()
@@ -420,17 +459,19 @@ class Batch:
 
 
 class Job:
-    """A host-buffer run in flight (sasa_b200_batch_submit_host .. sasa_b200_job_wait)."""
+    """A host-buffer run in flight (sasa_b200_batch_submit_host .. sasa_b200_job_wait).  `result` is a BatchResult, or the
+    (complex, isolated) pair of a grouped run."""
 
-    def __init__(self, batch: Batch, handle, result: BatchResult, keep):
+    def __init__(self, batch: Batch, handle, result, keep):
         self.batch, self._h, self.result, self._keep = batch, handle, result, keep
 
-    def wait(self) -> BatchResult:
+    def wait(self):
         if self._h is None:
             return self.result
         st = _lib.Stats()
         h, self._h = self._h, None
         self.batch.engine._check(self.batch._L.sasa_b200_job_wait(h, C.byref(st)))
-        self.result.stats = st.as_dict()
+        for r in (self.result if isinstance(self.result, tuple) else (self.result,)):
+            r.stats = st.as_dict()
         self._keep = None
         return self.result
