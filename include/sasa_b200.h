@@ -227,6 +227,43 @@ SASA_B200_API int sasa_b200_batch_run_groups_masks_device(sasa_b200_batch *batch
                                             const sasa_b200_outputs *d_out_isolated, uint32_t *d_exposed,
                                             uint32_t *d_exposed_isolated, void *stream);
 
+/* Pairwise buried area: which partner group buries how much of every atom, from one grouped pass.  For atom i of group g and
+ * another group h of the same structure, buried_h(i) = count_isolated(i) - count_{g+h}(i), where count_{g+h}(i) is i's count
+ * when only the atoms of g and h exist (in original order, same id_class rule): the points of i open with g alone that at least
+ * one atom of h hides.  The slot area is the reference's area expression on that count, ((4*pi*R^2) * buried_h(i)) * (1/n),
+ * bit for bit what atom_sasa would hold for that radius and count.  K = max_partners slots per atom, atoms in batch order (the
+ * indexing of counts): slot s of atom i is element i * K + s.  The slots in use hold the partners with buried_h(i) > 0 in
+ * ascending label order; the rest hold partner = UINT32_MAX, count 0 and area 0.0f.  A slot is in use exactly when its count
+ * is non-zero, so the label UINT32_MAX is not reserved.  Partners are enumerated among the atom's neighbours in the complex.
+ * So buried_h(i) <= count_isolated(i) - count(i), max_h buried_h(i) <= count_isolated(i) - count(i) <= sum_h buried_h(i)
+ * (a point hidden by two partners counts for both), and with exactly two groups in a structure the one slot in use holds
+ * count_isolated(i) - count(i). */
+typedef struct sasa_b200_pair_outputs {
+    uint32_t max_partners;     /* K: slots per atom, 1..16                                                           */
+    uint32_t *partner;         /* [n_atoms*K] partner group label per slot, UINT32_MAX = unused                      */
+    uint32_t *buried_counts;   /* [n_atoms*K] nullable: buried_h(i)                                                  */
+    float *buried_area;        /* [n_atoms*K] nullable: the area expression above on buried_counts                   */
+    uint32_t *partners_needed; /* nullable, ONE u32: the largest number of partners of an atom in this run           */
+} sasa_b200_pair_outputs;      /* (host pointers for _host, device pointers for _device)                             */
+
+/* out / out_isolated: bit for bit what sasa_b200_batch_run_groups_* gives for the same input; every field nullable.  An atom
+ * with more than K partners gets its K lowest-label partners, and the call returns SASA_B200_ERR_INVALID_ARGUMENT with a
+ * message naming the K the batch needs; *partners_needed receives that maximum on every run, successful or not, and out /
+ * out_isolated are still complete.  group == NULL, pairs or pairs->partner NULL with atoms in the batch, K outside 1..16 or a
+ * slot-buffer size that overflows size_t: SASA_B200_ERR_INVALID_ARGUMENT; params->flags != 0: SASA_B200_ERR_UNSUPPORTED.
+ * Non-finite input: SASA_B200_ERR_NON_FINITE with both output sets NaN-filled for that structure and its slots set to
+ * partner UINT32_MAX, count 0, area NaN.  An empty batch does nothing.  The host form uses the per-chunk pipeline; the device
+ * form behaves like sasa_b200_batch_run_groups_device: stream-ordered, with the too-few-slots error deferred to
+ * sasa_b200_batch_sync like SASA_B200_ERR_NON_FINITE (which takes precedence when both occur). */
+SASA_B200_API int sasa_b200_batch_run_group_pairs_host(sasa_b200_batch *batch, const float *xyzr, const uint32_t *id_class,
+                                         const uint32_t *group, const sasa_b200_params *params, const sasa_b200_outputs *out,
+                                         const sasa_b200_outputs *out_isolated, const sasa_b200_pair_outputs *pairs,
+                                         sasa_b200_stats *stats /* nullable */);
+SASA_B200_API int sasa_b200_batch_run_group_pairs_device(sasa_b200_batch *batch, const float *d_xyzr, const uint32_t *d_id_class,
+                                           const uint32_t *d_group, const sasa_b200_params *params, const sasa_b200_outputs *d_out,
+                                           const sasa_b200_outputs *d_out_isolated, const sasa_b200_pair_outputs *d_pairs,
+                                           void *stream);
+
 /* MD-trajectory form (what mdsasa-bolt feeds calculate_sasa_internal per frame): a batch
  * created with S = n_frames equal-sized structures; xyz holds n_frames * n_atoms_per_frame
  * * 3 floats, radii n_atoms_per_frame floats shared by every frame (12 B/atom/frame on the

@@ -5,14 +5,14 @@ the thin Python host layer used by the tests and the benchmark: a ctypes binding
 Engine / Batch wrapper (``engine``) and a mirror of the reference's public interface for the path
 (``api``: ``calculate_sasa_internal``, ``SASAOptions`` ...).  There is no CPU fallback.
 """
-from .api import (Atom, AtomLevel, ChainLevel, ChainResult, InterfaceResult, InterfaceSurfaceResult,  # noqa: F401
-                  ProteinLevel, ProteinResult, ResidueLevel, ResidueResult, SASACalcError, SASAOptions, SurfaceResult,
+from .api import (Atom, AtomLevel, ChainLevel, ChainResult, GroupPairResult, InterfacePairsResult,  # noqa: F401
+                  InterfaceResult, InterfaceSurfaceResult, ProteinLevel, ProteinResult, ResidueLevel, ResidueResult, SASACalcError, SASAOptions, SurfaceResult,
                   TrajectoryInterfaceResult, calculate_sasa_internal, default_engine, surface_points, trajectory_interface)
-from .engine import Batch, BatchResult, Engine, SasaB200Error  # noqa: F401
+from .engine import Batch, BatchResult, Engine, PairResult, SasaB200Error, group_pair_table  # noqa: F401
 from .structure import read_structure  # noqa: F401
 
 __all__ = ["Atom", "AtomLevel", "ResidueLevel", "ChainLevel", "ProteinLevel", "ChainResult", "ResidueResult",
            "ProteinResult", "SASACalcError", "SASAOptions", "SurfaceResult", "InterfaceResult", "InterfaceSurfaceResult",
-           "TrajectoryInterfaceResult", "calculate_sasa_internal", "default_engine",
+           "GroupPairResult", "InterfacePairsResult", "TrajectoryInterfaceResult", "calculate_sasa_internal", "default_engine",
            "surface_points", "trajectory_interface", "Engine",
-           "Batch", "BatchResult", "SasaB200Error", "read_structure"]
+           "Batch", "BatchResult", "PairResult", "SasaB200Error", "group_pair_table", "read_structure"]

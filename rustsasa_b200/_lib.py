@@ -28,6 +28,7 @@ EXPORTS = [
     "sasa_b200_batch_run_atom_range_peers_device", "sasa_b200_batch_run_groups_host", "sasa_b200_batch_run_groups_device",
     "sasa_b200_batch_run_masks_host", "sasa_b200_batch_run_masks_device", "sasa_b200_batch_run_groups_masks_host",
     "sasa_b200_batch_run_groups_masks_device", "sasa_b200_batch_run_groups_frames_host", "sasa_b200_batch_submit_groups_frames_host",
+    "sasa_b200_batch_run_group_pairs_host", "sasa_b200_batch_run_group_pairs_device",
 ]
 
 
@@ -39,6 +40,11 @@ class Params(C.Structure):
 class Outputs(C.Structure):
     _fields_ = [("counts", C.c_void_p), ("atom_sasa", C.c_void_p), ("seg_sasa", C.c_void_p),
                 ("protein", C.c_void_p)]
+
+
+class PairOutputs(C.Structure):
+    _fields_ = [("max_partners", C.c_uint32), ("partner", C.c_void_p), ("buried_counts", C.c_void_p),
+                ("buried_area", C.c_void_p), ("partners_needed", C.c_void_p)]
 
 
 class Stats(C.Structure):
@@ -94,6 +100,10 @@ def load() -> C.CDLL:
                                                          C.POINTER(Stats)]
     L.sasa_b200_batch_submit_groups_frames_host.argtypes = [vp, vp, vp, vp, C.POINTER(Params), C.POINTER(Outputs), C.POINTER(Outputs),
                                                             C.POINTER(vp)]
+    L.sasa_b200_batch_run_group_pairs_host.argtypes = [vp, vp, vp, vp, C.POINTER(Params), C.POINTER(Outputs), C.POINTER(Outputs),
+                                                       C.POINTER(PairOutputs), C.POINTER(Stats)]
+    L.sasa_b200_batch_run_group_pairs_device.argtypes = [vp, vp, vp, vp, C.POINTER(Params), C.POINTER(Outputs), C.POINTER(Outputs),
+                                                         C.POINTER(PairOutputs), vp]
     L.sasa_b200_batch_submit_host.argtypes = [vp, vp, vp, C.POINTER(Params), C.POINTER(Outputs), C.POINTER(vp)]
     L.sasa_b200_batch_submit_frames_host.argtypes = [vp, vp, vp, C.POINTER(Params), C.POINTER(Outputs), C.POINTER(vp)]
     L.sasa_b200_job_wait.argtypes = [vp, C.POINTER(Stats)]

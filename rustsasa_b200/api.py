@@ -15,6 +15,8 @@ The numeric core is the C ABI (include/sasa_b200.h); there is no CPU path here.
 from one grouped batch call.  ``process_surface`` and ``surface_points`` give the dot surface: the solvent-accessible test
 points themselves, from the exposed-point masks of the same batch call.  ``process_interface_surface`` gives both: the buried
 area and the interface patches, the test points that partner groups bury, from one grouped batch call with masks.
+``process_interface_pairs`` gives the pairwise interfaces: how much of every chain group each other group buries, from one
+grouped batch call with partner slots.
 """
 from __future__ import annotations
 
@@ -23,7 +25,7 @@ from typing import Any, List, Optional, Sequence
 
 import numpy as np
 
-from .engine import Batch, Engine
+from .engine import Batch, Engine, SasaB200Error, group_pair_table
 from .structure import (PackedStructure, SASACalcError, Structure, build_atoms_and_mapping,  # noqa: F401
                         load_radii_from_file, read_structure)
 
@@ -95,6 +97,29 @@ class InterfaceSurfaceResult:
     interface: InterfaceResult
     points: np.ndarray
     atom_index: np.ndarray
+
+
+@dataclass
+class GroupPairResult:
+    """One contacting pair of chain groups of ``SASAOptions.process_interface_pairs``: their group labels (a < b), the chain ids
+    of each, and the area of group a that group b buries and the area of group b that group a buries (float64 sums over the
+    per-atom areas in atom order)."""
+    group_a: int
+    group_b: int
+    chains_a: str
+    chains_b: str
+    buried_a: float
+    buried_b: float
+
+
+@dataclass
+class InterfacePairsResult:
+    """One structure of ``SASAOptions.process_interface_pairs``: the :class:`InterfaceResult` of ``process_interface``, the
+    contacting pairs of chain groups, and at residue level, per residue, ``{partner group: buried area}`` (float64 sums over the
+    residue's atoms in atom order; None at the other levels)."""
+    interface: InterfaceResult
+    pairs: List[GroupPairResult]
+    residue_partners: Optional[List[dict]] = None
 
 
 @dataclass
@@ -322,6 +347,16 @@ class SASAOptions:
         ``process_interface``."""
         return self._run_many(structures, engine, list(chain_groups) if chain_groups is not None else [], surface=True)
 
+    def process_interface_pairs(self, structures: Sequence[Structure], chain_groups: Optional[Sequence[str]] = None,
+                                max_partners: int = 4, engine: Optional[Engine] = None) -> List:
+        """Pairwise interfaces: per structure an :class:`InterfacePairsResult` with what ``process_interface`` gives for the
+        same arguments, one :class:`GroupPairResult` per contacting pair of chain groups, and at residue level the buried area
+        of every residue by each partner group -- all from ONE grouped batch call with ``max_partners`` partner slots per atom
+        (rerun once with as many slots as the batch needs when an atom has more partners; an atom with more than 16 partners
+        raises the run's :class:`SasaB200Error`).  Chain grouping and error reporting are those of ``process_interface``."""
+        return self._run_many(structures, engine, list(chain_groups) if chain_groups is not None else [],
+                              max_partners=int(max_partners))
+
     @staticmethod
     def _chain_groups(atom_chain: np.ndarray, chain_groups: List[str]) -> np.ndarray:
         """Dense per-atom group labels of one structure."""
@@ -336,8 +371,29 @@ class SASAOptions:
             out[i] = label[c]
         return out
 
+    @staticmethod
+    def _pairs_result(interface: InterfaceResult, p: PackedStructure, group: np.ndarray, partner: np.ndarray, area: np.ndarray,
+                      level: str) -> InterfacePairsResult:
+        chains = {}
+        for g, c in zip(group.tolist(), p.atom_chain):
+            if c not in chains.setdefault(g, ""):
+                chains[g] += c
+        table = group_pair_table(partner, area, group, [0, group.shape[0]])[0]
+        rows = [GroupPairResult(a, b, chains.get(a, ""), chains.get(b, ""), ab, ba) for a, b, ab, ba in table]
+        residue = None
+        if level == "residue":
+            residue = []
+            for b0, b1 in p.seg_be.tolist():
+                acc = {}
+                for i in range(b0, b1):
+                    for h, v in zip(partner[i].tolist(), area[i].tolist()):
+                        if h != 0xFFFFFFFF or v > 0:
+                            acc[h] = acc.get(h, 0.0) + v
+                residue.append(acc)
+        return InterfacePairsResult(interface, rows, residue)
+
     def _run_many(self, structures: Sequence[Structure], engine: Optional[Engine], chain_groups: Optional[List[str]],
-                  surface: bool = False) -> List:
+                  surface: bool = False, max_partners: Optional[int] = None) -> List:
         eng = engine or default_engine()
         packed: List[Optional[PackedStructure]] = []
         results: List = [None] * len(structures)
@@ -374,8 +430,19 @@ class SASAOptions:
                 res = run(xyzr, id_class, self.probe_radius, self.n_points, want=want)
             else:   # the protein totals give the buried area: always requested
                 group = np.concatenate([self._chain_groups(packed[i].atom_chain, chain_groups) for i in good])
-                run = batch.run_groups_masks_host if surface else batch.run_groups_host
-                cpx, iso = run(xyzr, group, id_class, self.probe_radius, self.n_points, want=tuple(set(want) | {"protein"}))
+                gwant = tuple(set(want) | {"protein"})
+                if max_partners is not None:
+                    try:
+                        cpx, iso, pairs = batch.run_group_pairs_host(xyzr, group, id_class, self.probe_radius, self.n_points,
+                                                                     want=gwant, max_partners=max_partners)
+                    except SasaB200Error as e:
+                        if not max_partners < getattr(e, "needed", 0) <= 16:   # (a run holds at most 16 slots per atom)
+                            raise
+                        cpx, iso, pairs = batch.run_group_pairs_host(xyzr, group, id_class, self.probe_radius, self.n_points,
+                                                                     want=gwant, max_partners=e.needed)
+                else:
+                    run = batch.run_groups_masks_host if surface else batch.run_groups_host
+                    cpx, iso = run(xyzr, group, id_class, self.probe_radius, self.n_points, want=gwant)
         finally:
             batch.close()
 
@@ -408,5 +475,7 @@ class SASAOptions:
                     buried = iso.exposed[a0:a1] & ~cpx.exposed[a0:a1]
                     pts, atom = surface_points(xyzr[a0:a1], buried, self.n_points, self.probe_radius)
                     r = InterfaceSurfaceResult(r, pts, atom)
+                if max_partners is not None:
+                    r = self._pairs_result(r, packed[i], group[a0:a1], pairs.partner[a0:a1], pairs.buried_area[a0:a1], level)
                 results[i] = r
         return results

@@ -47,7 +47,7 @@ struct Points {
 };
 
 // The fused kernels of one shared-memory configuration, by attribute slot (kernel_slot).
-constexpr int kKernelSlots = 12;
+constexpr int kKernelSlots = 14;
 struct Proto {
     int nt, minb;
     uint32_t cmax;
@@ -55,9 +55,10 @@ struct Proto {
     const void *fn[kKernelSlots];
 };
 // Slots: plain runs has_cls + 2 * tight, masked runs 4 + the same (tight: n_points <= 128, no statistics / forced streaming),
-// grouped runs 8 + has_cls and masked grouped runs 10 + has_cls (always tight: they take no flags, and with n_points > 128 they take
-// the large-structure path).
-int kernel_slot(bool grouped, bool masked, bool has_cls, bool tight) {
+// grouped runs 8 + has_cls, masked grouped runs 10 + has_cls and pairwise buried area 12 + has_cls (always tight: they take no
+// flags, and with n_points > 128 they take the large-structure path).
+int kernel_slot(bool grouped, bool masked, bool has_cls, bool tight, bool pairs = false) {
+    if (pairs) return 12 + (has_cls ? 1 : 0);
     return grouped ? (masked ? 10 : 8) + (has_cls ? 1 : 0) : (masked ? 4 : 0) + (has_cls ? 1 : 0) + (tight ? 2 : 0);
 }
 #define SASA_PROTO(NT, MINB, CMAX)                                                                                     \
@@ -72,7 +73,9 @@ int kernel_slot(bool grouped, bool masked, bool has_cls, bool tight) {
               (const void *)sasa_tight_groups_kernel<NT, MINB, false, CMAX>,                                           \
               (const void *)sasa_tight_groups_kernel<NT, MINB, true, CMAX>,                                            \
               (const void *)sasa_tight_groups_masks_kernel<NT, MINB, false, CMAX>,                                     \
-              (const void *)sasa_tight_groups_masks_kernel<NT, MINB, true, CMAX> } }
+              (const void *)sasa_tight_groups_masks_kernel<NT, MINB, true, CMAX>,                                      \
+              (const void *)sasa_tight_group_pairs_kernel<NT, MINB, false, CMAX>,                                      \
+              (const void *)sasa_tight_group_pairs_kernel<NT, MINB, true, CMAX> } }
 // Shared-memory configurations of the fused kernel.  nmax is derived from the per-CTA budget that lets `minb` CTAs share one SM
 // (228 KB per SM, 1 KB reserved per CTA, 227 KB per CTA max); both keep 32 warps resident per SM (64 registers/thread).
 const Proto kProtos[] = {SASA_PROTO(512, 2, 8192), SASA_PROTO(1024, 1, 16384)};
@@ -119,6 +122,8 @@ struct sasa_b200_job {
     std::chrono::steady_clock::time_point t_begin;
     uint32_t launches = 0;
     bool active = false;
+    const sasa_b200_pair_outputs *pairs = nullptr;   // pairwise buried-area runs: the caller's slot outputs (partners_needed is
+                                                     // written when the job is waited for)
 };
 
 struct sasa_b200_job;
@@ -135,6 +140,7 @@ struct sasa_b200_ctx {
     std::map<uint32_t, Points> points;
     int *d_err = nullptr;
     unsigned long long *d_stat = nullptr;
+    uint32_t *d_needed = nullptr;   // pairwise buried area, device form: partners needed by the last run [0] and since the last sync [1]
     std::vector<SmallCfg> cfgs;
     std::string err;
     std::mutex mu;
@@ -507,10 +513,10 @@ int check_params(sasa_b200_ctx *ctx, const sasa_b200_params *p) {
 // joined back into `st` (so the caller still sees one stream-ordered unit of work).  Large-structure pipelines stay
 // on `st`.
 // gp: grouped runs (group labels and isolated outputs), else null.  mp: exposed-point masks, else null.  mpi: the isolated
-// masks of a masked grouped run (gp and mp set), else null.
+// masks of a masked grouped run (gp and mp set), else null.  pp: the partner slots of a pairwise buried-area run (gp set), else null.
 int enqueue_chunk(sasa_b200_batch *b, int variant, const Chunk &ch, const KParams &base, cudaStream_t st,
                   uint32_t *launches, const uint32_t *order_override = nullptr, const GroupParams *gp = nullptr,
-                  const MaskParams *mp = nullptr, const MaskParams *mpi = nullptr) {
+                  const MaskParams *mp = nullptr, const MaskParams *mpi = nullptr, const PairParams *pp = nullptr) {
     sasa_b200_ctx *ctx = b->ctx;
     int n_small = 0;
     for (const Launch &L : ch.launches) n_small += L.cfg >= 0;
@@ -529,7 +535,7 @@ int enqueue_chunk(sasa_b200_batch *b, int variant, const Chunk &ch, const KParam
         if (L.cfg < 0 || all_large) {
             if (ctx->large_used) CU_TRY(ctx, cudaStreamWaitEvent(st, ctx->ev_large, 0));
             int rc = large_enqueue(ctx->sm_count, ctx->large, kp, &b->h_order[variant][L.order_off], L.n_work,
-                                   b->h_off.data(), b->h_seg_off.empty() ? nullptr : b->h_seg_off.data(), st, launches, 0, 1, gp, mp, mpi);
+                                   b->h_off.data(), b->h_seg_off.empty() ? nullptr : b->h_seg_off.data(), st, launches, 0, 1, gp, mp, mpi, pp);
             if (rc != 0) return fail(ctx, rc, "large-structure path failed: %s", cudaGetErrorString(cudaGetLastError()));
             CU_TRY(ctx, cudaEventRecord(ctx->ev_large, st));
             ctx->large_used = true;
@@ -547,9 +553,9 @@ int enqueue_chunk(sasa_b200_batch *b, int variant, const Chunk &ch, const KParam
             CU_TRY(ctx, cudaStreamWaitEvent(ls, ctx->ev_fork, 0));
         }
         // (kernel arguments past the kernel's own are not read)
-        void *args[] = {(void *)&kp, gp ? (void *)gp : (void *)mp, (void *)mp, (void *)mpi};
+        void *args[] = {(void *)&kp, gp ? (void *)gp : (void *)mp, pp ? (void *)pp : (void *)mp, (void *)mpi};
         const bool tight = kp.n_points <= 128 && (kp.flags & 3u) == 0;
-        const int slot = kernel_slot(grouped, mp != nullptr, has_cls, tight);
+        const int slot = kernel_slot(grouped, mp != nullptr, has_cls, tight, pp != nullptr);
         const void *fn = kProtos[c.proto].fn[slot];
         if (!ctx->attr_done[c.proto][slot]) {
             cudaError_t ea = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -585,6 +591,11 @@ int finish_run(sasa_b200_batch *b, sasa_b200_stats *stats) {
     if (stats) *stats = b->last;
     if (h_err == SASA_B200_ERR_NON_FINITE)
         return fail(ctx, SASA_B200_ERR_NON_FINITE, "non-finite coordinate or radius in the input (the reference panics here)");
+    if (h_err == SASA_B200_ERR_INVALID_ARGUMENT) {   // only raised by the pairs kernels: an atom with more partners than slots
+        uint32_t need = 0;
+        CU_TRY(ctx, cudaMemcpy(&need, ctx->d_needed + 1, sizeof need, cudaMemcpyDeviceToHost));
+        return fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "too few partner slots: the batch needs max_partners = %u", need);
+    }
     if (h_err) return fail(ctx, h_err, "device-side error %d", h_err);
     return SASA_B200_OK;
 }
@@ -658,6 +669,8 @@ int sasa_b200_create(int device, sasa_b200_ctx **out_ctx) {
     }
     if ((e = cudaMalloc(&ctx->d_err, sizeof(int))) != cudaSuccess) return bail(SASA_B200_ERR_OUT_OF_MEMORY, "cudaMalloc", e);
     if ((e = cudaMalloc(&ctx->d_stat, 3 * sizeof(unsigned long long))) != cudaSuccess) return bail(SASA_B200_ERR_OUT_OF_MEMORY, "cudaMalloc", e);
+    if ((e = cudaMalloc(&ctx->d_needed, 2 * sizeof(uint32_t))) != cudaSuccess) return bail(SASA_B200_ERR_OUT_OF_MEMORY, "cudaMalloc", e);
+    cudaMemset(ctx->d_needed, 0, 2 * sizeof(uint32_t));
     cudaMemset(ctx->d_err, 0, sizeof(int));
     cudaMemset(ctx->d_stat, 0, 3 * sizeof(unsigned long long));
     int rc = build_cfgs(ctx);
@@ -704,6 +717,7 @@ void sasa_b200_destroy(sasa_b200_ctx *ctx) {
     large_release(ctx->large);
     cudaFree(ctx->d_err);
     cudaFree(ctx->d_stat);
+    cudaFree(ctx->d_needed);
     cudaFree(ctx->arena);
     delete ctx;
 }
@@ -874,10 +888,25 @@ static int check_masks(sasa_b200_batch *b, const uint32_t *exposed, const sasa_b
     return SASA_B200_OK;
 }
 
+// Checks of the pairwise buried-area entry points: slot outputs for every atom, 1..16 slots per atom, a slot buffer whose size
+// fits a size_t.
+static int check_pairs(sasa_b200_batch *b, const sasa_b200_pair_outputs *pairs) {
+    if (!pairs) return b->n_atoms ? fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "pairs is NULL") : SASA_B200_OK;
+    if (pairs->max_partners < 1 || pairs->max_partners > 16)
+        return fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "max_partners must be 1..16, got %u", pairs->max_partners);
+    if (!pairs->partner && b->n_atoms) return fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "pairs->partner is NULL");
+    if (b->n_atoms && pairs->max_partners > SIZE_MAX / 4 / b->n_atoms)
+        return fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "the slot buffers (%zu atoms x %u slots) overflow size_t", b->n_atoms,
+                    pairs->max_partners);
+    return SASA_B200_OK;
+}
+
 // d_iso: grouped runs; masked: d_exposed receives the exposed-point masks, and with d_iso d_exposed_iso the isolated ones.
+// pairs (with d_iso): pairwise buried area, d_pairs receives the partner slots.
 static int run_device_impl(sasa_b200_batch *b, const float *d_xyzr, const uint32_t *d_id_class, const uint32_t *d_group,
                            const sasa_b200_params *params, const sasa_b200_outputs *d_out, const sasa_b200_outputs *d_iso, void *stream,
-                           bool masked = false, uint32_t *d_exposed = nullptr, uint32_t *d_exposed_iso = nullptr) {
+                           bool masked = false, uint32_t *d_exposed = nullptr, uint32_t *d_exposed_iso = nullptr, bool pairs = false,
+                           const sasa_b200_pair_outputs *d_pairs = nullptr) {
     if (!b) return SASA_B200_ERR_INVALID_ARGUMENT;
     sasa_b200_ctx *ctx = b->ctx;
     std::lock_guard<std::mutex> lk(ctx->mu);
@@ -891,7 +920,14 @@ static int run_device_impl(sasa_b200_batch *b, const float *d_xyzr, const uint32
     const int variant = (d_id_class ? 1 : 0) + 2 + (grouped ? 4 : 0);
     CU_TRY(ctx, cudaSetDevice(ctx->device));
     if (grouped && (rc = prepare_groups(b, d_group, params, d_iso, variant)) != 0) return rc;
+    if (pairs && (rc = check_pairs(b, d_pairs)) != 0) return rc;
+    if (pairs && !d_pairs) pairs = false;   // (an empty batch: no slots to write)
     cudaStream_t st = stream ? (cudaStream_t)stream : ctx->streams[0];
+    PairParams pp{};
+    if (pairs) {
+        pp = PairParams{d_pairs->partner, d_pairs->buried_counts, d_pairs->buried_area, ctx->d_needed, d_pairs->max_partners};
+        CU_TRY(ctx, cudaMemsetAsync(ctx->d_needed, 0, sizeof(uint32_t), st));
+    }
     RunArgs ra;
     ra.d_xyzr = reinterpret_cast<const float4 *>(d_xyzr);
     ra.d_cls = d_id_class;
@@ -907,8 +943,10 @@ static int run_device_impl(sasa_b200_batch *b, const float *d_xyzr, const uint32
         CU_TRY(ctx, cudaMemsetAsync(b->d_counters, 0, b->n_counters[variant] * sizeof(uint32_t), st));
     for (const Chunk &ch : b->plan[variant])
         if ((rc = enqueue_chunk(b, variant, ch, base, st, &b->launches_last, nullptr, grouped ? &gp : nullptr, masked ? &mp : nullptr,
-                                masked && grouped ? &mpi : nullptr)) != 0)
+                                masked && grouped ? &mpi : nullptr, pairs ? &pp : nullptr)) != 0)
             return rc;
+    if (pairs && d_pairs->partners_needed)
+        CU_TRY(ctx, cudaMemcpyAsync(d_pairs->partners_needed, ctx->d_needed, sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
     return SASA_B200_OK;
 }
 
@@ -937,6 +975,13 @@ int sasa_b200_batch_run_groups_masks_device(sasa_b200_batch *b, const float *d_x
     return run_device_impl(b, d_xyzr, d_id_class, d_group, params, d_out, d_out_isolated, stream, true, d_exposed, d_exposed_isolated);
 }
 
+int sasa_b200_batch_run_group_pairs_device(sasa_b200_batch *b, const float *d_xyzr, const uint32_t *d_id_class, const uint32_t *d_group,
+                                           const sasa_b200_params *params, const sasa_b200_outputs *d_out,
+                                           const sasa_b200_outputs *d_out_isolated, const sasa_b200_pair_outputs *d_pairs, void *stream) {
+    if (b && !d_out_isolated) return fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "d_out_isolated is NULL");
+    return run_device_impl(b, d_xyzr, d_id_class, d_group, params, d_out, d_out_isolated, stream, false, nullptr, nullptr, true, d_pairs);
+}
+
 int sasa_b200_batch_sync(sasa_b200_batch *b, sasa_b200_stats *stats) {
     if (!b) return SASA_B200_ERR_INVALID_ARGUMENT;
     sasa_b200_ctx *ctx = b->ctx;
@@ -946,6 +991,7 @@ int sasa_b200_batch_sync(sasa_b200_batch *b, sasa_b200_stats *stats) {
     int rc = finish_run(b, stats);
     cudaMemset(ctx->d_err, 0, sizeof(int));
     cudaMemset(ctx->d_stat, 0, 3 * sizeof(unsigned long long));
+    cudaMemset(ctx->d_needed, 0, 2 * sizeof(uint32_t));
     return rc;
 }
 
@@ -962,7 +1008,7 @@ static sasa_b200_job *job_acquire(sasa_b200_ctx *ctx) {
     } else {
         j = new sasa_b200_job();
         if (cudaEventCreate(&j->ev0) != cudaSuccess || cudaEventCreate(&j->ev1) != cudaSuccess ||
-            cudaHostAlloc((void **)&j->h_status, 4 * sizeof(unsigned long long), cudaHostAllocDefault) != cudaSuccess ||
+            cudaHostAlloc((void **)&j->h_status, 5 * sizeof(unsigned long long), cudaHostAllocDefault) != cudaSuccess ||
             cudaHostAlloc((void **)&j->h_ready, kMaxGatedChunks * sizeof(uint32_t), cudaHostAllocDefault) != cudaSuccess) {
             if (j->ev0) cudaEventDestroy(j->ev0);
             if (j->ev1) cudaEventDestroy(j->ev1);
@@ -992,7 +1038,8 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
                             const uint32_t *id_class, const sasa_b200_params *params, const sasa_b200_outputs *out,
                             sasa_b200_job **out_job, const uint8_t *ridx = nullptr, size_t n_palette = 0,
                             const uint32_t *group = nullptr, const sasa_b200_outputs *out_iso = nullptr, bool masked = false,
-                            uint32_t *exposed = nullptr, uint32_t *exposed_iso = nullptr) {
+                            uint32_t *exposed = nullptr, uint32_t *exposed_iso = nullptr, bool pairs = false,
+                            const sasa_b200_pair_outputs *pair_out = nullptr) {
     sasa_b200_ctx *ctx = b->ctx;
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (!out || !out_job) return fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "out / out_job is NULL");
@@ -1009,6 +1056,9 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
     const size_t W = mask_words(params->n_points);
     const int variant = (id_class ? 1 : 0) + (grouped ? 4 : 0);
     if (grouped && (rc = prepare_groups(b, group, params, out_iso, variant)) != 0) return rc;
+    if (pairs && (rc = check_pairs(b, pair_out)) != 0) return rc;
+    if (pairs && !pair_out) pairs = false;   // (an empty batch: no slots to write)
+    const size_t K = pairs ? pair_out->max_partners : 0;
     const bool indexed = xyz3 != nullptr && ridx != nullptr;   // 13 B/atom: coordinates + a palette index per atom
     const bool frames = xyz3 != nullptr;                       // any 12-byte coordinate form
     size_t fN = 0;  // atoms per frame (MD form) / palette entries (indexed form)
@@ -1031,6 +1081,7 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
     job->batch = b;
     job->t_begin = std::chrono::steady_clock::now();
     job->launches = 0;
+    job->pairs = pairs ? pair_out : nullptr;
     // carve the arena
     auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
     size_t o = 0;
@@ -1052,6 +1103,9 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
     const size_t o_iprot = o;  o += (grouped && out_iso->protein) ? al(S * 12) : 0;
     const size_t o_mask = o;   o += masked ? al(N * W * 4) : 0;
     const size_t o_imask = o;  o += (masked && grouped) ? al(N * W * 4) : 0;
+    const size_t o_ppart = o;  o += pairs ? al(N * K * 4) : 0;
+    const size_t o_pcnt = o;   o += (pairs && pair_out->buried_counts) ? al(N * K * 4) : 0;
+    const size_t o_parea = o;  o += (pairs && pair_out->buried_area) ? al(N * K * 4) : 0;
     cudaStream_t s0 = ctx->streams[0];
     // the previous job may still be running on the sibling streams: this job's first stream starts behind all of them
     if (ctx->tail_valid)
@@ -1131,6 +1185,13 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
     unsigned long long *d_status = reinterpret_cast<unsigned long long *>(base_p + o_status);
     kbase.err_flag = reinterpret_cast<int *>(d_status);
     kbase.stat = d_status + 1;
+    // pairwise buried area: the partners-needed words sit behind the statistics (status word 4) and come back with them
+    PairParams pp{};
+    if (pairs)
+        pp = PairParams{reinterpret_cast<uint32_t *>(base_p + o_ppart),
+                        pair_out->buried_counts ? reinterpret_cast<uint32_t *>(base_p + o_pcnt) : nullptr,
+                        pair_out->buried_area ? reinterpret_cast<float *>(base_p + o_parea) : nullptr,
+                        reinterpret_cast<uint32_t *>(d_status + 4), (uint32_t)K};
     // MD form: the fused kernels read the 12-byte coordinates and the shared radius table directly; only batches with
     // structures on the large-structure path still expand to float4 first
     // (per plan: round 1 asked "any plan", so a 5,001-atom frame -- fused without id classes, large path with them -- lost both
@@ -1214,7 +1275,7 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
             }
         }
         if ((rc = enqueue_chunk(b, variant, ch, kbase, st, &job->launches, nullptr, grouped ? &gp : nullptr, masked ? &mp : nullptr,
-                                (masked && grouped) ? &mpi : nullptr)) != 0)
+                                (masked && grouped) ? &mpi : nullptr, pairs ? &pp : nullptr)) != 0)
             return job_abort(ctx, job, rc);
         if (na && out->counts)
             J_TRY(cudaMemcpyAsync(out->counts + ch.a0, base_p + o_cnt + ch.a0 * 4, na * 4, cudaMemcpyDeviceToHost, st));
@@ -1240,6 +1301,15 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
             if (na && masked)
                 J_TRY(cudaMemcpyAsync(exposed_iso + ch.a0 * W, base_p + o_imask + ch.a0 * W * 4, na * W * 4, cudaMemcpyDeviceToHost, st));
         }
+        if (na && pairs) {
+            J_TRY(cudaMemcpyAsync(pair_out->partner + ch.a0 * K, base_p + o_ppart + ch.a0 * K * 4, na * K * 4, cudaMemcpyDeviceToHost, st));
+            if (pair_out->buried_counts)
+                J_TRY(cudaMemcpyAsync(pair_out->buried_counts + ch.a0 * K, base_p + o_pcnt + ch.a0 * K * 4, na * K * 4, cudaMemcpyDeviceToHost,
+                                      st));
+            if (pair_out->buried_area)
+                J_TRY(cudaMemcpyAsync(pair_out->buried_area + ch.a0 * K, base_p + o_parea + ch.a0 * K * 4, na * K * 4, cudaMemcpyDeviceToHost,
+                                      st));
+        }
     }
     // join the sibling streams into the first one, read the status words back, free the arena in stream order
     for (int i = 1; i < kStreams; ++i) {
@@ -1247,7 +1317,7 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
         J_TRY(cudaStreamWaitEvent(s0, ctx->ev_tail[i], 0));
     }
     ctx->tail_valid = true;
-    J_TRY(cudaMemcpyAsync(job->h_status, d_status, 32, cudaMemcpyDeviceToHost, s0));
+    J_TRY(cudaMemcpyAsync(job->h_status, d_status, pairs ? 40 : 32, cudaMemcpyDeviceToHost, s0));
     J_TRY(cudaEventRecord(job->ev1, s0));
     J_TRY(cudaFreeAsync(job->d_arena, s0));
     job->d_arena = nullptr;
@@ -1279,8 +1349,13 @@ static int wait_job_impl(sasa_b200_job *job, sasa_b200_stats *stats) {
         b->launches_last = job->launches;
         if (stats) *stats = b->last;
         const int h_err = (int)(job->h_status[0] & 0xffffffffull);
+        const uint32_t need = (uint32_t)(job->h_status[4] & 0xffffffffull);   // pairwise buried area: partners needed
+        if (job->pairs && job->pairs->partners_needed) *job->pairs->partners_needed = need;
         if (h_err == SASA_B200_ERR_NON_FINITE)
             rc = fail(ctx, SASA_B200_ERR_NON_FINITE, "non-finite coordinate or radius in the input (the reference panics here)");
+        else if (job->pairs && h_err == SASA_B200_ERR_INVALID_ARGUMENT)
+            rc = fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "too few partner slots: max_partners = %u, the batch needs max_partners = %u",
+                      job->pairs->max_partners, need);
         else if (h_err)
             rc = fail(ctx, h_err, "device-side error %d", h_err);
     }
@@ -1381,6 +1456,18 @@ int sasa_b200_batch_run_groups_masks_host(sasa_b200_batch *b, const float *xyzr,
     sasa_b200_job *job = nullptr;
     int rc = submit_host_impl(b, xyzr, nullptr, nullptr, id_class, params, out, &job, nullptr, 0, group, out_isolated, true, exposed,
                               exposed_isolated);
+    if (rc) return rc;
+    return wait_job_impl(job, stats);
+}
+
+int sasa_b200_batch_run_group_pairs_host(sasa_b200_batch *b, const float *xyzr, const uint32_t *id_class, const uint32_t *group,
+                                         const sasa_b200_params *params, const sasa_b200_outputs *out,
+                                         const sasa_b200_outputs *out_isolated, const sasa_b200_pair_outputs *pairs, sasa_b200_stats *stats) {
+    if (!b) return SASA_B200_ERR_INVALID_ARGUMENT;
+    if (!out_isolated) return fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "out_isolated is NULL");
+    sasa_b200_job *job = nullptr;
+    int rc = submit_host_impl(b, xyzr, nullptr, nullptr, id_class, params, out, &job, nullptr, 0, group, out_isolated, false, nullptr,
+                              nullptr, true, pairs);
     if (rc) return rc;
     return wait_job_impl(job, stats);
 }

@@ -110,6 +110,29 @@ struct GroupAtoms {
     }
 };
 
+// Pairwise buried area (sasa_b200_batch_run_group_pairs_*), a kernel argument of its own next to GroupParams: k slots per atom in
+// batch order (slot s of atom i at i * k + s) holding the partner groups that bury a point of the atom, in ascending label order.
+// needed: two words, the largest number of partners of an atom in this run [0] and since the last sasa_b200_batch_sync [1].
+struct PairParams {
+    uint32_t *partner;
+    uint32_t *counts;   // nullable
+    float *area;        // nullable
+    uint32_t *needed;
+    uint32_t k;
+};
+
+// The evaluation of atom i (group gi) with only the atoms of gi and gh present: every other atom reads as the far-away sentinel.
+template <bool GLOBAL>
+struct PairAtoms {
+    const float4 *a;
+    const uint32_t *grp;
+    uint32_t gi, gh;
+    __device__ __forceinline__ float4 operator()(int j) const {
+        const uint32_t gj = GLOBAL ? __ldg(grp + j) : grp[j];
+        return (gj == gi || gj == gh) ? (GLOBAL ? __ldg(a + j) : a[j]) : make_float4(1.0e18f, 1.0e18f, 1.0e18f, 0.0f);
+    }
+};
+
 // Exposed-point masks (sasa_b200_batch_run_masks_*), a kernel argument of its own next to KParams: mask_words(n_points) u32 per
 // atom in batch order, bit b of word w set when point 32 w + b is exposed.  Every routine writes an atom's whole row with the
 // lanes w < W of its warp (one coalesced store), so no row is left unwritten and the buffer needs no zero-fill.
@@ -608,6 +631,91 @@ __device__ __forceinline__ float atom_fast(const KParams &p, const float4 *ent, 
         }
     }
     return (float)exposed;
+}
+
+// ---------------------------------------------------------------------------------------
+// Pairwise buried area: the slot row of one atom.  Partners are enumerated warp-uniformly in ascending label order; one with a
+// non-zero buried count takes the next slot, held by lane n (so lane s < k ends up holding slot s).  n counts every partner with a
+// non-zero count, also past the k slots.
+// ---------------------------------------------------------------------------------------
+struct PairSlot {
+    uint32_t label, count;   // this lane's slot
+    int n;                   // partners with a non-zero count (warp-uniform)
+};
+
+__device__ __forceinline__ PairSlot pair_empty() { return PairSlot{0xffffffffu, 0u, 0}; }
+
+__device__ __forceinline__ void pair_take(PairSlot &ps, uint32_t h, int buried) {
+    if (buried <= 0) return;
+    if (lane_id() == ps.n) {
+        ps.label = h;
+        ps.count = (uint32_t)buried;
+    }
+    ++ps.n;
+}
+
+// The atom's row (one coalesced store per array from lanes s < k), and the number of partners into both `needed` words.  More
+// partners than slots raise SASA_B200_ERR_INVALID_ARGUMENT (1) in the error flag unless an error is already there, so a
+// non-finite structure (4, written by exchange) always wins.
+__device__ __forceinline__ void pair_store(const PairParams &pp, size_t atom, const PairSlot &ps, float radius, float probe, float inv_n,
+                                           int *err_flag) {
+    const int lane = lane_id();
+    if (lane < (int)pp.k) {
+        const bool used = lane < ps.n;
+        const size_t o = atom * pp.k + (size_t)lane;
+        pp.partner[o] = used ? ps.label : 0xffffffffu;
+        if (pp.counts) pp.counts[o] = used ? ps.count : 0u;
+        if (pp.area) pp.area[o] = used ? atom_area(radius, probe, (float)ps.count, inv_n) : 0.0f;
+    }
+    if (lane == 0 && ps.n > 0) {
+        atomicMax(pp.needed, (unsigned)ps.n);
+        atomicMax(pp.needed + 1, (unsigned)ps.n);
+        if (ps.n > (int)pp.k) atomicCAS(err_flag, 0, 1);
+    }
+}
+
+// The slot rows of atoms [a0, a0 + N) of a structure with non-finite input: no partner, count 0, area NaN.
+__device__ __forceinline__ void pair_blank_rows(const PairParams &pp, size_t a0, size_t N, size_t tid, size_t nth) {
+    const float qn = __int_as_float(0x7fc00000);
+    for (size_t i = tid; i < N * pp.k; i += nth) {
+        pp.partner[a0 * pp.k + i] = 0xffffffffu;
+        if (pp.counts) pp.counts[a0 * pp.k + i] = 0u;
+        if (pp.area) pp.area[a0 * pp.k + i] = qn;
+    }
+}
+
+// Partner enumeration of an atom without a candidate list (the cold paths): the smallest label above `prev` (any label when
+// `first`) other than gi among the atoms within reach of atom `pos` in the cell rows around it -- the rows the streaming routine
+// scans.  Returns false when there is none.  A superset of the partners is harmless: one that buries nothing is dropped.
+template <typename AtomAcc, typename CellT>
+__device__ __forceinline__ bool pair_next_scan(const Grid &g, const CellT *cell, const AtomAcc &atoms, const uint32_t *grp, int pos,
+                                               const float4 ai, float reach_i, uint32_t gi, bool first, uint32_t prev, uint32_t &next) {
+    const int lane = lane_id();
+    const int cx = cell_coord(ai.x, g.minx, g.inv_c, g.nx), cy = cell_coord(ai.y, g.miny, g.inv_c, g.ny),
+              cz = cell_coord(ai.z, g.minz, g.inv_c, g.nz);
+    const Rows rows = rows_of(g, cell, cx, cy, cz);
+    bool any = false;
+    uint32_t lo = 0xffffffffu;
+    for (int t0 = 0; t0 < rows.total; t0 += 32) {
+        const int idx = t0 + lane;
+        const int j = row_lookup(rows, idx);
+        if (idx < rows.total && j != pos) {
+            const uint32_t gj = grp[j];
+            if (gj != gi && (first || gj > prev)) {
+                const float4 aj = atoms(j);
+                const float dx = ai.x - aj.x, dy = ai.y - aj.y, dz = ai.z - aj.z;
+                const float d2 = fmaf(dx, dx, fmaf(dy, dy, dz * dz));
+                const float cut = reach_i + aj.w;
+                if (d2 <= cut * cut) {
+                    any = true;
+                    lo = min(lo, gj);
+                }
+            }
+        }
+    }
+    if (!__any_sync(kFull, any)) return false;
+    next = __reduce_min_sync(kFull, lo);
+    return true;
 }
 
 }  // namespace sasa

@@ -668,12 +668,17 @@ __device__ __forceinline__ float large_eval_atom(const KParams &p, const Grid &g
 // HAS_MASK: every atom also writes its mask row in the complex (mp) and with its group standing alone (mpi).  The cap path
 // writes both from cap_atom_groups; every other atom (n_points > 128, more than kNbCap neighbours) streams both evaluations,
 // because atom_fast keeps no per-point result.
-template <bool HAS_MASK>
+// HAS_PAIRS: every atom also writes its partner slots (pp).  The cap path gets them from cap_atom_groups; every other atom with an
+// other-group neighbour (or with too many neighbours to tell) enumerates its partners over the cell rows and is evaluated once more
+// per partner with only its group and the partner's present (PairAtoms).
+template <bool HAS_MASK, bool HAS_PAIRS = false>
 __device__ __forceinline__ void large_groups_body(const KParams &p, const GroupParams &gp, int N, uint32_t a0, LargeHeader *h,
                                                   const float4 *__restrict__ sorted, const uint32_t *__restrict__ orig,
                                                   const uint32_t *__restrict__ cls_sorted, const uint32_t *__restrict__ grp_sorted,
                                                   const uint32_t *__restrict__ cells, const uint32_t *__restrict__ bstart, float *val,
-                                                  float *val_iso, uint32_t blk, const MaskParams &mp, const MaskParams &mpi) {
+                                                  float *val_iso, uint32_t blk, const MaskParams &mp, const MaskParams &mpi,
+                                                  const PairParams &pp = PairParams{}) {
+    static_assert(!(HAS_MASK && HAS_PAIRS), "masks and pair slots are separate instantiations");
     __shared__ __align__(16) float4 s_ent[8 * kNbCap];
     __shared__ uint32_t s_cand[8 * kNbCap];
     __shared__ __align__(16) float4 s_ptab[128];
@@ -684,6 +689,8 @@ __device__ __forceinline__ void large_groups_body(const KParams &p, const GroupP
             large_blank_masks(p, mp, N, a0);
             large_blank_masks(p, mpi, N, a0);
         }
+        if (HAS_PAIRS)
+            pair_blank_rows(pp, a0, (size_t)N, (size_t)blockIdx.x * blockDim.x + threadIdx.x, (size_t)gridDim.x * blockDim.x);
         return;
     }
     const Grid g = h->grid;
@@ -726,12 +733,41 @@ __device__ __forceinline__ void large_groups_body(const KParams &p, const GroupP
             uint32_t *const mrow = HAS_MASK ? mask_row(mp, p.n_points, a0 + orig[pos]) : nullptr;
             uint32_t *const irow = HAS_MASK ? mask_row(mpi, p.n_points, a0 + orig[pos]) : nullptr;
             float cnt, cnt_iso;
+            PairSlot ps;
             if (k >= 0) pairs += (unsigned)k;
             if (k >= 0 && use_cap) {
                 int iso;
-                cnt = (float)cap_atom_groups<false, HAS_MASK>(p.cap, atoms, ai, p.probe, w_cand, k, grp_sorted, gi, s_ptab, (int)p.n_points,
-                                                              nbody, 0ull, &iso, mrow, irow);
+                cnt = (float)cap_atom_groups<false, HAS_MASK, HAS_PAIRS>(p.cap, atoms, ai, p.probe, w_cand, k, grp_sorted, gi, s_ptab,
+                                                                         (int)p.n_points, nbody, 0ull, &iso, mrow, irow, &ps);
                 cnt_iso = (float)iso;
+            } else if (HAS_PAIRS) {
+                bool other = true;   // an atom whose complex neighbours all share its group has no partner
+                if (k >= 0) {
+                    bool o = false;
+                    for (int q = lane; q < k; q += 32) o |= grp_sorted[w_cand[q]] != gi;
+                    other = __any_sync(kFull, o);
+                }
+                cnt = large_eval_atom(p, g, atoms, cells, cls_sorted, pos, ai, k, w_cand, w_ent, s_pts, streamed);
+                __syncwarp();
+                const GroupAtoms<true> iso_atoms{sorted, grp_sorted, gi};
+                const int k2 = cc.total >= 0 ? gather_cached(p, iso_atoms, cls_sorted, pos, ai, cc, w_cand)
+                                             : gather_candidates(p, g, iso_atoms, cells, cls_sorted, pos, ai, w_cand);
+                cnt_iso = large_eval_atom(p, g, iso_atoms, cells, cls_sorted, pos, ai, k2, w_cand, w_ent, s_pts, streamed);
+                ps = pair_empty();
+                bool first = true;
+                uint32_t gh = 0u;
+                const float reach_i = ai.w + 2.0f * p.probe + kCutSlack;
+                while (other && cnt_iso > 0.0f &&
+                       pair_next_scan(g, cells, atoms, grp_sorted, pos, ai, reach_i, gi, first, gh, gh)) {
+                    first = false;
+                    __syncwarp();
+                    const PairAtoms<true> pair_atoms{sorted, grp_sorted, gi, gh};
+                    const int k3 = cc.total >= 0 ? gather_cached(p, pair_atoms, cls_sorted, pos, ai, cc, w_cand)
+                                                 : gather_candidates(p, g, pair_atoms, cells, cls_sorted, pos, ai, w_cand);
+                    unsigned long long pair_streamed = 0;   // (the statistics count each atom's complex and isolated evaluations only)
+                    const float cp = large_eval_atom(p, g, pair_atoms, cells, cls_sorted, pos, ai, k3, w_cand, w_ent, s_pts, pair_streamed);
+                    pair_take(ps, gh, (int)cnt_iso - (int)cp);
+                }
             } else if (HAS_MASK) {
                 cnt = atom_streaming<GlobalAtoms, uint32_t, false, true>(p, g, atoms, cells, cls_sorted, pos, w_ent, nullptr, mrow);
                 __syncwarp();
@@ -749,6 +785,7 @@ __device__ __forceinline__ void large_groups_body(const KParams &p, const GroupP
             const uint32_t oi = orig[pos];
             large_store(p, lane, a0 + oi, oi, val, atom_area(ai.w, p.probe, cnt, p.inv_n), (uint32_t)cnt);
             large_store(iso_outputs(p, gp), lane, a0 + oi, oi, val_iso, atom_area(ai.w, p.probe, cnt_iso, p.inv_n), (uint32_t)cnt_iso);
+            if (HAS_PAIRS) pair_store(pp, a0 + oi, ps, ai.w, p.probe, p.inv_n, p.err_flag);
             __syncwarp();
         }
     }
@@ -765,6 +802,15 @@ __global__ void __launch_bounds__(256, 2) large_groups_kernel(const KParams p, c
                                                               float *val, float *val_iso, uint32_t blk) {
     large_groups_body<false>(p, gp, N, a0, h, sorted, orig, cls_sorted, grp_sorted, cells, bstart, val, val_iso, blk, MaskParams{},
                              MaskParams{});
+}
+
+__global__ void __launch_bounds__(256, 2) large_group_pairs_kernel(const KParams p, const GroupParams gp, const PairParams pp, int N,
+                                                                   uint32_t a0, LargeHeader *h, const float4 *__restrict__ sorted,
+                                                                   const uint32_t *__restrict__ orig, const uint32_t *__restrict__ cls_sorted,
+                                                                   const uint32_t *__restrict__ grp_sorted, const uint32_t *__restrict__ cells,
+                                                                   const uint32_t *__restrict__ bstart, float *val, float *val_iso, uint32_t blk) {
+    large_groups_body<false, true>(p, gp, N, a0, h, sorted, orig, cls_sorted, grp_sorted, cells, bstart, val, val_iso, blk, MaskParams{},
+                                   MaskParams{}, pp);
 }
 
 __global__ void __launch_bounds__(256, 2) large_groups_masks_kernel(const KParams p, const GroupParams gp, const MaskParams mp,
@@ -980,11 +1026,12 @@ inline int large_reserve(LargeWorkspace &w, uint32_t n_atoms) {
 // (BASELINE cfg5): the cell list is built for the whole structure, only the work blocks owned by `range_rank` are
 // evaluated, and no sums are produced.  Grouped runs (gp set; no atom-range split, no flags) go through
 // large_groups_kernel and produce the level sums of both value vectors.  Masked runs (mp set; no atom-range split) take the
-// masked instantiations of the cells / atoms kernels; masked grouped runs (gp, mp and mpi set) large_groups_masks_kernel.
+// masked instantiations of the cells / atoms kernels; masked grouped runs (gp, mp and mpi set) large_groups_masks_kernel; pairwise
+// buried area (gp and pp set) large_group_pairs_kernel.
 inline int large_enqueue(int sm_count, LargeWorkspace &w, const KParams &kp, const uint32_t *order, uint32_t n_work,
                          const uint32_t *off, const uint32_t *seg_off, cudaStream_t st, uint32_t *launches,
                          uint32_t range_rank = 0, uint32_t range_n = 1, const GroupParams *gp = nullptr,
-                         const MaskParams *mp = nullptr, const MaskParams *mpi = nullptr) {
+                         const MaskParams *mp = nullptr, const MaskParams *mpi = nullptr, const PairParams *pp = nullptr) {
     for (uint32_t q = 0; q < n_work; ++q) {
         const uint32_t sid = order[q];
         const uint32_t a0 = off[sid];
@@ -1019,7 +1066,10 @@ inline int large_enqueue(int sm_count, LargeWorkspace &w, const KParams &kp, con
         if (gp) {
             large_scatter_groups_kernel<<<gc, 256, 0, st>>>(gp->grp + a0, N, w.hdr, w.cells, w.cellid, w.rank, w.grp_sorted);
             const int ga = std::max(1, std::min((N + 8 * (int)blk - 1) / (8 * (int)blk), sm_count * 2));
-            if (mp)
+            if (pp)
+                large_group_pairs_kernel<<<ga, 256, 0, st>>>(kp, *gp, *pp, N, a0, w.hdr, w.sorted, w.orig, cls ? w.cls_sorted : nullptr,
+                                                             w.grp_sorted, w.cells, w.bstart, w.val, w.val_iso, blk);
+            else if (mp)
                 large_groups_masks_kernel<<<ga, 256, 0, st>>>(kp, *gp, *mp, *mpi, N, a0, w.hdr, w.sorted, w.orig, cls ? w.cls_sorted : nullptr,
                                                               w.grp_sorted, w.cells, w.bstart, w.val, w.val_iso, blk);
             else

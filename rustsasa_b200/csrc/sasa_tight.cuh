@@ -212,6 +212,15 @@ __device__ __noinline__ int tight_cold_atom_iso(const float *px, const float *py
     return tight_cold_eval<HAS_CLS>(px, py, pz, n_points, n_body, probe, near2, m_min, m_max, g, GroupAtoms<false>{s_atom, s_grp, s_grp[pos]},
                                     s_cell, s_cls, s_pts, pos, ent, cand, misc);
 }
+// The same with only the atom's group and partner group gh present (pairwise buried area).
+template <bool HAS_CLS>
+__device__ __noinline__ int tight_cold_atom_pair(const float *px, const float *py, const float *pz, uint32_t n_points, uint32_t n_body,
+                                                 float probe, float near2, int m_min, int m_max, Grid g, const float4 *s_atom,
+                                                 const uint32_t *s_grp, uint32_t gh, const uint16_t *s_cell, const uint32_t *s_cls,
+                                                 const float4 *s_pts, int pos, float4 *ent, uint16_t *cand, int *misc) {
+    return tight_cold_eval<HAS_CLS>(px, py, pz, n_points, n_body, probe, near2, m_min, m_max, g,
+                                    PairAtoms<false>{s_atom, s_grp, s_grp[pos], gh}, s_cell, s_cls, s_pts, pos, ent, cand, misc);
+}
 // The isolated evaluation of a masked grouped run: the atom streams with its group standing alone and writes its isolated row.
 template <bool HAS_CLS>
 __device__ __noinline__ int tight_cold_atom_iso_mask(const float *px, const float *py, const float *pz, uint32_t n_points, uint32_t n_body,
@@ -225,9 +234,11 @@ __device__ __noinline__ int tight_cold_atom_iso_mask(const float *px, const floa
 // HAS_GRP: grouped run -- every atom is evaluated in the complex and with its group standing alone (the cap path in one pass,
 // cap_atom_groups; the cold path twice), and the output stage runs once per value array.
 // HAS_MASK: every atom also writes its exposed-point mask row (mp); cold atoms stream.  With HAS_GRP also its isolated row (mpi).
-template <int NT, int MINB, bool HAS_CLS, uint32_t CMAX, bool HAS_GRP, bool HAS_MASK = false>
+// HAS_PAIRS (with HAS_GRP): every atom also writes its partner slots (pp).  Cap-path atoms get them from cap_atom_groups; a cold
+// atom enumerates its partners over the cell rows and is evaluated once more per partner with only its group and the partner's.
+template <int NT, int MINB, bool HAS_CLS, uint32_t CMAX, bool HAS_GRP, bool HAS_MASK = false, bool HAS_PAIRS = false>
 __device__ __forceinline__ void tight_kernel_body(const KParams &p, const GroupParams &gp, const MaskParams &mp = MaskParams{},
-                                                  const MaskParams &mpi = MaskParams{}) {
+                                                  const MaskParams &mpi = MaskParams{}, const PairParams &pp = PairParams{}) {
     extern __shared__ __align__(16) unsigned char smem[];
     constexpr int NW = NT / 32;
     constexpr uint32_t NMAX = max_atoms(NT, MINB, CMAX, HAS_CLS, HAS_GRP);
@@ -262,6 +273,7 @@ __device__ __forceinline__ void tight_kernel_body(const KParams &p, const GroupP
         if (!ok) {
             if (HAS_MASK) mask_zero_rows(mp, p.n_points, a0, (size_t)N, threadIdx.x, NT);
             if (HAS_GRP && HAS_MASK) mask_zero_rows(mpi, p.n_points, a0, (size_t)N, threadIdx.x, NT);
+            if (HAS_PAIRS) pair_blank_rows(pp, a0, (size_t)N, threadIdx.x, NT);
             continue;
         }
         // the structure's cell grid (eight CTA-uniform values) in uniform registers
@@ -332,7 +344,12 @@ __device__ __forceinline__ void tight_kernel_body(const KParams &p, const GroupP
                     uint32_t *const mrow = HAS_MASK ? mask_row(mp, p.n_points, a0 + V.orig[pos]) : nullptr;
                     uint32_t *const irow = HAS_GRP && HAS_MASK ? mask_row(mpi, p.n_points, a0 + V.orig[pos]) : nullptr;
                     if (k <= kNbCap) {
-                        if (HAS_GRP)
+                        if (HAS_PAIRS) {
+                            PairSlot ps;
+                            cnt = cap_atom_groups<true, false, true>(p.cap, SmemAtoms{V.atom}, ai, p.probe, w_nba, k, V.grp, V.grp[pos],
+                                                                     V.ptab, (int)p.n_points, nbody, p.cap_tex, &cnt_iso, nullptr, nullptr, &ps);
+                            pair_store(pp, a0 + V.orig[pos], ps, ai.w, p.probe, p.inv_n, p.err_flag);
+                        } else if (HAS_GRP)
                             cnt = cap_atom_groups<true, HAS_MASK>(p.cap, SmemAtoms{V.atom}, ai, p.probe, w_nba, k, V.grp, V.grp[pos], V.ptab,
                                                                   (int)p.n_points, nbody, p.cap_tex, &cnt_iso, mrow, irow);
                         else
@@ -351,6 +368,20 @@ __device__ __forceinline__ void tight_kernel_body(const KParams &p, const GroupP
                         if (HAS_GRP)
                             cnt_iso = tight_cold_atom_iso<HAS_CLS>(p.px, p.py, p.pz, p.n_points, p.n_body, p.probe, p.near2, p.m_min,
                                                                    p.m_max, g, V.atom, V.grp, V.cell, V.cls, V.ptab, pos, w_ent, w_cand, V.misc);
+                        if (HAS_PAIRS) {
+                            PairSlot ps = pair_empty();
+                            const uint32_t gi = V.grp[pos];
+                            bool first = true;
+                            uint32_t h = 0u;
+                            while (cnt_iso > 0 && pair_next_scan(g, V.cell, SmemAtoms{V.atom}, V.grp, pos, ai, ai.w + reach0, gi, first, h, h)) {
+                                first = false;
+                                const int cp = tight_cold_atom_pair<HAS_CLS>(p.px, p.py, p.pz, p.n_points, p.n_body, p.probe, p.near2,
+                                                                             p.m_min, p.m_max, g, V.atom, V.grp, h, V.cell, V.cls, V.ptab,
+                                                                             pos, w_ent, w_cand, V.misc);
+                                pair_take(ps, h, cnt_iso - cp);
+                            }
+                            pair_store(pp, a0 + V.orig[pos], ps, ai.w, p.probe, p.inv_n, p.err_flag);
+                        }
                     }
                     if (lane == 0) {
                         const int oi = (int)V.orig[pos];
@@ -392,6 +423,12 @@ __global__ void __launch_bounds__(NT, MINB) sasa_tight_masks_kernel(const KParam
 template <int NT, int MINB, bool HAS_CLS, uint32_t CMAX>
 __global__ void __launch_bounds__(NT, MINB) sasa_tight_groups_kernel(const KParams p, const GroupParams gp) {
     tight_kernel_body<NT, MINB, HAS_CLS, CMAX, true>(p, gp);
+}
+
+// Pairwise buried area (n_points <= 128): the grouped run's outputs plus every atom's partner slots (pp).
+template <int NT, int MINB, bool HAS_CLS, uint32_t CMAX>
+__global__ void __launch_bounds__(NT, MINB) sasa_tight_group_pairs_kernel(const KParams p, const GroupParams gp, const PairParams pp) {
+    tight_kernel_body<NT, MINB, HAS_CLS, CMAX, true, false, true>(p, gp, MaskParams{}, MaskParams{}, pp);
 }
 
 // Grouped runs with exposed-point masks (n_points <= 128): the grouped run's outputs plus every atom's mask row in the complex

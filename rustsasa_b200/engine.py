@@ -8,7 +8,7 @@ from __future__ import annotations
 
 import ctypes as C
 from dataclasses import dataclass
-from typing import Optional
+from typing import Any, Optional
 
 import numpy as np
 
@@ -82,6 +82,49 @@ class BatchResult:
     stats: Optional[dict] = None
     exposed: Optional[np.ndarray] = None   # (n_atoms, W) uint32 exposed-point masks (run_masks_host, run_groups_masks_host),
                                            # W = ceil(n_points / 32)
+
+
+@dataclass
+class PairResult:
+    """Partner slots of a pairwise buried-area run (``Batch.run_group_pairs_host`` / ``_device``), K = max_partners slots per
+    atom in batch order: ``partner`` (N, K) uint32 partner group labels in ascending order, ``buried_counts`` (N, K) uint32 the
+    points of the atom open with its group alone that the partner hides, ``buried_area`` (N, K) float32 the reference's area
+    expression on that count.  Unused slots hold partner 0xFFFFFFFF, count 0 and area 0; a slot is in use exactly when its count
+    is non-zero.  ``needed``: the largest number of partners of an atom (an int; a one-element device tensor for the device
+    form)."""
+    partner: Any = None
+    buried_counts: Any = None
+    buried_area: Any = None
+    needed: Any = None
+
+
+def group_pair_table(partner, buried_area, group, struct_off):
+    """Pairwise interface table from the partner slots of a pairwise buried-area run: per structure a list of rows
+    ``(g, h, area of g buried by h, area of h buried by g)``, one for each contacting pair of labels g < h, in ascending (g, h)
+    order.  A slot counts when its partner label is not 0xFFFFFFFF or its area is positive.  Each area is a float64 sum over
+    the per-atom float32 slot areas, added in batch atom order."""
+    partner = np.asarray(partner, np.uint32)
+    n = partner.shape[0]
+    partner = partner.reshape(n, -1)
+    area = np.asarray(buried_area, np.float32).reshape(n, -1)
+    group = np.asarray(group, np.uint32).reshape(-1)
+    off = np.asarray(struct_off, np.int64).reshape(-1)
+    S = off.shape[0] - 1
+    used = (partner != np.uint32(0xFFFFFFFF)) | (area > 0)
+    atom, slot = np.nonzero(used)                        # atom-major: batch atom order
+    sid = np.searchsorted(off, atom, side="right") - 1
+    g = group[atom].astype(np.int64)
+    h = partner[atom, slot].astype(np.int64)
+    tables = [[] for _ in range(max(S, 0))]
+    if atom.shape[0] == 0:
+        return tables
+    keys, inv = np.unique(np.stack([sid, g, h], axis=1), axis=0, return_inverse=True)
+    sums = np.zeros(keys.shape[0], np.float64)
+    np.add.at(sums, inv.reshape(-1), area[atom, slot].astype(np.float64))   # unbuffered, in index (= atom) order
+    by_key = {tuple(int(x) for x in k): float(v) for k, v in zip(keys, sums)}
+    for (s, a, b) in sorted({(s, min(a, b), max(a, b)) for (s, a, b) in by_key}):
+        tables[s].append((a, b, by_key.get((s, a, b), 0.0), by_key.get((s, b, a), 0.0)))
+    return tables
 
 
 class Engine:
@@ -309,6 +352,58 @@ class Batch:
                                                                   C.byref(outs[0]), C.byref(outs[1]), C.byref(st)))
         cpx.stats = iso.stats = st.as_dict()
         return cpx, iso
+
+    def run_group_pairs_host(self, xyzr, group, id_class=None, probe_radius=1.4, n_points=100, simd_lanes=8, flags=0,
+                             want=("counts", "atom", "seg", "protein"), max_partners=4):
+        """Pairwise buried area: run_groups_host plus, for every atom, which partner groups bury how much of it.  Returns
+        (complex, isolated, pairs): the first two are run_groups_host's BatchResults bit for bit, pairs a :class:`PairResult` of
+        (n_atoms, max_partners) arrays.  When an atom has more than max_partners partners, :class:`SasaB200Error` is raised
+        with ``needed`` (the max_partners the batch needs) and ``result`` (the (complex, isolated, pairs) triple, complete
+        except for the partners past the slots) set on the exception."""
+        xyzr = _np(xyzr, np.float32, (-1, 4))
+        assert xyzr.shape[0] == self.n_atoms, "xyzr does not match struct_off"
+        group = _np(group, np.uint32)
+        assert group is None or group.shape[0] == self.n_atoms, "group does not match struct_off"
+        id_class = _np(id_class, np.uint32)
+        cpx, iso = self._host_outputs(want, "numpy"), self._host_outputs(want, "numpy")
+        K = int(max_partners)
+        shape = (self.n_atoms, max(K, 0))
+        pairs = PairResult(np.zeros(shape, np.uint32), np.zeros(shape, np.uint32), np.zeros(shape, np.float32))
+        needed = np.zeros(1, np.uint32)
+        outs = [_lib.Outputs(_ptr(r.counts), _ptr(r.atom_sasa), _ptr(r.seg_sasa), _ptr(r.protein)) for r in (cpx, iso)]
+        po = _lib.PairOutputs(K, _ptr(pairs.partner), _ptr(pairs.buried_counts), _ptr(pairs.buried_area), _ptr(needed))
+        prm = self._params(probe_radius, n_points, simd_lanes, flags)
+        st = _lib.Stats()
+        rc = self._L.sasa_b200_batch_run_group_pairs_host(self._h, _ptr(xyzr), _ptr(id_class), _ptr(group), C.byref(prm),
+                                                          C.byref(outs[0]), C.byref(outs[1]), C.byref(po), C.byref(st))
+        pairs.needed = int(needed[0])
+        cpx.stats = iso.stats = st.as_dict()
+        if rc != _lib.OK:
+            err = SasaB200Error(rc, self._L.sasa_b200_last_error(self.engine._h).decode())
+            err.needed, err.result = pairs.needed, (cpx, iso, pairs)
+            raise err
+        return cpx, iso, pairs
+
+    def run_group_pairs_device(self, d_xyzr, d_group, d_id_class=None, probe_radius=1.4, n_points=100, simd_lanes=8, flags=0,
+                               want=("counts", "atom", "seg", "protein"), max_partners=4, stream=None):
+        """run_group_pairs_host on torch CUDA tensors: allocates every output on the input's device, enqueues on `stream` (None
+        = torch's current stream) and returns (complex, isolated, pairs) of tensors without synchronising; ``pairs.needed`` is a
+        one-element int32 tensor.  Too few slots is reported by ``Batch.sync`` (:class:`SasaB200Error`), like non-finite
+        input."""
+        import torch
+        dev = d_xyzr.device
+        cpx, iso = self._device_outputs(want, dev), self._device_outputs(want, dev)
+        K = int(max_partners)
+        shape = (self.n_atoms, max(K, 0))
+        pairs = PairResult(torch.empty(shape, dtype=torch.int32, device=dev), torch.empty(shape, dtype=torch.int32, device=dev),
+                           torch.empty(shape, dtype=torch.float32, device=dev), torch.zeros(1, dtype=torch.int32, device=dev))
+        outs = [_lib.Outputs(_ptr(r.counts), _ptr(r.atom_sasa), _ptr(r.seg_sasa), _ptr(r.protein)) for r in (cpx, iso)]
+        po = _lib.PairOutputs(K, _ptr(pairs.partner), _ptr(pairs.buried_counts), _ptr(pairs.buried_area), _ptr(pairs.needed))
+        prm = self._params(probe_radius, n_points, simd_lanes, flags)
+        self.engine._check(self._L.sasa_b200_batch_run_group_pairs_device(self._h, _ptr(d_xyzr), _ptr(d_id_class), _ptr(d_group),
+                                                                         C.byref(prm), C.byref(outs[0]), C.byref(outs[1]), C.byref(po),
+                                                                         _stream(stream)))
+        return cpx, iso, pairs
 
     def _groups_frames_args(self, xyz, radii, group):
         xyz = _np(xyz, np.float32, (-1, 3))
