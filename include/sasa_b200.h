@@ -292,6 +292,38 @@ SASA_B200_API int sasa_b200_batch_submit_groups_frames_host(sasa_b200_batch *bat
                                               const sasa_b200_outputs *out, const sasa_b200_outputs *out_isolated,
                                               sasa_b200_job **out_job);
 
+/* Pairwise buried area of MD frames: per frame, how much of every group each partner group buries, summed on the device.  The
+ * batch, xyz, radii and group are exactly as in sasa_b200_batch_run_groups_frames_host; the labels must be 0 .. n_labels - 1.
+ * The run is the pairwise buried-area run of sasa_b200_batch_run_group_pairs_host on the frames (K = max(1, n_labels - 1) slots
+ * per atom, so no atom can have more partners than slots); its slot rows stay in device memory and only their sums come back.
+ *   pair_area      [S * L * L]: element (s * L + g) * L + h is the sum of the slot areas with partner h over the atoms of group
+ *                  g in frame s -- started at 0.0, added in float64, in the frame's atom order.  This is what
+ *                  rustsasa_b200.group_pair_table computes from the slots on the host, bit for bit.  The diagonal is 0, and a
+ *                  label with no atoms has zero rows and columns.
+ *   seg_pair_area  [n_segments * L], nullable: element q * L + h is the same float64 atom-order sum over segment q's atom range
+ *                  (relative to its frame's first atom, as everywhere in this ABI). */
+typedef struct sasa_b200_pair_sums {
+    uint32_t n_labels;       /* L, 1..17: group labels are 0 .. L - 1                                                 */
+    double *pair_area;       /* [S * L * L]                                                                           */
+    double *seg_pair_area;   /* [n_segments * L], nullable                                                            */
+} sasa_b200_pair_sums;       /* (host pointers)                                                                       */
+
+/* out: bit for bit sasa_b200_batch_run_frames_host; out_isolated: bit for bit sasa_b200_batch_run_groups_frames_host; every
+ * field of both nullable.  xyz, radii or group NULL with atoms in the batch, out_isolated NULL, sums or sums->pair_area NULL
+ * with atoms in the batch, n_labels outside 1..17, a label >= n_labels, frames of unequal size or an output size that overflows
+ * size_t: SASA_B200_ERR_INVALID_ARGUMENT; params->flags != 0: SASA_B200_ERR_UNSUPPORTED.  Non-finite input:
+ * SASA_B200_ERR_NON_FINITE with both output sets NaN-filled, and the frame's L x L block and all its segment rows NaN, for that
+ * frame only.  An empty batch does nothing.  Uses the per-chunk pipeline; submit / sasa_b200_job_wait split the run as for
+ * sasa_b200_batch_submit_groups_frames_host. */
+SASA_B200_API int sasa_b200_batch_run_group_pairs_frames_host(sasa_b200_batch *batch, const float *xyz, const float *radii,
+                                                const uint32_t *group, const sasa_b200_params *params,
+                                                const sasa_b200_outputs *out, const sasa_b200_outputs *out_isolated,
+                                                const sasa_b200_pair_sums *sums, sasa_b200_stats *stats /* nullable */);
+SASA_B200_API int sasa_b200_batch_submit_group_pairs_frames_host(sasa_b200_batch *batch, const float *xyz, const float *radii,
+                                                   const uint32_t *group, const sasa_b200_params *params,
+                                                   const sasa_b200_outputs *out, const sasa_b200_outputs *out_isolated,
+                                                   const sasa_b200_pair_sums *sums, sasa_b200_job **out_job);
+
 /* Indexed-radius form: 13 bytes per atom on the wire instead of 16.  Proteins use a handful of distinct radii (ProtOr,
  * radii/protor.config, has ten), so the extraction step (build_atoms_and_mapping, src/options.rs:81-116) can emit
  * coordinates as 3 floats per atom plus ONE BYTE per atom indexing a palette of at most 256 radii.  With eight GPUs pulling

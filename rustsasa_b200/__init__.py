@@ -8,11 +8,11 @@ Engine / Batch wrapper (``engine``) and a mirror of the reference's public inter
 from .api import (Atom, AtomLevel, ChainLevel, ChainResult, GroupPairResult, InterfacePairsResult,  # noqa: F401
                   InterfaceResult, InterfaceSurfaceResult, ProteinLevel, ProteinResult, ResidueLevel, ResidueResult, SASACalcError, SASAOptions, SurfaceResult,
                   TrajectoryInterfaceResult, calculate_sasa_internal, default_engine, surface_points, trajectory_interface)
-from .engine import Batch, BatchResult, Engine, PairResult, SasaB200Error, group_pair_table  # noqa: F401
+from .engine import Batch, BatchResult, Engine, PairResult, PairSums, SasaB200Error, group_pair_table  # noqa: F401
 from .structure import read_structure  # noqa: F401
 
 __all__ = ["Atom", "AtomLevel", "ResidueLevel", "ChainLevel", "ProteinLevel", "ChainResult", "ResidueResult",
            "ProteinResult", "SASACalcError", "SASAOptions", "SurfaceResult", "InterfaceResult", "InterfaceSurfaceResult",
            "GroupPairResult", "InterfacePairsResult", "TrajectoryInterfaceResult", "calculate_sasa_internal", "default_engine",
            "surface_points", "trajectory_interface", "Engine",
-           "Batch", "BatchResult", "PairResult", "SasaB200Error", "group_pair_table", "read_structure"]
+           "Batch", "BatchResult", "PairResult", "PairSums", "SasaB200Error", "group_pair_table", "read_structure"]

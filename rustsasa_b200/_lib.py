@@ -29,6 +29,7 @@ EXPORTS = [
     "sasa_b200_batch_run_masks_host", "sasa_b200_batch_run_masks_device", "sasa_b200_batch_run_groups_masks_host",
     "sasa_b200_batch_run_groups_masks_device", "sasa_b200_batch_run_groups_frames_host", "sasa_b200_batch_submit_groups_frames_host",
     "sasa_b200_batch_run_group_pairs_host", "sasa_b200_batch_run_group_pairs_device",
+    "sasa_b200_batch_run_group_pairs_frames_host", "sasa_b200_batch_submit_group_pairs_frames_host",
 ]
 
 
@@ -45,6 +46,10 @@ class Outputs(C.Structure):
 class PairOutputs(C.Structure):
     _fields_ = [("max_partners", C.c_uint32), ("partner", C.c_void_p), ("buried_counts", C.c_void_p),
                 ("buried_area", C.c_void_p), ("partners_needed", C.c_void_p)]
+
+
+class PairSums(C.Structure):
+    _fields_ = [("n_labels", C.c_uint32), ("pair_area", C.c_void_p), ("seg_pair_area", C.c_void_p)]
 
 
 class Stats(C.Structure):
@@ -104,6 +109,10 @@ def load() -> C.CDLL:
                                                        C.POINTER(PairOutputs), C.POINTER(Stats)]
     L.sasa_b200_batch_run_group_pairs_device.argtypes = [vp, vp, vp, vp, C.POINTER(Params), C.POINTER(Outputs), C.POINTER(Outputs),
                                                          C.POINTER(PairOutputs), vp]
+    L.sasa_b200_batch_run_group_pairs_frames_host.argtypes = [vp, vp, vp, vp, C.POINTER(Params), C.POINTER(Outputs),
+                                                              C.POINTER(Outputs), C.POINTER(PairSums), C.POINTER(Stats)]
+    L.sasa_b200_batch_submit_group_pairs_frames_host.argtypes = [vp, vp, vp, vp, C.POINTER(Params), C.POINTER(Outputs),
+                                                                 C.POINTER(Outputs), C.POINTER(PairSums), C.POINTER(vp)]
     L.sasa_b200_batch_submit_host.argtypes = [vp, vp, vp, C.POINTER(Params), C.POINTER(Outputs), C.POINTER(vp)]
     L.sasa_b200_batch_submit_frames_host.argtypes = [vp, vp, vp, C.POINTER(Params), C.POINTER(Outputs), C.POINTER(vp)]
     L.sasa_b200_job_wait.argtypes = [vp, C.POINTER(Stats)]

@@ -126,12 +126,17 @@ class InterfacePairsResult:
 class TrajectoryInterfaceResult:
     """``trajectory_interface``: per frame the protein totals (global, polar, non-polar) in the complex and with every group
     standing alone, (F, 3) float32 each, the buried area isolated - complex of the global totals (F,), and with residue ranges
-    given, the segment sums (F, G) of both."""
+    given, the segment sums (F, G) of both.  With ``pairs=True``: ``pair_labels`` (L,) the distinct labels in ascending order,
+    ``pair_area`` (F, L, L) float64, element [f, a, b] the area of group pair_labels[a] that group pair_labels[b] buries in frame f,
+    and with residue ranges given ``seg_pair_area`` (F, G, L) float64, the area of each residue that each group buries."""
     complex: np.ndarray
     isolated: np.ndarray
     buried: np.ndarray
     complex_seg: Optional[np.ndarray] = None
     isolated_seg: Optional[np.ndarray] = None
+    pair_labels: Optional[np.ndarray] = None
+    pair_area: Optional[np.ndarray] = None
+    seg_pair_area: Optional[np.ndarray] = None
 
 
 class AtomLevel:
@@ -184,7 +189,8 @@ _TRAJECTORY_STAGING_BYTES = 256 << 20
 
 
 def trajectory_interface(xyz, radii, group, seg_be=None, seg_polar=None, probe_radius: float = 1.4, n_points: int = 100,
-                         frames_per_call: Optional[int] = None, engine: Optional[Engine] = None) -> TrajectoryInterfaceResult:
+                         frames_per_call: Optional[int] = None, engine: Optional[Engine] = None,
+                         pairs: bool = False) -> TrajectoryInterfaceResult:
     """Buried surface area along an MD trajectory.  ``xyz`` (F, N, 3) frames (any array, a numpy memmap included: blocks of
     frames are copied into page-locked staging), ``radii`` (N,) and ``group`` (N,) labels shared by every frame; ``seg_be``
     (G, 2) residue ranges within a frame and ``seg_polar`` (G,) their polar flags, both optional.
@@ -193,7 +199,11 @@ def trajectory_interface(xyz, radii, group, seg_be=None, seg_polar=None, probe_r
     it fits 256 MB of staging, else as many frames as do).  Two batches alternate, so the next block is staged and submitted
     before the current one is waited for: the host copy of block k + 1 and its transfer overlap the kernels of block k, and a
     trajectory of any length runs with bounded memory.  The results equal one ``run_groups_frames_host`` over all frames bit
-    for bit."""
+    for bit.
+
+    ``pairs=True`` adds, per frame, how much of every group each other group buries (and per residue, with residue ranges),
+    summed on the device by ``Batch.submit_group_pairs_frames_host``: the labels are numbered 0 .. L - 1 in ascending order, and
+    more than 17 distinct labels raise ValueError."""
     eng = engine or default_engine()
     if not isinstance(xyz, np.ndarray):
         xyz = np.asarray(xyz, np.float32)
@@ -207,12 +217,23 @@ def trajectory_interface(xyz, radii, group, seg_be=None, seg_polar=None, probe_r
     seg = None if seg_be is None else np.ascontiguousarray(seg_be, np.uint32).reshape(-1, 2)
     pol = None if seg_polar is None or seg is None else np.ascontiguousarray(seg_polar, np.uint8).reshape(-1)
     G = 0 if seg is None else seg.shape[0]
+    labels = None
+    if pairs:
+        labels, dense = np.unique(group, return_inverse=True)
+        if labels.shape[0] > 17:
+            raise ValueError(f"pairs=True supports at most 17 distinct group labels, got {labels.shape[0]}")
+        group = dense.astype(np.uint32).reshape(-1)
+    L = 1 if labels is None else max(1, labels.shape[0])
     if frames_per_call is None:
         frames_per_call = max(1, _TRAJECTORY_STAGING_BYTES // max(1, N * 12))
     B = max(1, min(int(frames_per_call), F))
     want = ("protein", "seg") if G else ("protein",)
     out = TrajectoryInterfaceResult(np.zeros((F, 3), np.float32), np.zeros((F, 3), np.float32), np.zeros(F, np.float32),
                                     np.zeros((F, G), np.float32) if G else None, np.zeros((F, G), np.float32) if G else None)
+    if pairs:
+        out.pair_labels = labels
+        out.pair_area = np.zeros((F, L, L), np.float64)
+        out.seg_pair_area = np.zeros((F, G, L), np.float64) if G else None
     if F == 0:
         return out
 
@@ -224,6 +245,8 @@ def trajectory_interface(xyz, radii, group, seg_be=None, seg_polar=None, probe_r
             self.batch = Batch(eng, (np.arange(fb + 1) * N).astype(np.uint64), *topo)
             self.stage = eng.pinned_empty((fb, N, 3), np.float32)
             self.res = (self.batch._host_outputs(want, "pinned"), self.batch._host_outputs(want, "pinned"))
+            if pairs:
+                self.res += (self.batch._pair_sums(L, True, "pinned"),)
 
     slots = {}
 
@@ -239,6 +262,8 @@ def trajectory_interface(xyz, radii, group, seg_be=None, seg_polar=None, probe_r
         f0, f1 = blocks[k]
         s = slot_for(k, f1 - f0)
         np.copyto(s.stage, xyz[f0:f1], casting="same_kind")
+        if pairs:
+            return s, s.batch.submit_group_pairs_frames_host(s.stage, radii, group, L, probe_radius, n_points, want=want, result=s.res)
         return s, s.batch.submit_groups_frames_host(s.stage, radii, group, probe_radius, n_points, want=want, result=s.res)
 
     pending = None
@@ -247,13 +272,17 @@ def trajectory_interface(xyz, radii, group, seg_be=None, seg_polar=None, probe_r
         for k in range(len(blocks)):
             s, job = pending
             pending = submit(k + 1) if k + 1 < len(blocks) else None
-            cpx, iso = job.wait()
+            cpx, iso, *sums = job.wait()
             f0, f1 = blocks[k]
             out.complex[f0:f1] = cpx.protein
             out.isolated[f0:f1] = iso.protein
             if G:
                 out.complex_seg[f0:f1] = cpx.seg_sasa.reshape(f1 - f0, G)
                 out.isolated_seg[f0:f1] = iso.seg_sasa.reshape(f1 - f0, G)
+            if pairs:
+                out.pair_area[f0:f1] = sums[0].pair_area
+                if G:
+                    out.seg_pair_area[f0:f1] = sums[0].seg_pair_area.reshape(f1 - f0, G, L)
     finally:
         if pending is not None:   # an error left a block in flight: its buffers stay alive until it is done
             try:

@@ -7,7 +7,7 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SRC = os.path.join(HERE, "csrc", "sasa_api.cu")
-DEPS = [os.path.join(HERE, "csrc", f) for f in ("sasa_api.cu", "sasa_device.cuh", "sasa_tight.cuh", "sasa_cap.cuh", "sasa_small.cuh", "sasa_large.cuh")]
+DEPS = [os.path.join(HERE, "csrc", f) for f in ("sasa_api.cu", "sasa_device.cuh", "sasa_tight.cuh", "sasa_cap.cuh", "sasa_small.cuh", "sasa_large.cuh", "sasa_pair_sums.cuh")]
 DEPS.append(os.path.join(os.path.dirname(HERE), "include", "sasa_b200.h"))
 OUT = os.path.join(HERE, "libsasa_b200.so")
 

@@ -27,6 +27,7 @@
 #include <vector>
 
 #include "sasa_large.cuh"
+#include "sasa_pair_sums.cuh"
 #include "sasa_small.cuh"
 #include "sasa_tight.cuh"
 
@@ -1039,7 +1040,7 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
                             sasa_b200_job **out_job, const uint8_t *ridx = nullptr, size_t n_palette = 0,
                             const uint32_t *group = nullptr, const sasa_b200_outputs *out_iso = nullptr, bool masked = false,
                             uint32_t *exposed = nullptr, uint32_t *exposed_iso = nullptr, bool pairs = false,
-                            const sasa_b200_pair_outputs *pair_out = nullptr) {
+                            const sasa_b200_pair_outputs *pair_out = nullptr, const sasa_b200_pair_sums *sums = nullptr) {
     sasa_b200_ctx *ctx = b->ctx;
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (!out || !out_job) return fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "out / out_job is NULL");
@@ -1056,9 +1057,9 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
     const size_t W = mask_words(params->n_points);
     const int variant = (id_class ? 1 : 0) + (grouped ? 4 : 0);
     if (grouped && (rc = prepare_groups(b, group, params, out_iso, variant)) != 0) return rc;
-    if (pairs && (rc = check_pairs(b, pair_out)) != 0) return rc;
-    if (pairs && !pair_out) pairs = false;   // (an empty batch: no slots to write)
-    const size_t K = pairs ? pair_out->max_partners : 0;
+    // sums (pairwise buried area of MD frames): the slot rows stay in the arena, only their sums per frame and segment come back
+    if (pairs && !sums && (rc = check_pairs(b, pair_out)) != 0) return rc;
+    if (pairs && !sums && !pair_out) pairs = false;   // (an empty batch: no slots to write)
     const bool indexed = xyz3 != nullptr && ridx != nullptr;   // 13 B/atom: coordinates + a palette index per atom
     const bool frames = xyz3 != nullptr;                       // any 12-byte coordinate form
     size_t fN = 0;  // atoms per frame (MD form) / palette entries (indexed form)
@@ -1071,6 +1072,21 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
                 return fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "run_frames needs equal-sized structures");
     }
     if (indexed && (n_palette == 0 || n_palette > 256)) return fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "the radius palette holds 1..256 entries");
+    // K = L - 1 slots hold every partner an atom can have, so the too-few-slots failure of the pairs kernels cannot occur
+    const uint32_t L = sums ? sums->n_labels : 0;
+    if (sums) {
+        if (L < 1 || L > kPairSumsMaxLabels) return fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "n_labels must be 1..%u, got %u", kPairSumsMaxLabels, L);
+        if (!sums->pair_area && N) return fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "sums->pair_area is NULL");
+        for (size_t i = 0; i < fN; ++i)
+            if (group[i] >= L)
+                return fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "group[%zu] = %u is not below n_labels = %u", i, group[i], L);
+        if ((N && std::max<size_t>(1, L - 1) > SIZE_MAX / 4 / N) || (S && (size_t)L * L > SIZE_MAX / 8 / S) || (G && L > SIZE_MAX / 8 / G))
+            return fail(ctx, SASA_B200_ERR_INVALID_ARGUMENT, "the pair outputs (%zu frames, %zu segments, %u labels) overflow size_t", S, G, L);
+        if (!N) pairs = false;
+    }
+    const bool want_sums = sums && sums->pair_area;
+    const bool want_seg_sums = want_sums && sums->seg_pair_area && G;
+    const size_t K = sums ? std::max<size_t>(1, L - 1) : pairs ? pair_out->max_partners : 0;
     // grouped MD form: `group` holds the fN labels of one frame, shared by every frame; they cross the wire once and are
     // expanded on the device chunk by chunk (expand_frame_labels_kernel)
     const bool frame_labels = frames && grouped;
@@ -1104,8 +1120,10 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
     const size_t o_mask = o;   o += masked ? al(N * W * 4) : 0;
     const size_t o_imask = o;  o += (masked && grouped) ? al(N * W * 4) : 0;
     const size_t o_ppart = o;  o += pairs ? al(N * K * 4) : 0;
-    const size_t o_pcnt = o;   o += (pairs && pair_out->buried_counts) ? al(N * K * 4) : 0;
-    const size_t o_parea = o;  o += (pairs && pair_out->buried_area) ? al(N * K * 4) : 0;
+    const size_t o_pcnt = o;   o += (pairs && pair_out && pair_out->buried_counts) ? al(N * K * 4) : 0;
+    const size_t o_parea = o;  o += (pairs && (sums || pair_out->buried_area)) ? al(N * K * 4) : 0;
+    const size_t o_psum = o;   o += want_sums ? al(S * L * L * 8) : 0;
+    const size_t o_pseg = o;   o += want_seg_sums ? al(G * L * 8) : 0;
     cudaStream_t s0 = ctx->streams[0];
     // the previous job may still be running on the sibling streams: this job's first stream starts behind all of them
     if (ctx->tail_valid)
@@ -1189,9 +1207,10 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
     PairParams pp{};
     if (pairs)
         pp = PairParams{reinterpret_cast<uint32_t *>(base_p + o_ppart),
-                        pair_out->buried_counts ? reinterpret_cast<uint32_t *>(base_p + o_pcnt) : nullptr,
-                        pair_out->buried_area ? reinterpret_cast<float *>(base_p + o_parea) : nullptr,
+                        (pair_out && pair_out->buried_counts) ? reinterpret_cast<uint32_t *>(base_p + o_pcnt) : nullptr,
+                        (sums || pair_out->buried_area) ? reinterpret_cast<float *>(base_p + o_parea) : nullptr,
                         reinterpret_cast<uint32_t *>(d_status + 4), (uint32_t)K};
+    double *d_psum = reinterpret_cast<double *>(base_p + o_psum), *d_pseg = reinterpret_cast<double *>(base_p + o_pseg);
     // MD form: the fused kernels read the 12-byte coordinates and the shared radius table directly; only batches with
     // structures on the large-structure path still expand to float4 first
     // (per plan: round 1 asked "any plan", so a 5,001-atom frame -- fused without id classes, large path with them -- lost both
@@ -1301,7 +1320,25 @@ static int submit_host_impl(sasa_b200_batch *b, const float *xyzr, const float *
             if (na && masked)
                 J_TRY(cudaMemcpyAsync(exposed_iso + ch.a0 * W, base_p + o_imask + ch.a0 * W * 4, na * W * 4, cudaMemcpyDeviceToHost, st));
         }
-        if (na && pairs) {
+        if (want_sums && ch.s1 > ch.s0) {
+            // the chunk's slot rows -> per-frame L x L blocks and per-segment rows, behind the chunk's kernels on its stream
+            const uint32_t ns = ch.s1 - ch.s0;
+            pair_sums_kernel<<<(ns + 3) / 4, 128, 0, st>>>(b->d_off, gp.grp, pp.partner, pp.area, (uint32_t)K, L, ch.s0, ch.s1, d_psum);
+            ++job->launches;
+            if (want_seg_sums && ch.g1 > ch.g0) {
+                const size_t nt = (ch.g1 - ch.g0) * L;
+                seg_pair_sums_kernel<<<(unsigned)((nt + 255) / 256), 256, 0, st>>>(b->d_off, b->d_seg_off, b->d_seg_be, pp.partner, pp.area,
+                                                                                   (uint32_t)K, L, ch.s0, ch.s1, (uint32_t)ch.g0,
+                                                                                   (uint32_t)ch.g1, d_psum, d_pseg);
+                ++job->launches;
+            }
+            J_TRY(cudaGetLastError());
+            const size_t blk = (size_t)L * L;
+            J_TRY(cudaMemcpyAsync(sums->pair_area + ch.s0 * blk, d_psum + ch.s0 * blk, ns * blk * 8, cudaMemcpyDeviceToHost, st));
+            if (want_seg_sums && ch.g1 > ch.g0)
+                J_TRY(cudaMemcpyAsync(sums->seg_pair_area + ch.g0 * L, d_pseg + ch.g0 * L, (ch.g1 - ch.g0) * L * 8, cudaMemcpyDeviceToHost, st));
+        }
+        if (na && pairs && pair_out) {
             J_TRY(cudaMemcpyAsync(pair_out->partner + ch.a0 * K, base_p + o_ppart + ch.a0 * K * 4, na * K * 4, cudaMemcpyDeviceToHost, st));
             if (pair_out->buried_counts)
                 J_TRY(cudaMemcpyAsync(pair_out->buried_counts + ch.a0 * K, base_p + o_pcnt + ch.a0 * K * 4, na * K * 4, cudaMemcpyDeviceToHost,
@@ -1434,6 +1471,28 @@ int sasa_b200_batch_run_groups_frames_host(sasa_b200_batch *b, const float *xyz,
                                            const sasa_b200_outputs *out_isolated, sasa_b200_stats *stats) {
     sasa_b200_job *job = nullptr;
     int rc = sasa_b200_batch_submit_groups_frames_host(b, xyz, radii, group, params, out, out_isolated, &job);
+    if (rc) return rc;
+    return wait_job_impl(job, stats);
+}
+
+int sasa_b200_batch_submit_group_pairs_frames_host(sasa_b200_batch *b, const float *xyz, const float *radii, const uint32_t *group,
+                                                   const sasa_b200_params *params, const sasa_b200_outputs *out,
+                                                   const sasa_b200_outputs *out_isolated, const sasa_b200_pair_sums *sums,
+                                                   sasa_b200_job **out_job) {
+    if (!b) return SASA_B200_ERR_INVALID_ARGUMENT;
+    if (!out_isolated) return fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "out_isolated is NULL");
+    if (b->n_atoms && (!xyz || !radii)) return fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "xyz / radii is NULL");
+    if (!sums && b->n_atoms) return fail(b->ctx, SASA_B200_ERR_INVALID_ARGUMENT, "sums is NULL");
+    return submit_host_impl(b, nullptr, xyz, radii, nullptr, params, out, out_job, nullptr, 0, group, out_isolated, false, nullptr,
+                            nullptr, sums != nullptr, nullptr, sums);
+}
+
+int sasa_b200_batch_run_group_pairs_frames_host(sasa_b200_batch *b, const float *xyz, const float *radii, const uint32_t *group,
+                                                const sasa_b200_params *params, const sasa_b200_outputs *out,
+                                                const sasa_b200_outputs *out_isolated, const sasa_b200_pair_sums *sums,
+                                                sasa_b200_stats *stats) {
+    sasa_b200_job *job = nullptr;
+    int rc = sasa_b200_batch_submit_group_pairs_frames_host(b, xyz, radii, group, params, out, out_isolated, sums, &job);
     if (rc) return rc;
     return wait_job_impl(job, stats);
 }

@@ -98,6 +98,17 @@ class PairResult:
     needed: Any = None
 
 
+@dataclass
+class PairSums:
+    """Device-side sums of a pairwise buried-area run of MD frames (``Batch.run_group_pairs_frames_host``), labels 0 .. L - 1:
+    ``pair_area`` (S, L, L) float64, element [s, g, h] the area of group g that group h buries in frame s, and ``seg_pair_area``
+    (n_segments, L) float64, element [q, h] the area of segment q that h buries, or None.  Both are float64 sums of the per-atom
+    slot areas in atom order, bit for bit what :func:`group_pair_table` and per-segment sums of the slots give on the host."""
+    n_labels: int
+    pair_area: Any = None
+    seg_pair_area: Any = None
+
+
 def group_pair_table(partner, buried_area, group, struct_off):
     """Pairwise interface table from the partner slots of a pairwise buried-area run: per structure a list of rows
     ``(g, h, area of g buried by h, area of h buried by g)``, one for each contacting pair of labels g < h, in ascending (g, h)
@@ -444,6 +455,51 @@ class Batch:
                                                                             C.byref(h)))
         return Job(self, h, tuple(res), (xyz, radii, group))
 
+    def _pair_sums(self, n_labels, seg_pairs, out):
+        alloc = (lambda shape: self.engine.pinned_empty(shape, np.float64)) if out == "pinned" else (lambda shape: np.zeros(shape, np.float64))
+        L = int(n_labels)
+        return PairSums(L, alloc((max(self.S, 0), L, L)), alloc((self.n_seg, L)) if seg_pairs and self.n_seg else None)
+
+    def run_group_pairs_frames_host(self, xyz, radii, group, n_labels=None, probe_radius=1.4, n_points=100, simd_lanes=8, flags=0,
+                                    want=("protein",), seg_pairs=True, result=None):
+        """Pairwise buried area of MD frames: run_groups_frames_host plus, per frame, how much of every group each partner group
+        buries, summed on the device.  ``group`` (N,) holds labels 0 .. n_labels - 1 (default: max + 1), n_labels <= 17.  Returns
+        (complex, isolated, sums): the first two are run_groups_frames_host's BatchResults bit for bit, ``sums`` a
+        :class:`PairSums` (its ``seg_pair_area`` when the batch has segments and ``seg_pairs``).  `result`: a (complex, isolated,
+        sums) triple to write into instead of new arrays."""
+        xyz, radii, group = self._groups_frames_args(xyz, radii, group)
+        if n_labels is None:
+            n_labels = int(group.max()) + 1 if group is not None and group.size else 1
+        cpx, iso, sums = result if result is not None else (self._host_outputs(want, "numpy"), self._host_outputs(want, "numpy"),
+                                                            self._pair_sums(n_labels, seg_pairs, "numpy"))
+        outs = [_lib.Outputs(_ptr(r.counts), _ptr(r.atom_sasa), _ptr(r.seg_sasa), _ptr(r.protein)) for r in (cpx, iso)]
+        ps = _lib.PairSums(sums.n_labels, _ptr(sums.pair_area), _ptr(sums.seg_pair_area))
+        prm = self._params(probe_radius, n_points, simd_lanes, flags)
+        st = _lib.Stats()
+        self.engine._check(self._L.sasa_b200_batch_run_group_pairs_frames_host(self._h, _ptr(xyz), _ptr(radii), _ptr(group), C.byref(prm),
+                                                                              C.byref(outs[0]), C.byref(outs[1]), C.byref(ps), C.byref(st)))
+        cpx.stats = iso.stats = st.as_dict()
+        return cpx, iso, sums
+
+    def submit_group_pairs_frames_host(self, xyz, radii, group, n_labels=None, probe_radius=1.4, n_points=100, simd_lanes=8, flags=0,
+                                       want=("protein",), seg_pairs=True, result=None) -> "Job":
+        """Asynchronous run_group_pairs_frames_host: returns at once with a Job whose ``wait()`` returns (complex, isolated,
+        sums).  The outputs are page-locked; xyz should be too (``Engine.pinned_empty``), and the inputs must stay alive until
+        wait returns."""
+        xyz, radii, group = self._groups_frames_args(xyz, radii, group)
+        if n_labels is None:
+            n_labels = int(group.max()) + 1 if group is not None and group.size else 1
+        res = result if result is not None else (self._host_outputs(want, "pinned"), self._host_outputs(want, "pinned"),
+                                                 self._pair_sums(n_labels, seg_pairs, "pinned"))
+        outs = [_lib.Outputs(_ptr(r.counts), _ptr(r.atom_sasa), _ptr(r.seg_sasa), _ptr(r.protein)) for r in res[:2]]
+        ps = _lib.PairSums(res[2].n_labels, _ptr(res[2].pair_area), _ptr(res[2].seg_pair_area))
+        prm = self._params(probe_radius, n_points, simd_lanes, flags)
+        h = C.c_void_p()
+        self.engine._check(self._L.sasa_b200_batch_submit_group_pairs_frames_host(self._h, _ptr(xyz), _ptr(radii), _ptr(group),
+                                                                                 C.byref(prm), C.byref(outs[0]), C.byref(outs[1]),
+                                                                                 C.byref(ps), C.byref(h)))
+        return Job(self, h, tuple(res), (xyz, radii, group))
+
     def _device_outputs(self, want, dev) -> BatchResult:
         import torch
         r = BatchResult()
@@ -554,8 +610,8 @@ class Batch:
 
 
 class Job:
-    """A host-buffer run in flight (sasa_b200_batch_submit_host .. sasa_b200_job_wait).  `result` is a BatchResult, or the
-    (complex, isolated) pair of a grouped run."""
+    """A host-buffer run in flight (sasa_b200_batch_submit_host .. sasa_b200_job_wait).  `result` is a BatchResult, the
+    (complex, isolated) pair of a grouped run, or the (complex, isolated, sums) triple of a pairwise run of frames."""
 
     def __init__(self, batch: Batch, handle, result, keep):
         self.batch, self._h, self.result, self._keep = batch, handle, result, keep
@@ -567,6 +623,7 @@ class Job:
         h, self._h = self._h, None
         self.batch.engine._check(self.batch._L.sasa_b200_job_wait(h, C.byref(st)))
         for r in (self.result if isinstance(self.result, tuple) else (self.result,)):
-            r.stats = st.as_dict()
+            if isinstance(r, BatchResult):
+                r.stats = st.as_dict()
         self._keep = None
         return self.result
